@@ -2,6 +2,7 @@
 """bench.py -- the headline benchmark of the dispatch hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--components all|none]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -19,6 +20,11 @@ HBM peak using the LOGICAL bytes of SURVEY.md section 8(d) (80 B per evaluated p
 feasible plan); `cpu_baseline` = the reference's own pool_n.c compiled -O3, run on the host cores
 on a bounded sample; `components` = the other kernels of the path (K2 20k x 20k time-to-optimal,
 K3 LCM/s at 2000 x 2000, K1 cost build GB/s at 20k x 20k), each with its own roofline figure.
+
+`--dump-outputs DIR` writes what the last timed step computed, as float64 .npy files (rank 0):
+pool_merged_plans.npy [plans, 9] (pool_n.c record layout: 4 pick-up customers, 4 drop-off
+customers, cost) and pool_shard_counters.npy [8, 3] (kept, evaluated, feasible per logical shard).
+The inputs are seeded, so two builds can be compared output for output.
 
 `--impl reference` times ONLY the reference CPU implementation (oracle/_ref/pool_n_big64, the
 unmodified pool_n.c with its shard count raised so that a step is a bounded 1/8 sample).
@@ -252,9 +258,13 @@ def main():
     ap.add_argument("--components", default="all", choices=["all", "none"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--pool-large", type=int, default=5000, help="customers of the north-star pool component (0: skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 0)
-    args.steps = max(args.steps, 1)
 
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.impl == "reference":
@@ -305,10 +315,11 @@ def main():
     all_blocks = torch.zeros((world * slots, cap + 1, 9), dtype=torch.int32, device=dev)
     slot_plans = torch.zeros((slots, cap, 9), dtype=torch.int32, device=dev)
     slot_counts = torch.zeros(slots, dtype=torch.int32, device=dev)
-    slot_shard_l = []
+    slot_shard_l, slot_real = [], []
     for r in range(world):
         sh_r = parallel.shards_for_rank(r, world)
         slot_shard_l += sh_r + [0] * (slots - len(sh_r))   # padding slots carry count 0
+        slot_real += [True] * len(sh_r) + [False] * (slots - len(sh_r))
     slot_shard = torch.tensor(slot_shard_l, dtype=torch.int32, device=dev)
 
     def pool_step(want_stats=False):
@@ -373,6 +384,13 @@ def main():
     if rank == 0:
         last = merged_last[0][: int(merged_last[1].item())].cpu().numpy()
         assert last.tolist() == golden, "timed steps produced a different result than the golden merge"
+        if args.dump_outputs:
+            headers = (all_blocks if world > 1 else blocks)[:, 0, :].cpu().numpy()[slot_real]   # shard order
+            kept, evaluated, feasible = dispatch.Engine.headers_host_view(headers)
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "pool_merged_plans.npy"), last.astype(np.float64))
+            np.save(os.path.join(args.dump_outputs, "pool_shard_counters.npy"),
+                    np.stack([kept, evaluated, feasible], axis=1).astype(np.float64))
     step_ms = [a.elapsed_time(b) for a, b in zip(ev0, ev1)]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -421,7 +439,7 @@ def main():
                 "pool_select_share_of_step": sel_ms / max(sum(step_ms), 1e-9)}
 
     # ---- e2e: the public host API with host buffers ----------------------------------------------
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
 
     def e2e_step():
         if world == 1:

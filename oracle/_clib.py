@@ -21,16 +21,17 @@ def build(force: bool = False) -> str:
     return _SO
 
 
-def build_ref(force: bool = False, ref_dir: str = "/root/reference"):
+def build_ref(force: bool = False, ref_dir: str | None = None):
     """Compile the reference's own pool_n.c (where it lies) into oracle/_ref/pool_n_big.
 
-    Returns the binary path, or None when neither the binary nor the reference tree exists
-    (the GPU box only has the prebuilt file that travelled with the snapshot).
+    ref_dir defaults to $TD_REFERENCE_DIR, a checkout of boguszjelinski/taxidispatcher.
+    Returns the binary path, or None when neither the binary nor the reference tree exists.
     """
+    ref_dir = ref_dir or os.environ.get("TD_REFERENCE_DIR", "")
     out = os.path.join(_HERE, "_ref", "pool_n_big")
     if os.path.exists(out) and os.path.exists(out + "64") and os.path.exists(out + "512") and not force:
         return out
-    if not os.path.exists(os.path.join(ref_dir, "pool_n.c")):
+    if not ref_dir or not os.path.exists(os.path.join(ref_dir, "pool_n.c")):
         return out if os.path.exists(out) else None
     subprocess.check_call(["make", "-C", _HERE, "ref", "REF=" + ref_dir])
     return out

@@ -1,7 +1,7 @@
 """Deterministic synthetic inputs for every BASELINE.json config (SURVEY.md section 8(d)).
 
 TEST INFRASTRUCTURE (part of oracle/): importable from tests/, bench.py and
-__graft_entry__.smoke() only.  Nothing here reads /root/reference.
+__graft_entry__.smoke() only.  Nothing here reads the reference's sources.
 
 All generators use numpy.random.default_rng(seed) (PCG64); costs are int32.
 """
@@ -80,6 +80,34 @@ POOL722_MD5 = "6bfbc99dc994e1e15f988363e197ccc6"
 POOL722_EVALUATED = [382592136, 383212296, 384193104, 391107600, 367492056, 378532392, 381004824, 374816856]
 POOL722_FEASIBLE = [2268957, 2201027, 1922139, 1909089, 2339340, 1986344, 1958445, 2069043]
 POOL722_KEPT = [86, 87, 85, 82, 89, 86, 85, 78]
+
+
+def pool_crosscheck_cases():
+    """Inputs of the pool cross-check against the compiled pool_n.c: [(pool size, demand, shard)], 9 cases x 2 shards --
+    ragged waits and losses, from == to trips, every pool size, over MAX_STAND = 51 stands (pool_n.c:179-185)."""
+    rng = np.random.default_rng(424242)
+    out = []
+    for case in range(9):
+        k = 2 + case % 3
+        n = int(rng.integers(12, 64 if k == 4 else 120))
+        fr = rng.integers(0, 51, n)
+        to = np.where(rng.random(n) < 0.15, fr, rng.integers(0, 51, n))
+        dem = np.stack([np.arange(n), fr, to, rng.integers(0, 9, n), rng.integers(0, 60, n)], axis=1).astype(np.int32)
+        for shard in (0, int(rng.integers(1, 8))):
+            out.append((k, dem, shard))
+    return out
+
+
+# readDemand quirks (pool_n.c:30-54): a blank line, a short record and FEWER lines than rec-number
+DEMAND_QUIRKS_REC_NUMBER = 40
+DEMAND_QUIRKS_RUNS = ((2, 0), (3, 1), (4, 0))      # (pool size, shard)
+
+
+def demand_quirks_csv() -> str:
+    lines = demand_csv(pool_demand(40, seed=9)).splitlines()
+    lines[7] = ""                       # blank line -> a record of zeros
+    lines[11] = "11,3"                  # to / wait / loss stay 0
+    return "\n".join(lines[:33]) + "\n"  # seven fewer records than DEMAND_QUIRKS_REC_NUMBER
 
 
 # ---- config 5: 20k x 20k ----------------------------------------------------------------------

@@ -3,7 +3,7 @@
   find / merge        ctypes front end of oracle/pool_oracle.c (our C restatement of
                       pool_n.c:101-207,226-229 and findpool.c:83-108)
   run_reference       runs the compiled reference binary oracle/_ref/pool_n_big (built from
-                      /root/reference/pool_n.c by oracle/Makefile) on a temp CSV and parses its
+                      $TD_REFERENCE_DIR/pool_n.c by oracle/Makefile) on a temp CSV and parses its
                       CSV output and the three counters it prints
 """
 from __future__ import annotations
@@ -70,14 +70,19 @@ def reference_binary():
 
 def run_reference(demand, pool_size, shard, workdir=None):
     """Run the compiled reference on one shard.  Returns (plans [m,9] int32 in pool_n layout, stats)."""
+    dem = np.asarray(demand, dtype=np.int32).reshape(-1, 5)
+    return run_reference_csv(demand_csv(dem), len(dem), pool_size, shard, workdir)
+
+
+def run_reference_csv(text, rec_number, pool_size, shard, workdir=None):
+    """`pool_n pool_size shard demand.csv rec_number out.csv` on a demand file of the given text."""
     exe = reference_binary()
     if exe is None or not os.path.exists(exe):
         raise FileNotFoundError("oracle/_ref/pool_n_big is not built (make -C oracle ref)")
-    dem = np.asarray(demand, dtype=np.int32).reshape(-1, 5)
     with tempfile.TemporaryDirectory(dir=workdir) as td:
         with open(os.path.join(td, "demand.csv"), "w") as f:
-            f.write(demand_csv(dem))
-        res = subprocess.run([exe, str(pool_size), str(shard), "demand.csv", str(len(dem)), "out.csv"],
+            f.write(text)
+        res = subprocess.run([exe, str(pool_size), str(shard), "demand.csv", str(rec_number), "out.csv"],
                              cwd=td, capture_output=True, text=True, check=True)
         plans = parse_result_csv(open(os.path.join(td, "out.csv")).read(), pool_size)
     # count_all is a 32-bit `int` in the reference (pool_n.c:28) and wraps beyond 2^31 leaf plans per shard

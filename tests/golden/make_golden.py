@@ -1,16 +1,18 @@
 #!/usr/bin/env python
-"""Regenerates tests/golden/*.json.  Run from the repo root IN THE BUILD CONTAINER:
+"""Regenerates tests/golden/*.json.  Run from the repo root with a checkout of the reference:
 
-    python tests/golden/make_golden.py [--skip-722]
+    TD_REFERENCE_DIR=<checkout of boguszjelinski/taxidispatcher> python tests/golden/make_golden.py [--skip-722]
+        [--only-crosscheck]
 
 Sources of truth (nothing here touches the CUDA path):
-  pool_*      the compiled reference oracle/_ref/pool_n_big (pool_n.c from /root/reference,
+  pool_*      the compiled reference oracle/_ref/pool_n_big (pool_n.c from $TD_REFERENCE_DIR,
               built by `make -C oracle ref`), 8 logical shards, merged in shard order
-              (findpool.c:83-108 restated in oracle/pool_oracle.c)
+              (findpool.c:83-108 restated in oracle/pool_oracle.c); pool_reference_crosscheck.json
+              holds its single-shard answers for the cross-checks of tests/test_oracle.py
   lcm_*       the reference LCM bodies executed by numpy (oracle/lcm_ref.py)
   assign_*    scipy.optimize.linear_sum_assignment / linprog(HiGHS) on the reference layout and
               the literals of python.py:7, glpk.mod:27-31, procedure.py:32-51
-The committed JSON travels to the GPU box; /root/reference does not.
+The tests read the committed JSON; the cross-checks run the compiled reference instead where it is built.
 """
 from __future__ import annotations
 
@@ -28,6 +30,7 @@ sys.path.insert(0, ROOT)
 from oracle import assign_ref, cost_ref, gen_inputs as g, lcm_ref, pool_ref  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
+CROSSCHECK = "pool_reference_crosscheck.json"
 
 
 def sha(arr) -> str:
@@ -90,9 +93,23 @@ def large_slices(spec):
                                     "n_shards": 512, "demand_sha256": sha(dem), "slices": slices})
 
 
+def crosscheck():
+    """What the two cross-checks of tests/test_oracle.py compare against, for checkouts without the compiled reference:
+    its plans and counters on gen_inputs.pool_crosscheck_cases() and on gen_inputs.demand_quirks_csv()."""
+    cases = [{"pool_size": k, "shard": sh, "demand_sha256": sha(dem), "plans": p.tolist(), "stats": st}
+             for k, dem, sh in g.pool_crosscheck_cases() for p, st in [pool_ref.run_reference(dem, k, sh)]]
+    text = g.demand_quirks_csv()
+    quirks = [{"pool_size": k, "shard": sh,
+               "plans": pool_ref.run_reference_csv(text, g.DEMAND_QUIRKS_REC_NUMBER, k, sh)[0].tolist()}
+              for k, sh in g.DEMAND_QUIRKS_RUNS]
+    dump(CROSSCHECK, {"source": "oracle/_ref/pool_n_big (pool_n.c compiled by `make -C oracle ref`)",
+                      "cases": cases, "demand_quirks": quirks})
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--skip-722", action="store_true")
+    ap.add_argument("--only-crosscheck", action="store_true", help="only write " + CROSSCHECK)
     ap.add_argument("--only-large", type=int, default=0, help="only write pool<N>.json for N customers (minutes of CPU)")
     ap.add_argument("--large-slices", default="", help="N:t0,t1,...: slices t of the 512-way shard rule of pool_n.c for N "
                                                         "customers (north-star size; ~10 CPU-minutes per slice, run in parallel)")
@@ -108,6 +125,9 @@ def main():
         dump("pool%d.json" % a.only_large, c)
         return
     assert pool_ref.reference_binary(), "build oracle/_ref first: make -C oracle ref"
+    crosscheck()
+    if a.only_crosscheck:
+        return
 
     # ---- pool: small cases (KAT P1) with the inputs inlined ---------------------------------
     small = []
