@@ -181,6 +181,35 @@ int td_assign_certify(const int32_t *cost, int n, int n_real_rows, int n_real_co
                       void *workspace, size_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Batches of small independent instances     replace the per-instance loops of heuristic.py:20-40
+ *     (1000 random 100 x 100 cases, each through LCM and the exact solver) and python.py:6-25.
+ *
+ * One launch per call, one CTA per instance; the instance sits in shared memory, so sizes are
+ * limited to TD_BATCH_MAX_N.  Instance b is sizes[b] x sizes[b] row-major int32 at
+ * costs + offsets[b] (elements, a multiple of 4); costs is 16-byte aligned; sizes / offsets are
+ * DEVICE arrays; outputs use a stride of n_max per instance (slots past an instance's result hold
+ * -1, potentials 0).  Always asynchronous, no workspace.  An instance with size < 0 or > n_max, or
+ * an offset < 0 or not a multiple of 4, is withdrawn (objective / total INT64_MIN, n_pairs -1,
+ * last_min INT32_MIN, every col / row -1); the other instances are unaffected.  A size-0 instance
+ * has objective 0 and 0 pairs.
+ *
+ * td_assign_exact_batch runs the same routine as td_assign_exact does for a balanced n <= 232
+ * matrix, so both return the identical col_of_row; u_out / v_out (optional) are the dual
+ * potentials (see td_assign_certificate below).  td_lcm_batch runs the literal array algorithm
+ * of td_lcm with the same params for every instance and returns the same trace.
+ * ------------------------------------------------------------------------------------------ */
+#define TD_BATCH_MAX_N 232     /* 232^2 x 4 B = 210 KB of the 227 KB of shared memory of one CTA */
+int td_assign_exact_batch(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                          int32_t *col_of_row_out /* batch x n_max */, int64_t *objective_out /* batch */,
+                          int64_t *u_out /* batch x n_max or NULL */, int64_t *v_out /* batch x n_max or NULL */,
+                          void *stream);
+int td_lcm_batch(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                 const td_lcm_params *params /* host, same for every instance */,
+                 int32_t *rows_out /* batch x n_max */, int32_t *cols_out /* batch x n_max */,
+                 int32_t *n_pairs_out /* batch */, int64_t *total_out /* batch */,
+                 int32_t *last_min_out /* batch, may be NULL */, void *stream);
+
+/* ------------------------------------------------------------------------------------------
  * K4  pool finder            replaces one `pool_n <pool-size> <thread> <file> <n> <out>` process
  *     (pool_n.c:209-238): findPool :153-177, drop_customers :101-151, removeDuplicates :187-207,
  *     shard rule :226-229.

@@ -989,11 +989,18 @@ assign_kernel(AsgArgs a) {
 // row-reduced costs, greedy matching on tight cells -- only the rows that stay free are augmented.
 // Exact for any int32 costs (potentials and distances in int64); ties resolve to the smallest column, deterministic.
 // Leaves the dual potentials in the workspace like assign_kernel does (td_assign_read_duals / td_assign_certify).
-constexpr int kSmallN = 232;          // 232^2 * 4 B = 210 KB of the 227 KB
+// The body is a device routine shared by the single-instance kernel and the batched one (one CTA per instance), so both
+// return the same matching and the same potentials for the same matrix.  u_out / v_out may be NULL; the objective is
+// written to *objective_out and returned on thread 0.
+constexpr int kSmallN = TD_BATCH_MAX_N;   // 232^2 * 4 B = 210 KB of the 227 KB
 constexpr int kSmallThreads = 256;
-__global__ void __launch_bounds__(kSmallThreads)
-assign_small_kernel(const int32_t *__restrict__ cost, int n, int32_t *col_of_row_out, long long *objective_out, uint8_t *x_out,
-                    long long *u_out, long long *v_out, AsgCtrl *ctrl) {
+static_assert(kSmallN <= kSmallThreads, "column j lives in thread j");
+__host__ __device__ constexpr size_t small_smem_bytes(int n) {
+    return ((size_t(n) * n * 4 + 15) & ~size_t(15)) + size_t(n) * (8 + 4 + 4 + 4 + 4) + 64;
+}
+__device__ __forceinline__ long long
+assign_small_solve(const int32_t *__restrict__ cost, int n, int32_t *col_of_row_out, long long *objective_out, uint8_t *x_out,
+                   long long *u_out, long long *v_out) {
     extern __shared__ __align__(16) unsigned char ssm[];
     int32_t *c = reinterpret_cast<int32_t *>(ssm);                                   // [n][n]
     long long *u = reinterpret_cast<long long *>(ssm + ((size_t(n) * n * 4 + 15) & ~size_t(15)));   // [n]
@@ -1120,19 +1127,51 @@ assign_small_kernel(const int32_t *__restrict__ cost, int n, int32_t *col_of_row
         col_of_row_out[t] = j;
         part = c[t * n + j];
         if (x_out) x_out[size_t(t) * n + j] = 1;
-        u_out[t] = u[t];
-        v_out[t] = v;
+        if (u_out) u_out[t] = u[t];
+        if (v_out) v_out[t] = v;
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
     if (lane == 0) s_rk[w] = part;
     __syncthreads();
+    long long tot = 0;
     if (t == 0) {
-        long long tot = 0;
         for (int k = 0; k < kSmallThreads / 32; ++k) tot += s_rk[k];
         *objective_out = tot;
-        ctrl->objective = tot; ctrl->status = TD_OK; ctrl->phases = 1;
     }
+    return tot;
+}
+
+__global__ void __launch_bounds__(kSmallThreads)
+assign_small_kernel(const int32_t *__restrict__ cost, int n, int32_t *col_of_row_out, long long *objective_out, uint8_t *x_out,
+                    long long *u_out, long long *v_out, AsgCtrl *ctrl) {
+    const long long tot = assign_small_solve(cost, n, col_of_row_out, objective_out, x_out, u_out, v_out);
+    if (threadIdx.x == 0) { ctrl->objective = tot; ctrl->status = TD_OK; ctrl->phases = 1; }
+}
+
+// Batch: CTA b solves instance b (sizes[b] x sizes[b] at costs + offsets[b]) with the routine above.  Outputs have a stride
+// of n_max; the slots past an instance's size hold col -1 and potentials 0.  An instance whose size or offset is out of
+// range is withdrawn (objective INT64_MIN, every col -1) without touching its matrix.
+__global__ void __launch_bounds__(kSmallThreads)
+assign_batch_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict__ sizes, const int64_t *__restrict__ offsets,
+                    int n_max, int32_t *col_of_row_out, long long *objective_out, long long *u_out, long long *v_out) {
+    const int b = blockIdx.x;
+    const int n = sizes[b];
+    const long long off = offsets[b];
+    const size_t o = size_t(b) * n_max;
+    const bool bad = n < 0 || n > n_max || off < 0 || (off & 3) != 0;
+    const int keep = bad ? 0 : n;
+    for (int t = keep + threadIdx.x; t < n_max; t += kSmallThreads) {
+        col_of_row_out[o + t] = -1;
+        if (u_out) u_out[o + t] = 0;
+        if (v_out) v_out[o + t] = 0;
+    }
+    if (bad) {
+        if (threadIdx.x == 0) objective_out[b] = LLONG_MIN;
+        return;
+    }
+    assign_small_solve(costs + off, n, col_of_row_out + o, objective_out + b, nullptr, u_out ? u_out + o : nullptr,
+                       v_out ? v_out + o : nullptr);
 }
 
 static AsgArgs carve_assign(void *ws, int n, size_t *bytes) {
@@ -1265,7 +1304,7 @@ static int td::assign_run(const int32_t *cost, int n, int nr, int32_t *col_of_ro
     TD_CUDA_TRY(cudaMemsetAsync(a.ctrl, 0, sizeof(AsgCtrl), st));
     if (x_out) TD_CUDA_TRY(cudaMemsetAsync(x_out, 0, size_t(n) * n, st));
     if (n <= kSmallN && nr == n && !getenv("TD_ASSIGN_NO_SMALL")) {   // balanced and small: one CTA in shared memory
-        const size_t smem = ((size_t(n) * n * 4 + 15) & ~size_t(15)) + size_t(n) * (8 + 4 + 4 + 4 + 4) + 64;
+        const size_t smem = small_smem_bytes(n);
         TD_CUDA_TRY(cudaFuncSetAttribute(assign_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
         {
             ProfScope prof(TD_PROF_ASSIGN, st);
@@ -1333,6 +1372,26 @@ static int td::assign_run(const int32_t *cost, int n, int nr, int32_t *col_of_ro
                     h.t_prof[11] / 1e3, h.t_prof[15]);
         if (h.status != TD_OK) return h.status;
     }
+    return TD_OK;
+}
+
+extern "C" int td_assign_exact_batch(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                                     int32_t *col_of_row_out, int64_t *objective_out, int64_t *u_out, int64_t *v_out,
+                                     void *stream) {
+    using namespace td;
+    if (batch < 0 || n_max < 0 || n_max > TD_BATCH_MAX_N) return TD_ERR_INVALID;
+    if (batch == 0) return TD_OK;
+    if (!costs || !sizes || !offsets || !col_of_row_out || !objective_out) return TD_ERR_INVALID;
+    if ((reinterpret_cast<uintptr_t>(costs) & 15) != 0) return TD_ERR_INVALID;
+    if (!have_device()) return TD_ERR_NO_DEVICE;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t smem = small_smem_bytes(n_max);
+    TD_CUDA_TRY(cudaFuncSetAttribute(assign_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    assign_batch_kernel<<<batch, kSmallThreads, smem, st>>>(costs, sizes, offsets, n_max, col_of_row_out,
+                                                            reinterpret_cast<long long *>(objective_out),
+                                                            reinterpret_cast<long long *>(u_out),
+                                                            reinterpret_cast<long long *>(v_out));
+    TD_LAUNCH_CHECK();
     return TD_OK;
 }
 

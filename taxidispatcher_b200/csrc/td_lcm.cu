@@ -446,6 +446,96 @@ lcm_finalize_kernel(const unsigned long long *__restrict__ sorted, int n, td_lcm
     if (last_min_out) *last_min_out = last_min;
 }
 
+// ---- batches of small instances: one CTA per instance, the literal array algorithm in shared memory ---------------------
+// The working array d (n x n, n <= TD_BATCH_MAX_N) lives in shared memory and is overwritten with mask_value exactly like the
+// reference does, so "the mask is a value" holds by construction.  rk[i] caches row i's minimum key (value, i*n + j); the
+// whole-array first-index argmin is the block minimum of rk.  After row r and column c are masked:
+//   row r                   -> (mask, r*n + 0)             (every cell of the row is the mask now)
+//   a row cached at column c -> rescanned, one warp per row  (its minimum just changed to something unknown)
+//   every other row          -> min(rk[i], (mask, i*n + c))  (only cell c changed, and it was not the minimum)
+constexpr int kLcmBatchThreads = 256;
+
+__device__ __forceinline__ uint64_t lcm_row_min(const int32_t *d, int n, int i, int lane) {
+    uint64_t best = kKeyInf;
+    for (int j = lane; j < n; j += 32) { const uint64_t k = pack_key(d[i * n + j], uint32_t(i * n + j)); best = k < best ? k : best; }
+    return warp_min_u64(best);
+}
+
+__global__ void __launch_bounds__(kLcmBatchThreads)
+lcm_batch_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict__ sizes, const int64_t *__restrict__ offsets,
+                 int n_max, td_lcm_params prm, int32_t *rows_out, int32_t *cols_out, int32_t *n_pairs_out,
+                 long long *total_out, int32_t *last_min_out) {
+    extern __shared__ __align__(16) unsigned char lbs[];
+    const int b = blockIdx.x;
+    const int n = sizes[b];
+    const long long off = offsets[b];
+    const size_t o = size_t(b) * n_max;
+    const int t = threadIdx.x, lane = t & 31, w = t >> 5;
+    constexpr int nw = kLcmBatchThreads / 32;
+    const bool bad = n < 0 || n > n_max || off < 0 || (off & 3) != 0;
+    if (bad) {
+        for (int k = t; k < n_max; k += kLcmBatchThreads) { rows_out[o + k] = -1; cols_out[o + k] = -1; }
+        if (t == 0) {
+            n_pairs_out[b] = -1; total_out[b] = LLONG_MIN;
+            if (last_min_out) last_min_out[b] = INT32_MIN;
+        }
+        return;
+    }
+    unsigned long long *rk = reinterpret_cast<unsigned long long *>(lbs);      // [n]
+    int32_t *d = reinterpret_cast<int32_t *>(rk + n_max);                     // [n][n]
+    int *stale = reinterpret_cast<int *>(d + size_t(n_max) * n_max);          // rows to rescan [n]
+    __shared__ unsigned long long s_min[nw];
+    __shared__ int s_nstale;
+    const int32_t *src = costs + off;
+    for (int k = t; k < n * n; k += kLcmBatchThreads) d[k] = __ldg(src + k);
+    __syncthreads();
+    for (int i = w; i < n; i += nw) { const uint64_t k = lcm_row_min(d, n, i, lane); if (lane == 0) rk[i] = k; }
+    const int iters = (prm.max_iters < 0 || prm.max_iters > n) ? n : prm.max_iters;
+    long long total = 0;
+    int pairs = 0;
+    int32_t last_min = INT32_MAX;
+    for (int it = 0; it < iters; ++it) {
+        __syncthreads();                                  // rk complete
+        uint64_t m = t < n ? rk[t] : kKeyInf;
+        m = warp_min_u64(m);
+        if (lane == 0) s_min[w] = m;
+        if (t == 0) s_nstale = 0;
+        __syncthreads();
+        uint64_t g = s_min[0];
+#pragma unroll
+        for (int k = 1; k < nw; ++k) g = s_min[k] < g ? s_min[k] : g;
+        const int32_t v = key_value(g);
+        last_min = v;
+        if (prm.stop_above != INT32_MAX && v > prm.stop_above) break;
+        if (prm.stop_at_value != INT32_MAX && v >= prm.stop_at_value) break;
+        const int e = int(key_index(g)), r = e / n, c = e - r * n;
+        if (t == 0) { rows_out[o + pairs] = r; cols_out[o + pairs] = c; }
+        ++pairs;
+        if (prm.sum_below == INT32_MAX || v < prm.sum_below) total += v;
+        if (t < n) {
+            d[r * n + t] = prm.mask_value;
+            d[t * n + c] = prm.mask_value;
+            const uint64_t k = rk[t];
+            if (t == r) rk[t] = pack_key(prm.mask_value, uint32_t(r * n));
+            else if (int(key_index(k)) - t * n == c) stale[atomicAdd(&s_nstale, 1)] = t;
+            else { const uint64_t km = pack_key(prm.mask_value, uint32_t(t * n + c)); rk[t] = km < k ? km : k; }
+        }
+        __syncthreads();                                  // mask written, stale list complete
+        const int ns = s_nstale;
+        for (int s = w; s < ns; s += nw) { const int i = stale[s]; const uint64_t k = lcm_row_min(d, n, i, lane); if (lane == 0) rk[i] = k; }
+        if (prm.residual_size > 0 && n - pairs == prm.residual_size) break;
+    }
+    for (int k = pairs + t; k < n_max; k += kLcmBatchThreads) { rows_out[o + k] = -1; cols_out[o + k] = -1; }
+    if (t == 0) {
+        n_pairs_out[b] = pairs; total_out[b] = total;
+        if (last_min_out) last_min_out[b] = last_min;
+    }
+}
+
+static size_t lcm_batch_smem_bytes(int n_max) {
+    return size_t(n_max) * 8 + size_t(n_max) * n_max * 4 + size_t(n_max) * 4;
+}
+
 struct LcmWorkspace {
     int32_t *costT;
     unsigned long long *rowkey, *colkey, *picked, *sorted, *gkey2;
@@ -534,6 +624,24 @@ extern "C" int td_lcm(const int32_t *cost, int n, const td_lcm_params *params, i
     TD_LAUNCH_CHECK();
     lcm_finalize_kernel<<<1, kFinThreads, 0, st>>>(w.sorted, n, prm, w.ctrl, rows_out, cols_out, n_pairs_out,
                                                    reinterpret_cast<long long *>(total_out), last_min_out);
+    TD_LAUNCH_CHECK();
+    return TD_OK;
+}
+
+extern "C" int td_lcm_batch(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                            const td_lcm_params *params, int32_t *rows_out, int32_t *cols_out, int32_t *n_pairs_out,
+                            int64_t *total_out, int32_t *last_min_out, void *stream) {
+    using namespace td;
+    if (batch < 0 || n_max < 0 || n_max > TD_BATCH_MAX_N) return TD_ERR_INVALID;
+    if (batch == 0) return TD_OK;
+    if (!costs || !sizes || !offsets || !params || !rows_out || !cols_out || !n_pairs_out || !total_out) return TD_ERR_INVALID;
+    if ((reinterpret_cast<uintptr_t>(costs) & 15) != 0) return TD_ERR_INVALID;
+    if (!have_device()) return TD_ERR_NO_DEVICE;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t smem = lcm_batch_smem_bytes(n_max);
+    TD_CUDA_TRY(cudaFuncSetAttribute(lcm_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    lcm_batch_kernel<<<batch, kLcmBatchThreads, smem, st>>>(costs, sizes, offsets, n_max, *params, rows_out, cols_out, n_pairs_out,
+                                                            reinterpret_cast<long long *>(total_out), last_min_out);
     TD_LAUNCH_CHECK();
     return TD_OK;
 }

@@ -9,6 +9,7 @@ Host functions mirror the reference's names, argument order and return layouts
   LCM(n, c, ...)                                   heuristic.py:24-33, split.py:161-175,
                                                    greedy_opt.py:61-82, simulate.py:76-97
   LCM_java(cost)                                   Simulator.java:523-549
+  solve_batch(costs) / LCM_batch(costs, ...)       heuristic.py:20-40, python.py:6-25 over many instances
   find_pool(...) / find_pool_all(...) / pool_merge(...)   pool_n.c / findpool.c
 
 PyTorch is used only for device buffers, pinned staging and streams.  All arithmetic runs in the
@@ -29,7 +30,7 @@ from ._lib import BIG_COST, INT32_MAX, POOL_REC_W, AssignStats, LcmParams, PoolS
 
 __all__ = ["BIG_COST", "Engine", "calculate_cost", "solve", "solve_dispatch", "solve_full", "solve_assignment", "LCM", "LCM_heuristic",
            "LCM_split", "LCM_greedy_opt", "LCM_simulate", "LCM_java", "find_pool", "find_pool_all", "find_pool_block",
-           "find_pool_pairs", "pool_merge",
+           "find_pool_pairs", "pool_merge", "pack_batch", "run_batch", "solve_batch", "LCM_batch",
            "TaxiDispatchError"]
 
 
@@ -115,6 +116,71 @@ def _h2d_i32_many(arrays) -> list:
     ev.record()
     slot["ev"] = ev
     return [dev[off: off + arr.size].reshape(arr.shape) for arr, off in zip(arrs, offs)]
+
+
+BATCH_MAX_N = 232   # TD_BATCH_MAX_N: the largest instance the batched kernels hold in one CTA's shared memory
+
+
+def pack_batch(costs: Sequence):
+    """Square host matrices -> (packed, sizes, offsets, n_max) on the device for Engine.assign_batch / lcm_batch.
+    Instance b is stored row-major at packed[offsets[b]:], padded to a multiple of 4 elements; sizes (int32) and offsets
+    (int64) travel in the same pinned buffer, so the whole batch is ONE host->device copy."""
+    mats = []
+    for c in costs:
+        a = np.asarray(c)
+        if a.ndim != 2 or a.shape[0] != a.shape[1]:
+            raise ValueError("pack_batch takes square matrices, got shape %s" % (a.shape,))
+        mats.append(a)
+    B = len(mats)
+    sizes = np.array([a.shape[0] for a in mats], dtype=np.int32)
+    offsets = np.zeros(B, dtype=np.int64)
+    total = 0
+    for b, a in enumerate(mats):
+        offsets[b] = total
+        total += (a.size + 3) & ~3
+    meta = (total + 1) & ~1                               # sizes start here; offsets at an even int32 index (int64 view)
+    off_at = (meta + B + 1) & ~1
+    words = max(off_at + 2 * B, 4)
+    COPIED["h2d"] += words * 4
+    bucket = 1 << max(8, int(words - 1).bit_length())
+    slot = _PINNED.get(("batch", bucket)) if bucket <= (1 << 24) else None
+    if slot is None:
+        slot = {"buf": torch.empty(bucket, dtype=torch.int32).pin_memory(), "ev": None}
+        if bucket <= (1 << 24):
+            _PINNED[("batch", bucket)] = slot
+    if slot["ev"] is not None:
+        slot["ev"].synchronize()
+    host = slot["buf"].numpy()
+    for a, o in zip(mats, offsets):
+        host[o: o + a.size] = a.reshape(-1)
+    host[meta: meta + B] = sizes
+    host[off_at: off_at + 2 * B] = offsets.view(np.int32)
+    dev = slot["buf"][:words].to("cuda", non_blocking=True)
+    ev = torch.cuda.Event()
+    ev.record()
+    slot["ev"] = ev
+    n_max = int(sizes.max()) if B else 0
+    return dev[:max(total, 4)], dev[meta: meta + B], dev[off_at: off_at + 2 * B].view(torch.int64), n_max
+
+
+_NP_OF = {torch.int32: np.int32, torch.int64: np.int64}
+
+
+class _Arena:
+    """Several output tensors carved from ONE device buffer, so that a batch comes back in one device->host copy."""
+
+    def __init__(self, device, parts):
+        self.spec, off = [], 0
+        for numel, dtype in parts:
+            nbytes = int(numel) * np.dtype(_NP_OF[dtype]).itemsize
+            self.spec.append((off, nbytes, dtype))
+            off += (nbytes + 7) & ~7
+        self.buf = torch.empty(max(off, 8), dtype=torch.uint8, device=device)
+        self.views = [self.buf[o: o + nb].view(dt) for o, nb, dt in self.spec]
+
+    def host(self):
+        h = _d2h(self.buf)
+        return [h[o: o + nb].view(_NP_OF[dt]) for o, nb, dt in self.spec]
 
 
 class Engine:
@@ -227,6 +293,46 @@ class Engine:
         out["optimal"] = (c.min_reduced_cost >= 0 and c.max_matched_slack == 0 and c.sign_violations == 0 and
                           c.dual_objective == c.matched_real_cost)
         return out
+
+    # -- batches of small instances (td_assign_exact_batch / td_lcm_batch) -------------------------
+    def _batch_out(self, out, name, shape, dtype):
+        if out is not None and out.get(name) is not None:
+            return out[name]
+        return torch.empty(shape, dtype=dtype, device=self.device)
+
+    def assign_batch(self, packed: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor, n_max: int,
+                     want_duals: bool = False, out: Optional[dict] = None):
+        """Exact optimum of every instance of a pack_batch() buffer, one launch.  Returns device tensors
+        (col [B, n_max] int32, objective [B] int64, u, v) -- u / v are [B, n_max] int64 potentials or None.
+        `out` may supply any of them by name ("col", "objective", "u", "v")."""
+        B = int(sizes.numel())
+        col = self._batch_out(out, "col", (B, n_max), torch.int32)
+        obj = self._batch_out(out, "objective", (B,), torch.int64)
+        u = self._batch_out(out, "u", (B, n_max), torch.int64) if want_duals else None
+        v = self._batch_out(out, "v", (B, n_max), torch.int64) if want_duals else None
+        rc = self.lib.td_assign_exact_batch(_ptr(packed), _ptr(sizes), _ptr(offsets), B, int(n_max), _ptr(col), _ptr(obj),
+                                            _ptr(u), _ptr(v), _stream())
+        check(rc, "td_assign_exact_batch")
+        return col, obj, u, v
+
+    def lcm_batch(self, packed: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor, n_max: int, mask_value: int,
+                  stop_above: int = INT32_MAX, stop_at_value: int = INT32_MAX, sum_below: int = INT32_MAX,
+                  residual_size: int = 0, max_iters: int = -1, out: Optional[dict] = None):
+        """LCM of every instance of a pack_batch() buffer, one launch, the same params for all.  Returns device tensors
+        (rows [B, n_max], cols [B, n_max], n_pairs [B] int32, total [B] int64, last_min [B] int32); `out` may supply
+        any of them by name."""
+        B = int(sizes.numel())
+        rows = self._batch_out(out, "rows", (B, n_max), torch.int32)
+        cols = self._batch_out(out, "cols", (B, n_max), torch.int32)
+        npairs = self._batch_out(out, "n_pairs", (B,), torch.int32)
+        total = self._batch_out(out, "total", (B,), torch.int64)
+        last = self._batch_out(out, "last_min", (B,), torch.int32)
+        prm = LcmParams(int(mask_value), int(stop_above), int(stop_at_value), int(sum_below), int(residual_size),
+                        int(max_iters))
+        rc = self.lib.td_lcm_batch(_ptr(packed), _ptr(sizes), _ptr(offsets), B, int(n_max), ctypes.byref(prm), _ptr(rows),
+                                   _ptr(cols), _ptr(npairs), _ptr(total), _ptr(last), _stream())
+        check(rc, "td_lcm_batch")
+        return rows, cols, npairs, total, last
 
     # -- K4 ---------------------------------------------------------------------------------------
     def pool_find(self, demand: torch.Tensor, dist: torch.Tensor, pool_size: int, shard: int = 0, n_shards: int = 8,
@@ -508,6 +614,93 @@ def LCM(n: int, c, mask_value: int = BIG_COST, stop_above: int = INT32_MAX, stop
     eng = engine()
     cost = _h2d_i32(np.asarray(c).reshape(n, n))
     return Engine.lcm_host_view(*eng.lcm(cost, mask_value, stop_above, stop_at_value, sum_below, residual_size, max_iters))
+
+
+def _lcm_params(mask_value, stop_above, stop_at_value, sum_below, residual_size, max_iters):
+    return dict(mask_value=mask_value, stop_above=stop_above, stop_at_value=stop_at_value, sum_below=sum_below,
+                residual_size=residual_size, max_iters=max_iters)
+
+
+def run_batch(costs: Sequence, assign: bool = True, want_duals: bool = False, lcm: Optional[dict] = None):
+    """Exact assignment and / or LCM (`lcm` = its keyword parameters) of every square matrix in `costs`.  Instances up to
+    BATCH_MAX_N are uploaded once and served by one launch per kernel, both kernels reading the same packed buffer, and
+    come back in one device->host copy; larger ones take the single-instance path.  Returns (assign results, LCM
+    results): lists of (col_of_row, objective[, u, v]) and of LCM() dicts, None for the side not asked for."""
+    mats = [np.asarray(c) for c in costs]
+    fits = [a.ndim == 2 and a.shape[0] <= BATCH_MAX_N for a in mats]
+    small = [b for b, f in enumerate(fits) if f]
+    large = [b for b, f in enumerate(fits) if not f]
+    res_a = [None] * len(mats) if assign else None
+    res_l = [None] * len(mats) if lcm is not None else None
+    if small:
+        eng = engine()
+        packed, sizes, offsets, n_max = pack_batch([mats[b] for b in small])
+        B = len(small)
+        parts = []
+        if assign:
+            parts += [(B * n_max, torch.int32), (B, torch.int64)] + ([(B * n_max, torch.int64)] * 2 if want_duals else [])
+        if lcm is not None:
+            parts += [(B * n_max, torch.int32), (B * n_max, torch.int32), (B, torch.int32), (B, torch.int64), (B, torch.int32)]
+        arena = _Arena(eng.device, parts)
+        views = list(arena.views)
+        if assign:
+            names = ["col", "objective"] + (["u", "v"] if want_duals else [])
+            out = {k: views.pop(0) for k in names}
+            for k in ("col", "u", "v"):
+                if k in out:
+                    out[k] = out[k].view(B, n_max)
+            eng.assign_batch(packed, sizes, offsets, n_max, want_duals=want_duals, out=out)
+        if lcm is not None:
+            out = {k: views.pop(0) for k in ("rows", "cols", "n_pairs", "total", "last_min")}
+            out["rows"], out["cols"] = out["rows"].view(B, n_max), out["cols"].view(B, n_max)
+            eng.lcm_batch(packed, sizes, offsets, n_max, out=out, **lcm)
+        host = arena.host()                                        # the one read-back of the batch
+        if assign:
+            col, obj = host.pop(0).reshape(B, n_max), host.pop(0)
+            u = host.pop(0).reshape(B, n_max) if want_duals else None
+            v = host.pop(0).reshape(B, n_max) if want_duals else None
+            for k, b in enumerate(small):
+                n = mats[b].shape[0]
+                r = (col[k, :n].copy(), int(obj[k]))
+                res_a[b] = r + (u[k, :n].copy(), v[k, :n].copy()) if want_duals else r
+        if lcm is not None:
+            rows, cols = host.pop(0).reshape(B, n_max), host.pop(0).reshape(B, n_max)
+            npairs, total, last = host.pop(0), host.pop(0), host.pop(0)
+            for k, b in enumerate(small):
+                m = int(npairs[k])
+                res_l[b] = {"total": int(total[k]), "n_pairs": m, "rows": rows[k, :m].copy(), "cols": cols[k, :m].copy(),
+                            "last_min": int(last[k])}
+    for b in large:                                                # beyond one CTA's shared memory: one call each
+        a = mats[b]
+        if a.ndim != 2 or a.shape[0] != a.shape[1]:
+            raise ValueError("run_batch takes square matrices, got shape %s" % (a.shape,))
+        eng = engine()
+        n = a.shape[0]
+        c = _h2d_i32(a)
+        if assign:
+            col, obj, _, _ = eng.assign(c)
+            r = (_d2h(col), _d2h_int(obj))
+            if want_duals:
+                u, v = eng.assign_duals(n)
+                r = r + (_d2h(u), _d2h(v))
+            res_a[b] = r
+        if lcm is not None:
+            res_l[b] = Engine.lcm_host_view(*eng.lcm(c, **lcm))
+    return res_a, res_l
+
+
+def solve_batch(costs: Sequence, want_duals: bool = False):
+    """Exact optimum of every square matrix in `costs` (python.py:6-25, heuristic.py:37 run over many instances): a list
+    of (col_of_row, objective), or (col_of_row, objective, u, v) with the dual potentials when want_duals."""
+    return run_batch(costs, assign=True, want_duals=want_duals)[0]
+
+
+def LCM_batch(costs: Sequence, mask_value: int = BIG_COST, stop_above: int = INT32_MAX, stop_at_value: int = INT32_MAX,
+              sum_below: int = INT32_MAX, residual_size: int = 0, max_iters: int = -1):
+    """LCM() of every square matrix in `costs` with the same parameters (heuristic.py:24-33 run over many instances):
+    a list of the dicts LCM() returns."""
+    prm = _lcm_params(mask_value, stop_above, stop_at_value, sum_below, residual_size, max_iters)
+    return run_batch(costs, assign=False, lcm=prm)[1]
 
 
 def LCM_heuristic(n, c, mask: int = 100):

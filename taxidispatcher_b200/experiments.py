@@ -4,10 +4,11 @@
   solve_split        split.py:61-119   stands cut into size/4-wide ranges, one exact solve per range, then a
                                        last solve over the customers and cabs the ranges left unserved
   greedy_then_solve  greedy_opt.py:131-163   LCM prefix with a distance threshold, exact solve on the rest
+  lcm_vs_optimum     heuristic.py:20-40      LCM (mask 100) against the exact optimum on many small instances
 
 Every range of solve_split is an independent K1 + K2 instance: with a process group the ranges are spread
 over the ranks (parallel.instances_for_rank), the unserved ids are gathered, and the leftover solve runs
-once.  `solver` / `lcm` are injectable so that the host logic can be checked on CPU (tests only).
+once.  `solver` / `lcm` (and the batch functions) are injectable so that the host logic can be checked on CPU (tests only).
 """
 from __future__ import annotations
 
@@ -191,3 +192,20 @@ def greedy_then_solve(distances, demand, cabs, threshold: int = 10, solver: Opti
     n2, x2, cost_table2 = solver(distances, rest_demand, rest_cabs)
     res2 = count_sum(n2, cost_table2, x2, rest_demand, rest_cabs, distances, 0)
     return nn, res, n2, res2 + int(lcm_total)
+
+
+def lcm_vs_optimum(costs: Sequence, solver_batch: Optional[Callable] = None, lcm_batch: Optional[Callable] = None):
+    """heuristic.py:20-40: every square matrix of `costs` goes through LCM (mask 100, every value summed, :24-33) and
+    through the exact solver (:37).  Returns [(lcm_total, optimum)] per case; optimum <= lcm_total always holds (:40).
+    solver_batch(costs) -> [(col_of_row, objective)] and lcm_batch(costs) -> [LCM dict] are injectable (tests feed
+    oracles).  Without them the batch is uploaded once and both batched kernels run on the same packed buffer."""
+    if solver_batch is None and lcm_batch is None:
+        from . import dispatch
+        opt, lcm = dispatch.run_batch(costs, assign=True, lcm=dict(mask_value=100))
+    else:
+        if solver_batch is None or lcm_batch is None:
+            from . import dispatch
+            solver_batch = solver_batch or dispatch.solve_batch
+            lcm_batch = lcm_batch or (lambda cs: dispatch.LCM_batch(cs, mask_value=100))
+        opt, lcm = solver_batch(costs), lcm_batch(costs)
+    return [(int(l["total"]), int(o[1])) for l, o in zip(lcm, opt)]
