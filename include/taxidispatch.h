@@ -265,6 +265,31 @@ int td_pool_pairs(const int32_t *from, const int32_t *to, int n, const int32_t *
                   int32_t *pairs_out /* cap x 4 */, int32_t cap, int32_t *n_pairs_out /* 1 */,
                   void *workspace, size_t workspace_bytes, void *stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Exact 2-passenger pool, batched: minimum-cost maximum-cardinality pair matching
+ * (the optimum pool_optimum.py / pool_opt_min.py ask for; greedy counterpart: td_pool_pairs)
+ *
+ * Instance b has sizes[b] customers at from[offsets[b]..], to[offsets[b]..] (from < 0: removed row); the stand
+ * table dist (n_stands x n_stands, n_stands <= 128, every entry in [0, 2^22]) is shared by the whole batch.  The
+ * pair {i, j} is an edge when td_pool_pairs would accept (i, j) or (j, i); its row [custA, custB, plan, cost] is the
+ * accepted candidate smallest in (cost, A*n+B).  Among the matchings of maximum cardinality, one of minimum total
+ * cost is returned: pairs_out[b] holds its rows in (cost, A*n+B) order (n_max/2 rows per instance, unused rows -1),
+ * n_pairs_out[b] their count and cost_out[b] their total.  Which optimum comes back when several exist is not
+ * specified, but it depends on nothing but the instance: not on its position, its neighbours or n_max.
+ *
+ * One CTA per instance, one launch.  An instance with sizes[b] < 0 or > n_max, offsets[b] < 0 or a live row whose
+ * stand lies outside the table is withdrawn (n_pairs -1, cost INT64_MIN, rows -1); a table entry outside
+ * [0, 2^22] withdraws every instance.  The arguments are checked before anything else: TD_ERR_INVALID for batch < 0,
+ * n_max outside [0, TD_PAIRS_EXACT_MAX_N], a bad n_stands, a non-finite max_loss with accept_all == 0 or a NULL
+ * pointer with batch > 0; TD_ERR_WORKSPACE for a workspace smaller than td_pool_pairs_exact_workspace_bytes.
+ * ------------------------------------------------------------------------------------------ */
+#define TD_PAIRS_EXACT_MAX_N 4096
+size_t td_pool_pairs_exact_workspace_bytes(int batch, int n_max);
+int td_pool_pairs_exact_batch(const int32_t *from, const int32_t *to, const int32_t *sizes, const int64_t *offsets,
+                              int batch, int n_max, const int32_t *dist, int n_stands, int accept_all, double max_loss,
+                              int32_t *pairs_out /* batch x (n_max/2) x 4 */, int32_t *n_pairs_out /* batch */,
+                              int64_t *cost_out /* batch */, void *workspace, size_t workspace_bytes, void *stream);
+
 /* After an ASYNCHRONOUS td_pool_find / td_pool_find_shards call (stats == NULL) on `workspace`: waits for the
  * stream and reads the per-shard counters back (one small copy).  *overflow_out != 0: the record list was too
  * small for a single pass -- counts_out holds -1 and the call has to be repeated synchronously (stats != NULL),
@@ -319,6 +344,10 @@ int tdh_assign_exact_rect(const int32_t *cost, int n, int n_real_rows, int n_rea
 int tdh_pool_find(const int32_t *demand, int n, const int32_t *dist, int n_stands, int pool_size,
                   int shard, int n_shards, int32_t *plans_out, int32_t cap, int32_t *n_plans_out,
                   td_pool_stats *stats);
+/* one instance of td_pool_pairs_exact_batch (what a JNI binding of Simulator.findPool calls); pairs_out holds n/2
+ * rows; a live row with a stand outside the table, or a table entry outside [0, 2^22], is TD_ERR_INVALID here */
+int tdh_pool_pairs_exact(const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
+                         int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out);
 /* all n_shards logical shards + merge, i.e. what `findpool` produces (findpool.c:122-176) */
 int tdh_pool_find_all(const int32_t *demand, int n, const int32_t *dist, int n_stands, int pool_size,
                       int n_shards, int32_t *plans_out, int32_t cap, int32_t *n_plans_out,

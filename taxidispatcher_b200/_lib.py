@@ -17,6 +17,7 @@ TD_ERR_NO_DEVICE = -5
 TD_ERR_NOT_CONVERGED = -6
 INT32_MAX = 2**31 - 1
 BIG_COST = 250000
+PAIRS_EXACT_MAX_N = 4096    # TD_PAIRS_EXACT_MAX_N
 POOL_REC_W = 9
 PROF_COST, PROF_LCM, PROF_ASSIGN, PROF_POOL_ENUM, PROF_POOL_SELECT = range(5)
 
@@ -92,6 +93,10 @@ _SIGNATURES = {
     "td_pool_merge_workspace_bytes": (ctypes.c_size_t, [_I, _I]),
     "td_pool_merge": (_I, [c_vp, _I, _I, _I, c_vp, c_vp, c_vp, ctypes.c_size_t, c_vp]),
     "td_pool_merge_padded": (_I, [c_vp, c_vp, c_vp, _I, _I, _I, _I, c_vp, c_vp, c_vp, ctypes.c_size_t, c_vp]),
+    "td_pool_pairs_exact_workspace_bytes": (ctypes.c_size_t, [_I, _I]),
+    "td_pool_pairs_exact_batch": (_I, [c_vp, c_vp, c_vp, c_vp, _I, _I, c_vp, _I, _I, ctypes.c_double, c_vp, c_vp, c_vp, c_vp,
+                                       ctypes.c_size_t, c_vp]),
+    "tdh_pool_pairs_exact": (_I, [c_vp, c_vp, _I, c_vp, _I, _I, ctypes.c_double, c_vp, c_vp, c_vp]),
     "tdh_cost_matrix": (_I, [c_vp, _I, c_vp, _I, c_vp, _I, ctypes.c_int32, ctypes.c_int32, c_vp]),
     "tdh_lcm": (_I, [c_vp, _I, ctypes.POINTER(LcmParams), c_vp, c_vp, c_vp, c_vp, c_vp]),
     "tdh_assign_exact": (_I, [c_vp, _I, c_vp, c_vp, c_vp, ctypes.POINTER(AssignStats)]),

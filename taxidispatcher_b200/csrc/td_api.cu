@@ -1,6 +1,7 @@
 // td_api.cu -- library plumbing (version, errors, device probe, launch counter) and the
 // host-buffer twins tdh_* of the device entry points.
 #include "td_common.cuh"
+#include <cmath>
 #include <stdio.h>
 #include <string.h>
 #include <string>
@@ -231,6 +232,41 @@ extern "C" int tdh_pool_find(const int32_t *demand, int n, const int32_t *dist, 
     int m = *n_plans_out < cap ? *n_plans_out : cap;
     if (m > 0) TDH_TRY(cudaMemcpy(plans_out, d_plans.p, size_t(m) * TD_POOL_REC_W * 4, cudaMemcpyDeviceToHost));
     return *n_plans_out > cap ? TD_ERR_CAPACITY : TD_OK;
+}
+
+extern "C" int tdh_pool_pairs_exact(const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
+                                    int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out) {
+    if (n < 0 || n > TD_PAIRS_EXACT_MAX_N || n_stands < 1 || n_stands > 128 || !n_pairs_out || !cost_out) return TD_ERR_INVALID;
+    if (!accept_all && !std::isfinite(max_loss)) return TD_ERR_INVALID;
+    if (n > 0 && (!from || !to)) return TD_ERR_INVALID;
+    if (!dist || (n >= 2 && !pairs_out)) return TD_ERR_INVALID;
+    for (int k = 0; k < n_stands * n_stands; ++k) if (dist[k] < 0 || dist[k] > (1 << 22)) return TD_ERR_INVALID;
+    for (int i = 0; i < n; ++i) if (from[i] >= 0 && (from[i] >= n_stands || to[i] < 0 || to[i] >= n_stands)) return TD_ERR_INVALID;
+    if (!td::have_device()) return TD_ERR_NO_DEVICE;
+    td::DevBuf d_in, d_out, d_ws;
+    const size_t nn = size_t(n > 0 ? n : 1), words = 2 * nn + 2 + 2 + size_t(n_stands) * n_stands;   // from, to, size, offset, dist
+    TDH_TRY(d_in.alloc(words * 4));
+    std::vector<int32_t> h(words, 0);
+    if (n) { memcpy(h.data(), from, size_t(n) * 4); memcpy(h.data() + nn, to, size_t(n) * 4); }
+    h[2 * nn] = n;                                                     // size; the offset (int64 0) follows at an 8-byte boundary
+    const size_t off_at = (2 * nn + 1 + 1) & ~size_t(1), dist_at = off_at + 2;
+    memcpy(h.data() + dist_at, dist, size_t(n_stands) * n_stands * 4);
+    TDH_TRY(cudaMemcpy(d_in.p, h.data(), words * 4, cudaMemcpyHostToDevice));
+    const int rows = n / 2;
+    const size_t out_bytes = 16 + size_t(rows > 0 ? rows : 1) * 16;   // cost (8), count (4), pad, rows
+    TDH_TRY(d_out.alloc(out_bytes));
+    const size_t wsb = td_pool_pairs_exact_workspace_bytes(1, n);
+    TDH_TRY(d_ws.alloc(wsb));
+    int32_t *in = d_in.as<int32_t>();
+    char *out = d_out.as<char>();
+    TDH_RC(td_pool_pairs_exact_batch(in, in + nn, in + 2 * nn, reinterpret_cast<const int64_t *>(in + off_at), 1, n, in + dist_at,
+                                     n_stands, accept_all, max_loss, reinterpret_cast<int32_t *>(out + 16),
+                                     reinterpret_cast<int32_t *>(out + 8), reinterpret_cast<int64_t *>(out), d_ws.p, wsb, nullptr));
+    std::vector<char> host(out_bytes);
+    TDH_TRY(cudaMemcpy(host.data(), out, out_bytes, cudaMemcpyDeviceToHost));
+    memcpy(cost_out, host.data(), 8); memcpy(n_pairs_out, host.data() + 8, 4);
+    if (*n_pairs_out > 0) memcpy(pairs_out, host.data() + 16, size_t(*n_pairs_out) * 16);
+    return TD_OK;
 }
 
 extern "C" int tdh_pool_find_all(const int32_t *demand, int n, const int32_t *dist, int n_stands, int pool_size,

@@ -11,6 +11,7 @@ Host functions mirror the reference's names, argument order and return layouts
   LCM_java(cost)                                   Simulator.java:523-549
   solve_batch(costs) / LCM_batch(costs, ...)       heuristic.py:20-40, python.py:6-25 over many instances
   find_pool(...) / find_pool_all(...) / pool_merge(...)   pool_n.c / findpool.c
+  find_pool_pairs_exact(...) / find_pool_pairs_exact_batch(...)   the optimum of pool_optimum.py / pool_opt_min.py
 
 PyTorch is used only for device buffers, pinned staging and streams.  All arithmetic runs in the
 hand-written CUDA kernels behind the C ABI (include/taxidispatch.h).  There is no CPU fallback:
@@ -26,11 +27,11 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import BIG_COST, INT32_MAX, POOL_REC_W, AssignStats, LcmParams, PoolStats, TaxiDispatchError, check
+from ._lib import BIG_COST, INT32_MAX, PAIRS_EXACT_MAX_N, POOL_REC_W, AssignStats, LcmParams, PoolStats, TaxiDispatchError, check
 
 __all__ = ["BIG_COST", "Engine", "calculate_cost", "solve", "solve_dispatch", "solve_full", "solve_assignment", "LCM", "LCM_heuristic",
            "LCM_split", "LCM_greedy_opt", "LCM_simulate", "LCM_java", "find_pool", "find_pool_all", "find_pool_block",
-           "find_pool_pairs", "pool_merge", "pack_batch", "run_batch", "solve_batch", "LCM_batch",
+           "find_pool_pairs", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "pool_merge", "pack_batch", "run_batch", "solve_batch", "LCM_batch",
            "TaxiDispatchError"]
 
 
@@ -481,6 +482,24 @@ class Engine:
         check(rc, "td_pool_pairs")
         return out, cnt
 
+    def pool_pairs_exact_batch(self, frm: torch.Tensor, to: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor,
+                               n_max: int, dist: torch.Tensor, accept_all: bool = True, max_loss: float = 1.01,
+                               out: Optional[dict] = None):
+        """Minimum-cost maximum-cardinality pair matching of every instance (customers sizes[b] at frm / to[offsets[b]:]),
+        one launch.  Returns device tensors (rows [B, n_max // 2, 4] int32 = custA, custB, plan, cost in (cost, A*n+B)
+        order, n_pairs [B] int32, cost [B] int64); a withdrawn instance has n_pairs -1.  `out` may supply any of them by
+        name ("rows", "n_pairs", "cost")."""
+        B = int(sizes.numel())
+        rows = self._batch_out(out, "rows", (B, n_max // 2, 4), torch.int32)
+        npairs = self._batch_out(out, "n_pairs", (B,), torch.int32)
+        cost = self._batch_out(out, "cost", (B,), torch.int64)
+        ws = self._workspace("pairs_exact", self.lib.td_pool_pairs_exact_workspace_bytes(B, int(n_max)))
+        rc = self.lib.td_pool_pairs_exact_batch(_ptr(frm), _ptr(to), _ptr(sizes), _ptr(offsets), B, int(n_max), _ptr(dist),
+                                                int(dist.shape[0]), 1 if accept_all else 0, float(max_loss), _ptr(rows),
+                                                _ptr(npairs), _ptr(cost), _ptr(ws), ws.numel(), _stream())
+        check(rc, "td_pool_pairs_exact_batch")
+        return rows, npairs, cost
+
     def pool_merge(self, shard_plans: torch.Tensor, total: int, n: int, pool_size: int):
         out = torch.empty((max(total, 1), POOL_REC_W), dtype=torch.int32, device=self.device)
         cnt = torch.zeros(1, dtype=torch.int32, device=self.device)
@@ -772,6 +791,84 @@ def find_pool_pairs(frm, to, dist, accept_all: bool = True, max_loss: float = 1.
     eng = engine()
     out, cnt = eng.pool_pairs(_h2d_i32(frm), _h2d_i32(to), _h2d_i32(dist), accept_all, max_loss)
     return out[: int(cnt.item())].cpu().numpy()
+
+
+def pack_pairs_batch(instances: Sequence, dist):
+    """[(frm, to)] host arrays + the stand table -> (frm, to, sizes, offsets, n_max, dist) on the device for
+    Engine.pool_pairs_exact_batch.  Every part travels in ONE pinned buffer and ONE host->device copy."""
+    fr = [np.asarray(f, dtype=np.int32).reshape(-1) for f, _ in instances]
+    tt = [np.asarray(t, dtype=np.int32).reshape(-1) for _, t in instances]
+    for f, t in zip(fr, tt):
+        if f.shape != t.shape:
+            raise ValueError("frm and to of an instance differ in length")
+    d = np.ascontiguousarray(np.asarray(dist, dtype=np.int32))
+    B = len(fr)
+    sizes = np.array([len(f) for f in fr], dtype=np.int32)
+    offsets = np.zeros(B, dtype=np.int64)
+    total = 0
+    for b, f in enumerate(fr):
+        offsets[b] = total
+        total += (len(f) + 3) & ~3
+    to_at = total
+    meta = 2 * total
+    off_at = (meta + B + 1) & ~1                          # int64 view: even int32 index
+    dist_at = (off_at + 2 * B + 3) & ~3
+    words = max(dist_at + d.size, 4)
+    COPIED["h2d"] += words * 4
+    bucket = 1 << max(8, int(words - 1).bit_length())
+    key = ("pairs", bucket)
+    slot = _PINNED.get(key) if bucket <= (1 << 24) else None
+    if slot is None:
+        slot = {"buf": torch.empty(bucket, dtype=torch.int32).pin_memory(), "ev": None}
+        if bucket <= (1 << 24):
+            _PINNED[key] = slot
+    if slot["ev"] is not None:
+        slot["ev"].synchronize()
+    host = slot["buf"].numpy()
+    for f, t, o in zip(fr, tt, offsets):
+        host[o: o + len(f)] = f
+        host[to_at + o: to_at + o + len(t)] = t
+    host[meta: meta + B] = sizes
+    host[off_at: off_at + 2 * B] = offsets.view(np.int32)
+    host[dist_at: dist_at + d.size] = d.reshape(-1)
+    dev = slot["buf"][:words].to("cuda", non_blocking=True)
+    ev = torch.cuda.Event()
+    ev.record()
+    slot["ev"] = ev
+    n_max = int(sizes.max()) if B else 0
+    return (dev[:max(total, 1)], dev[to_at: to_at + max(total, 1)], dev[meta: meta + B],
+            dev[off_at: off_at + 2 * B].view(torch.int64), n_max, dev[dist_at: dist_at + d.size].reshape(d.shape))
+
+
+def find_pool_pairs_exact_batch(instances: Sequence, dist, accept_all: bool = True, max_loss: float = 1.01):
+    """The exact 2-passenger pool of every (frm, to) instance over one stand table: one pinned upload, one launch and one
+    read-back.  Returns per instance the rows (custA, custB, plan, cost) of a minimum-cost maximum-cardinality pairing
+    in (cost, A*n+B) order -- the layout find_pool_pairs returns -- or None for an instance the library withdrew (a
+    live row whose stand lies outside the table)."""
+    B = len(instances)
+    if B == 0:
+        return []
+    eng = engine()
+    frm, to, sizes, offsets, n_max, d = pack_pairs_batch(instances, dist)
+    if n_max > PAIRS_EXACT_MAX_N:
+        raise ValueError("an instance has %d customers; the exact pool takes at most %d" % (n_max, PAIRS_EXACT_MAX_N))
+    cap = n_max // 2
+    arena = _Arena(eng.device, [(B * cap * 4, torch.int32), (B, torch.int32), (B, torch.int64)])
+    rows_v, np_v, cost_v = arena.views
+    eng.pool_pairs_exact_batch(frm, to, sizes, offsets, n_max, d, accept_all, max_loss,
+                               out={"rows": rows_v.view(B, cap, 4), "n_pairs": np_v, "cost": cost_v})
+    rows, npairs, _ = arena.host()                                 # the one read-back of the batch
+    rows = rows.reshape(B, cap, 4)
+    return [None if npairs[b] < 0 else rows[b, : int(npairs[b])].copy() for b in range(B)]
+
+
+def find_pool_pairs_exact(frm, to, dist, accept_all: bool = True, max_loss: float = 1.01):
+    """The exact counterpart of find_pool_pairs: rows (custA, custB, plan, cost) of a maximum-cardinality pairing of
+    minimum total cost, in (cost, A*n+B) order; custA / custB are positions in the given arrays (from < 0: removed)."""
+    r = find_pool_pairs_exact_batch([(frm, to)], dist, accept_all, max_loss)[0]
+    if r is None:
+        raise TaxiDispatchError(_lib.TD_ERR_INVALID, "find_pool_pairs_exact", "a live customer's stand lies outside the table")
+    return r
 
 
 def pool_merge(shard_plans, n: int, pool_size: int):

@@ -5,6 +5,7 @@
                                        last solve over the customers and cabs the ranges left unserved
   greedy_then_solve  greedy_opt.py:131-163   LCM prefix with a distance threshold, exact solve on the rest
   lcm_vs_optimum     heuristic.py:20-40      LCM (mask 100) against the exact optimum on many small instances
+  pool_greedy_vs_optimum  pool_opt_min.py      the Simulator's greedy 2-passenger pool against the optimal pairing
 
 Every range of solve_split is an independent K1 + K2 instance: with a process group the ranges are spread
 over the ranks (parallel.instances_for_rank), the unserved ids are gathered, and the leftover solve runs
@@ -209,3 +210,23 @@ def lcm_vs_optimum(costs: Sequence, solver_batch: Optional[Callable] = None, lcm
             lcm_batch = lcm_batch or (lambda cs: dispatch.LCM_batch(cs, mask_value=100))
         opt, lcm = solver_batch(costs), lcm_batch(costs)
     return [(int(l["total"]), int(o[1])) for l, o in zip(lcm, opt)]
+
+
+def pool_greedy_vs_optimum(instances: Sequence, dist, accept_all: bool = True, max_loss: float = 1.01,
+                           greedy: Optional[Callable] = None, exact: Optional[Callable] = None):
+    """pool_opt_min.py: every (frm, to) instance of `instances` is pooled by the Simulator's greedy scan
+    (Simulator.java:681-758) and by the optimal pairing (minimum cost among the pairings of maximum cardinality, the
+    reference's ILP where it is feasible).  Returns [(greedy_count, greedy_cost, opt_count, opt_cost)] per case;
+    opt_count >= greedy_count, and opt_cost <= greedy_cost where the counts are equal.  greedy(frm, to, dist, accept_all,
+    max_loss) and exact(instances, dist, accept_all, max_loss) -> row arrays are injectable (tests feed oracles); without
+    them the greedy runs per instance and the exact pool is one batched launch."""
+    from . import dispatch
+    greedy = greedy or dispatch.find_pool_pairs
+    exact = exact or dispatch.find_pool_pairs_exact_batch
+    opt = exact(instances, dist, accept_all, max_loss)
+    out = []
+    for (f, t), o in zip(instances, opt):
+        g = greedy(f, t, dist, accept_all, max_loss) if len(f) >= 2 else np.zeros((0, 4), np.int32)
+        g, o = np.asarray(g).reshape(-1, 4), np.asarray(o).reshape(-1, 4)
+        out.append((len(g), int(g[:, 3].astype(np.int64).sum()), len(o), int(o[:, 3].astype(np.int64).sum())))
+    return out

@@ -37,9 +37,11 @@ ID, FROM, TO, CLNT_ASSIGNED, CLNT_ON_BOARD, TIME_STARTED = range(6)
 
 class CudaBackend:
     """The product backend: every primitive runs in libtaxidispatch.so on the GPU.  The cost matrix stays on the
-    device between K1 and the LCM / exact solve that consume it (the host copy is only read by the state machine)."""
+    device between K1 and the LCM / exact solve that consume it (the host copy is only read by the state machine).
+    exact_pool=True pools each step's customers by the optimal pairing (find_pool_pairs_exact) instead of the greedy
+    scan of Simulator.findPool; the default keeps the reference's greedy."""
 
-    def __init__(self):
+    def __init__(self, exact_pool: bool = False):
         import torch
         from . import dispatch
         self.d = dispatch
@@ -50,6 +52,7 @@ class CudaBackend:
         self._dist_dev = None      # (host stand table, device copy): the table does not change during a replay
         self._pin = [None, None]   # two pinned read-back buffers, used alternately (a step holds at most two cost matrices)
         self._pin_i = 0
+        self.exact_pool = exact_pool
 
     def _read_back(self, dev):
         """Device int32 tensor -> numpy through a reused pinned buffer (a 1300 x 1300 matrix per step: pageable read-backs
@@ -70,7 +73,8 @@ class CudaBackend:
 
     def pool_pairs(self, frm, to, dist):
         t0 = time.perf_counter()
-        r = self.d.find_pool_pairs(frm, to, dist, accept_all=True, max_loss=MAX_LOSS)   # Simulator.java:691
+        find = self.d.find_pool_pairs_exact if self.exact_pool else self.d.find_pool_pairs
+        r = find(frm, to, dist, accept_all=True, max_loss=MAX_LOSS)   # Simulator.java:691
         self.times["pool"] += time.perf_counter() - t0
         return r
 
