@@ -210,7 +210,35 @@ int td_lcm_batch(const int32_t *costs, const int32_t *sizes, const int64_t *offs
                  int32_t *last_min_out /* batch, may be NULL */, void *stream);
 
 /* ------------------------------------------------------------------------------------------
- * K4  pool finder            replaces one `pool_n <pool-size> <thread> <file> <n> <out>` process
+ * Batches of mid-size instances (n <= TD_BATCH_CLUSTER_MAX_N)   the paper's 400 x 400 split /
+ *     hybrid experiment (split.py:186-212, greedy_opt.py:129-163) and Simulator.java's
+ *     MAX_NON_LCM = 600 solver limit, over many instances.
+ *
+ * Exactly the arguments, layout and semantics of td_assign_exact_batch / td_lcm_batch above
+ * (packed instances, output stride n_max, -1 / 0 fill, withdrawal of an instance with a bad size or
+ * offset, batch == 0 launches nothing), for n_max up to 640.  One launch per call; every instance
+ * runs on one thread-block cluster of K CTAs (K = 1, 2, 4 or 8, the smallest whose share of the
+ * matrix fits one CTA's shared memory; it depends on n_max only) that holds the instance in its
+ * distributed shared memory.  Returns TD_ERR_CUDA when no such cluster fits the device.
+ *
+ * td_assign_exact_batch_cluster runs the algorithm of td_assign_exact_batch step for step: for
+ * every n <= 232 it returns the identical col_of_row, u, v and objective, and for any n the result
+ * does not depend on n_max or on the instance's position in the batch.  td_lcm_batch_cluster
+ * returns the literal trace of td_lcm for every params.
+ * ------------------------------------------------------------------------------------------ */
+#define TD_BATCH_CLUSTER_MAX_N 640   /* 8 CTAs x (640/8) x 640 x 4 B = 8 x 200 KB of shared memory */
+int td_assign_exact_batch_cluster(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                                  int32_t *col_of_row_out /* batch x n_max */, int64_t *objective_out /* batch */,
+                                  int64_t *u_out /* batch x n_max or NULL */, int64_t *v_out /* batch x n_max or NULL */,
+                                  void *stream);
+int td_lcm_batch_cluster(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                         const td_lcm_params *params /* host, same for every instance */,
+                         int32_t *rows_out /* batch x n_max */, int32_t *cols_out /* batch x n_max */,
+                         int32_t *n_pairs_out /* batch */, int64_t *total_out /* batch */,
+                         int32_t *last_min_out /* batch, may be NULL */, void *stream);
+
+/* ------------------------------------------------------------------------------------------
+ * K4  pool finder           replaces one `pool_n <pool-size> <thread> <file> <n> <out>` process
  *     (pool_n.c:209-238): findPool :153-177, drop_customers :101-151, removeDuplicates :187-207,
  *     shard rule :226-229.
  *

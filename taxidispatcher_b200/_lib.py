@@ -77,6 +77,8 @@ _SIGNATURES = {
     "td_assign_certify": (_I, [c_vp, _I, _I, _I, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_size_t, c_vp]),
     "td_assign_exact_batch": (_I, [c_vp, c_vp, c_vp, _I, _I, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "td_lcm_batch": (_I, [c_vp, c_vp, c_vp, _I, _I, ctypes.POINTER(LcmParams), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "td_assign_exact_batch_cluster": (_I, [c_vp, c_vp, c_vp, _I, _I, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "td_lcm_batch_cluster": (_I, [c_vp, c_vp, c_vp, _I, _I, ctypes.POINTER(LcmParams), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "td_pool_workspace_bytes":(ctypes.c_size_t, [_I, _I, _I, ctypes.c_int64]),
     "td_pool_find": (_I, [c_vp, _I, c_vp, _I, _I, _I, _I, c_vp, ctypes.c_int32, c_vp, ctypes.POINTER(PoolStats),
                           c_vp, ctypes.c_size_t, ctypes.c_int64, c_vp]),

@@ -31,7 +31,7 @@ from ._lib import BIG_COST, INT32_MAX, PAIRS_EXACT_MAX_N, POOL_REC_W, AssignStat
 
 __all__ = ["BIG_COST", "Engine", "calculate_cost", "solve", "solve_dispatch", "solve_full", "solve_assignment", "LCM", "LCM_heuristic",
            "LCM_split", "LCM_greedy_opt", "LCM_simulate", "LCM_java", "find_pool", "find_pool_all", "find_pool_block",
-           "find_pool_pairs", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "pool_merge", "pack_batch", "run_batch", "solve_batch", "LCM_batch",
+           "find_pool_pairs", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "pool_merge", "pack_batch", "pack_cost_matrices", "run_packed", "run_batch", "solve_batch", "LCM_batch",
            "TaxiDispatchError"]
 
 
@@ -120,6 +120,13 @@ def _h2d_i32_many(arrays) -> list:
 
 
 BATCH_MAX_N = 232   # TD_BATCH_MAX_N: the largest instance the batched kernels hold in one CTA's shared memory
+BATCH_CLUSTER_MAX_N = 640   # TD_BATCH_CLUSTER_MAX_N: the largest instance one 8-CTA cluster holds in its shared memory
+# run_batch sends the LCMs of fewer mid-size instances than this through single td_lcm calls.  One cluster LCM pays about
+# 2 us of cluster barrier and reductions per iteration (1.2 ms for a 600 x 600 instance, flat up to many instances per
+# launch), while a single td_lcm call takes 0.39 ms at 600 x 600.  Measured on one NVIDIA B200 at 1000 W
+# (profiles/cluster_batch_b200.json): at 600 x 600 the loop wins up to 3 instances (1.11 against 1.20 ms) and the cluster
+# from 4 (1.21 against 1.51 ms); at 240 x 240 both take 0.4 ms for 3.  The cluster assignment wins from one instance on.
+LCM_CLUSTER_MIN_BATCH = 4
 
 
 def pack_batch(costs: Sequence):
@@ -295,33 +302,44 @@ class Engine:
                           c.dual_objective == c.matched_real_cost)
         return out
 
-    # -- batches of small instances (td_assign_exact_batch / td_lcm_batch) -------------------------
+    # -- batches (td_assign_exact_batch / td_lcm_batch up to 232, the *_cluster kernels up to 640) ------
     def _batch_out(self, out, name, shape, dtype):
         if out is not None and out.get(name) is not None:
             return out[name]
         return torch.empty(shape, dtype=dtype, device=self.device)
 
+    @staticmethod
+    def _batch_kernel(n_max: int, name: str) -> str:
+        """One CTA per instance up to BATCH_MAX_N, one thread-block cluster per instance up to BATCH_CLUSTER_MAX_N."""
+        if n_max <= BATCH_MAX_N:
+            return name
+        if n_max <= BATCH_CLUSTER_MAX_N:
+            return name + "_cluster"
+        raise ValueError("batched %s holds instances up to %d rows, got n_max %d" % (name, BATCH_CLUSTER_MAX_N, n_max))
+
     def assign_batch(self, packed: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor, n_max: int,
                      want_duals: bool = False, out: Optional[dict] = None):
-        """Exact optimum of every instance of a pack_batch() buffer, one launch.  Returns device tensors
-        (col [B, n_max] int32, objective [B] int64, u, v) -- u / v are [B, n_max] int64 potentials or None.
-        `out` may supply any of them by name ("col", "objective", "u", "v")."""
+        """Exact optimum of every instance of a pack_batch() buffer, one launch (n_max <= BATCH_CLUSTER_MAX_N).  Returns
+        device tensors (col [B, n_max] int32, objective [B] int64, u, v) -- u / v are [B, n_max] int64 potentials or
+        None.  `out` may supply any of them by name ("col", "objective", "u", "v")."""
+        name = self._batch_kernel(int(n_max), "td_assign_exact_batch")
         B = int(sizes.numel())
         col = self._batch_out(out, "col", (B, n_max), torch.int32)
         obj = self._batch_out(out, "objective", (B,), torch.int64)
         u = self._batch_out(out, "u", (B, n_max), torch.int64) if want_duals else None
         v = self._batch_out(out, "v", (B, n_max), torch.int64) if want_duals else None
-        rc = self.lib.td_assign_exact_batch(_ptr(packed), _ptr(sizes), _ptr(offsets), B, int(n_max), _ptr(col), _ptr(obj),
-                                            _ptr(u), _ptr(v), _stream())
-        check(rc, "td_assign_exact_batch")
+        rc = getattr(self.lib, name)(_ptr(packed), _ptr(sizes), _ptr(offsets), B, int(n_max), _ptr(col), _ptr(obj),
+                                     _ptr(u), _ptr(v), _stream())
+        check(rc, name)
         return col, obj, u, v
 
     def lcm_batch(self, packed: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor, n_max: int, mask_value: int,
                   stop_above: int = INT32_MAX, stop_at_value: int = INT32_MAX, sum_below: int = INT32_MAX,
                   residual_size: int = 0, max_iters: int = -1, out: Optional[dict] = None):
-        """LCM of every instance of a pack_batch() buffer, one launch, the same params for all.  Returns device tensors
-        (rows [B, n_max], cols [B, n_max], n_pairs [B] int32, total [B] int64, last_min [B] int32); `out` may supply
-        any of them by name."""
+        """LCM of every instance of a pack_batch() buffer, one launch, the same params for all (n_max <=
+        BATCH_CLUSTER_MAX_N).  Returns device tensors (rows [B, n_max], cols [B, n_max], n_pairs [B] int32, total [B]
+        int64, last_min [B] int32); `out` may supply any of them by name."""
+        name = self._batch_kernel(int(n_max), "td_lcm_batch")
         B = int(sizes.numel())
         rows = self._batch_out(out, "rows", (B, n_max), torch.int32)
         cols = self._batch_out(out, "cols", (B, n_max), torch.int32)
@@ -330,9 +348,9 @@ class Engine:
         last = self._batch_out(out, "last_min", (B,), torch.int32)
         prm = LcmParams(int(mask_value), int(stop_above), int(stop_at_value), int(sum_below), int(residual_size),
                         int(max_iters))
-        rc = self.lib.td_lcm_batch(_ptr(packed), _ptr(sizes), _ptr(offsets), B, int(n_max), ctypes.byref(prm), _ptr(rows),
-                                   _ptr(cols), _ptr(npairs), _ptr(total), _ptr(last), _stream())
-        check(rc, "td_lcm_batch")
+        rc = getattr(self.lib, name)(_ptr(packed), _ptr(sizes), _ptr(offsets), B, int(n_max), ctypes.byref(prm), _ptr(rows),
+                                     _ptr(cols), _ptr(npairs), _ptr(total), _ptr(last), _stream())
+        check(rc, name)
         return rows, cols, npairs, total, last
 
     # -- K4 ---------------------------------------------------------------------------------------
@@ -640,63 +658,136 @@ def _lcm_params(mask_value, stop_above, stop_at_value, sum_below, residual_size,
                 residual_size=residual_size, max_iters=max_iters)
 
 
+def run_packed(packed: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor, n_max: int, ns: Sequence[int],
+               assign: bool = True, want_duals: bool = False, lcm: Optional[dict] = None):
+    """The launch and read-back half of run_batch for a packed buffer already on the device (pack_batch,
+    pack_cost_matrices): one launch per kernel, both reading the same buffer, and one device->host copy.  ns are the
+    instance sizes on the host (n_max <= BATCH_CLUSTER_MAX_N).  Returns (assign results, LCM results) as run_batch."""
+    eng = engine()
+    B = len(ns)
+    parts = []
+    if assign:
+        parts += [(B * n_max, torch.int32), (B, torch.int64)] + ([(B * n_max, torch.int64)] * 2 if want_duals else [])
+    if lcm is not None:
+        parts += [(B * n_max, torch.int32), (B * n_max, torch.int32), (B, torch.int32), (B, torch.int64), (B, torch.int32)]
+    arena = _Arena(eng.device, parts)
+    views = list(arena.views)
+    if assign:
+        names = ["col", "objective"] + (["u", "v"] if want_duals else [])
+        out = {k: views.pop(0) for k in names}
+        for k in ("col", "u", "v"):
+            if k in out:
+                out[k] = out[k].view(B, n_max)
+        eng.assign_batch(packed, sizes, offsets, n_max, want_duals=want_duals, out=out)
+    if lcm is not None:
+        out = {k: views.pop(0) for k in ("rows", "cols", "n_pairs", "total", "last_min")}
+        out["rows"], out["cols"] = out["rows"].view(B, n_max), out["cols"].view(B, n_max)
+        eng.lcm_batch(packed, sizes, offsets, n_max, out=out, **lcm)
+    host = arena.host()                                            # the one read-back of the batch
+    res_a = res_l = None
+    if assign:
+        col, obj = host.pop(0).reshape(B, n_max), host.pop(0)
+        u = host.pop(0).reshape(B, n_max) if want_duals else None
+        v = host.pop(0).reshape(B, n_max) if want_duals else None
+        res_a = []
+        for k, n in enumerate(ns):
+            r = (col[k, :n].copy(), int(obj[k]))
+            res_a.append(r + (u[k, :n].copy(), v[k, :n].copy()) if want_duals else r)
+    if lcm is not None:
+        rows, cols = host.pop(0).reshape(B, n_max), host.pop(0).reshape(B, n_max)
+        npairs, total, last = host.pop(0), host.pop(0), host.pop(0)
+        res_l = []
+        for k in range(B):
+            m = int(npairs[k])
+            res_l.append({"total": int(total[k]), "n_pairs": m, "rows": rows[k, :m].copy(), "cols": cols[k, :m].copy(),
+                          "last_min": int(last[k])})
+    return res_a, res_l
+
+
+def size_groups(ns: Sequence[int]):
+    """Positions of the instances per batched kernel: ([n <= BATCH_MAX_N], [BATCH_MAX_N < n <= BATCH_CLUSTER_MAX_N],
+    [larger])."""
+    small = [b for b, n in enumerate(ns) if n <= BATCH_MAX_N]
+    mid = [b for b, n in enumerate(ns) if BATCH_MAX_N < n <= BATCH_CLUSTER_MAX_N]
+    large = [b for b, n in enumerate(ns) if n > BATCH_CLUSTER_MAX_N]
+    return small, mid, large
+
+
+def pack_cost_matrices(dist_d: torch.Tensor, instances: Sequence, fill: int = BIG_COST, cutoff: Optional[int] = None,
+                       transpose: bool = False):
+    """calculate_cost (positional, square-padded with `fill`, optional cutoff) of every (cab_to, cust_from) pair of stand
+    index arrays, built by K1 straight into one packed device buffer in the layout of pack_batch: the n x n matrices
+    never cross PCIe.  transpose=True builds every matrix transposed (customer rows, cab columns; dist_d must then be the
+    transposed stand table).  The index arrays and the sizes / offsets travel in ONE host->device copy.  Returns
+    (packed, sizes, offsets, n_max, ns)."""
+    eng = engine()
+    cabs = [np.asarray(c, dtype=np.int32).reshape(-1) for c, _ in instances]
+    custs = [np.asarray(d, dtype=np.int32).reshape(-1) for _, d in instances]
+    ns = [max(len(c), len(d)) for c, d in zip(cabs, custs)]
+    B = len(ns)
+    offsets = np.zeros(B, dtype=np.int64)
+    total = 0
+    for b, n in enumerate(ns):
+        offsets[b] = total
+        total += (n * n + 3) & ~3
+    s = int(dist_d.shape[0]) if dist_d.numel() else 0
+    for c, d in zip(cabs, custs):
+        if len(c) and len(d) and (int(c.max()) >= s or int(c.min()) < 0 or int(d.max()) >= s or int(d.min()) < 0):
+            raise IndexError("stand index out of range of the distance table")   # as calculate_cost
+    idx = np.concatenate(cabs + custs + [np.zeros(1, np.int32)])
+    off_at = (B + 1) & ~1                                 # offsets at an even int32 index (int64 view)
+    meta = np.zeros(off_at + 2 * B + 1, dtype=np.int32)
+    meta[:B] = ns
+    meta[off_at: off_at + 2 * B] = offsets.view(np.int32)
+    idx_d, meta_d = _h2d_i32_many([idx, meta])
+    packed = torch.empty(max(total, 4), dtype=torch.int32, device=eng.device)
+    pos = [0]
+    for a in cabs + custs:
+        pos.append(pos[-1] + len(a))
+    for b, n in enumerate(ns):
+        if n == 0:
+            continue
+        cab_d = idx_d[pos[b]: pos[b + 1]]
+        cust_d = idx_d[pos[B + b]: pos[B + b + 1]]
+        rows, cols = (cust_d, cab_d) if transpose else (cab_d, cust_d)
+        eng.cost_matrix(dist_d, rows, cols, fill, cutoff, out=packed[int(offsets[b]): int(offsets[b]) + n * n].view(n, n))
+    return packed, meta_d[:B], meta_d[off_at: off_at + 2 * B].view(torch.int64), (max(ns) if B else 0), ns
+
+
 def run_batch(costs: Sequence, assign: bool = True, want_duals: bool = False, lcm: Optional[dict] = None):
-    """Exact assignment and / or LCM (`lcm` = its keyword parameters) of every square matrix in `costs`.  Instances up to
-    BATCH_MAX_N are uploaded once and served by one launch per kernel, both kernels reading the same packed buffer, and
-    come back in one device->host copy; larger ones take the single-instance path.  Returns (assign results, LCM
+    """Exact assignment and / or LCM (`lcm` = its keyword parameters) of every square matrix in `costs`.  The instances
+    are grouped by size: up to BATCH_MAX_N (one CTA each) and up to BATCH_CLUSTER_MAX_N (one thread-block cluster each),
+    every group uploaded once and served by one launch per kernel, both kernels reading the same packed buffer, and
+    read back in one device->host copy; larger ones take the single-instance path.  Returns (assign results, LCM
     results): lists of (col_of_row, objective[, u, v]) and of LCM() dicts, None for the side not asked for."""
     mats = [np.asarray(c) for c in costs]
-    fits = [a.ndim == 2 and a.shape[0] <= BATCH_MAX_N for a in mats]
-    small = [b for b, f in enumerate(fits) if f]
-    large = [b for b, f in enumerate(fits) if not f]
-    res_a = [None] * len(mats) if assign else None
-    res_l = [None] * len(mats) if lcm is not None else None
-    if small:
-        eng = engine()
-        packed, sizes, offsets, n_max = pack_batch([mats[b] for b in small])
-        B = len(small)
-        parts = []
-        if assign:
-            parts += [(B * n_max, torch.int32), (B, torch.int64)] + ([(B * n_max, torch.int64)] * 2 if want_duals else [])
-        if lcm is not None:
-            parts += [(B * n_max, torch.int32), (B * n_max, torch.int32), (B, torch.int32), (B, torch.int64), (B, torch.int32)]
-        arena = _Arena(eng.device, parts)
-        views = list(arena.views)
-        if assign:
-            names = ["col", "objective"] + (["u", "v"] if want_duals else [])
-            out = {k: views.pop(0) for k in names}
-            for k in ("col", "u", "v"):
-                if k in out:
-                    out[k] = out[k].view(B, n_max)
-            eng.assign_batch(packed, sizes, offsets, n_max, want_duals=want_duals, out=out)
-        if lcm is not None:
-            out = {k: views.pop(0) for k in ("rows", "cols", "n_pairs", "total", "last_min")}
-            out["rows"], out["cols"] = out["rows"].view(B, n_max), out["cols"].view(B, n_max)
-            eng.lcm_batch(packed, sizes, offsets, n_max, out=out, **lcm)
-        host = arena.host()                                        # the one read-back of the batch
-        if assign:
-            col, obj = host.pop(0).reshape(B, n_max), host.pop(0)
-            u = host.pop(0).reshape(B, n_max) if want_duals else None
-            v = host.pop(0).reshape(B, n_max) if want_duals else None
-            for k, b in enumerate(small):
-                n = mats[b].shape[0]
-                r = (col[k, :n].copy(), int(obj[k]))
-                res_a[b] = r + (u[k, :n].copy(), v[k, :n].copy()) if want_duals else r
-        if lcm is not None:
-            rows, cols = host.pop(0).reshape(B, n_max), host.pop(0).reshape(B, n_max)
-            npairs, total, last = host.pop(0), host.pop(0), host.pop(0)
-            for k, b in enumerate(small):
-                m = int(npairs[k])
-                res_l[b] = {"total": int(total[k]), "n_pairs": m, "rows": rows[k, :m].copy(), "cols": cols[k, :m].copy(),
-                            "last_min": int(last[k])}
-    for b in large:                                                # beyond one CTA's shared memory: one call each
-        a = mats[b]
+    for a in mats:
         if a.ndim != 2 or a.shape[0] != a.shape[1]:
             raise ValueError("run_batch takes square matrices, got shape %s" % (a.shape,))
+    small, mid, large = size_groups([a.shape[0] for a in mats])
+    res_a = [None] * len(mats) if assign else None
+    res_l = [None] * len(mats) if lcm is not None else None
+    lcm_single = set(large)
+    for group in (small, mid):
+        group_lcm = lcm
+        if lcm is not None and group is mid and len(group) < LCM_CLUSTER_MIN_BATCH:
+            group_lcm = None                                       # a few mid-size LCMs: single calls are faster
+            lcm_single.update(group)
+        if not group or (not assign and group_lcm is None):
+            continue
+        packed, sizes, offsets, n_max = pack_batch([mats[b] for b in group])
+        ra, rl = run_packed(packed, sizes, offsets, n_max, [mats[b].shape[0] for b in group], assign, want_duals, group_lcm)
+        for k, b in enumerate(group):
+            if assign:
+                res_a[b] = ra[k]
+            if group_lcm is not None:
+                res_l[b] = rl[k]
+    for b in sorted(lcm_single if lcm is not None else large):     # one call each
+        a = mats[b]
         eng = engine()
         n = a.shape[0]
         c = _h2d_i32(a)
-        if assign:
+        if assign and b in large:
             col, obj, _, _ = eng.assign(c)
             r = (_d2h(col), _d2h_int(obj))
             if want_duals:

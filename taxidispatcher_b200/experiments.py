@@ -5,6 +5,8 @@
                                        last solve over the customers and cabs the ranges left unserved
   greedy_then_solve  greedy_opt.py:131-163   LCM prefix with a distance threshold, exact solve on the rest
   lcm_vs_optimum     heuristic.py:20-40      LCM (mask 100) against the exact optimum on many small instances
+  split_hybrid_vs_optimum  split.py:186-212, greedy_opt.py:129-163   the paper's split / LCM / hybrid degradation over
+                                       many cases at once (batched stages)
   pool_greedy_vs_optimum  pool_opt_min.py      the Simulator's greedy 2-passenger pool against the optimal pairing
 
 Every range of solve_split is an independent K1 + K2 instance: with a process group the ranges are spread
@@ -210,6 +212,154 @@ def lcm_vs_optimum(costs: Sequence, solver_batch: Optional[Callable] = None, lcm
             lcm_batch = lcm_batch or (lambda cs: dispatch.LCM_batch(cs, mask_value=100))
         opt, lcm = solver_batch(costs), lcm_batch(costs)
     return [(int(l["total"]), int(o[1])) for l, o in zip(lcm, opt)]
+
+
+def _stage_runner(dist: np.ndarray, solver_batch: Optional[Callable], lcm_batch: Optional[Callable]):
+    """run(instances, assign, lcm=None, transpose=False) -> (col_of_row per instance or None, LCM dict per instance or
+    None) for instances given as (cab_to, cust_from) stand index arrays with calculate_cost semantics (positional, padded
+    with BIG_COST).  Without injected callables the matrices are built by K1 into packed device buffers and solved by
+    the batched kernels (one group per kernel); otherwise they are built on the host and handed to the callables."""
+    if solver_batch is None and lcm_batch is None:
+        from . import dispatch
+        dist_d = dispatch._h2d_i32(dist)
+        dist_t = []
+
+        def run_device(insts, assign, lcm=None, transpose=False):
+            if transpose and not dist_t:
+                dist_t.append(dist_d.t().contiguous())        # the stand table transposed: a layout copy
+            ns = [max(len(c), len(d)) for c, d in insts]
+            small, mid, large = dispatch.size_groups(ns)
+            if large:
+                raise ValueError("the batched experiment holds instances up to %d rows" % dispatch.BATCH_CLUSTER_MAX_N)
+            res_a, res_l = [None] * len(insts), [None] * len(insts)
+            for group in (small, mid):
+                if not group:
+                    continue
+                packed, sizes, offsets, n_max, gns = dispatch.pack_cost_matrices(
+                    dist_t[0] if transpose else dist_d, [insts[b] for b in group], transpose=transpose)
+                ra, rl = dispatch.run_packed(packed, sizes, offsets, n_max, gns, assign=assign, lcm=lcm)
+                for k, b in enumerate(group):
+                    res_a[b] = ra[k][0] if assign else None
+                    res_l[b] = rl[k] if lcm is not None else None
+            return (res_a if assign else None), (res_l if lcm is not None else None)
+        return run_device
+    if solver_batch is None or lcm_batch is None:
+        from . import dispatch
+        solver_batch = solver_batch or dispatch.solve_batch
+        lcm_batch = lcm_batch or dispatch.LCM_batch
+
+    def run_host(insts, assign, lcm=None, transpose=False):
+        mats = []
+        for c, d in insts:
+            c, d = np.asarray(c, dtype=np.int64), np.asarray(d, dtype=np.int64)
+            m = np.full((max(len(c), len(d)),) * 2, BIG_COST, dtype=np.int32)
+            if len(c) and len(d):
+                m[: len(c), : len(d)] = dist[c[:, None], d[None, :]]
+            mats.append(np.ascontiguousarray(m.T) if transpose else m)
+        return ([r[0] for r in solver_batch(mats)] if assign else None), (lcm_batch(mats, **lcm) if lcm is not None else None)
+    return run_host
+
+
+def split_hybrid_vs_optimum(distances, cases: Sequence, threshold: int = 10, solver_batch: Optional[Callable] = None,
+                            lcm_batch: Optional[Callable] = None):
+    """The paper's split / hybrid experiment (PDF p.5-6; split.py:186-212, greedy_opt.py:129-163) over many cases at once.
+    cases is a list of (demand, cabs) (lists of (id, from, to)); the stands are cut into len(distances) / 4 wide ranges
+    like split.py's main.  Returns per case (optimum, split total, LCM-split total, hybrid total, n2): the quantities of
+    greedy_then_solve (optimum, n2, hybrid), solve_split (split; None without demand or supply, split.py:62-64) and
+    split.py:209's LCM on the transposed cost matrix (SURVEY.md section 4 trap 5).
+    Three stages, each one batch over all cases: (1) optimum, greedy_opt LCM and split LCM on the full matrices, (2) the
+    hybrid rest instances and the four ranges of every case, (3) the split leftovers.  solver_batch(costs) ->
+    [(col_of_row, objective)] and lcm_batch(costs, **params) -> [LCM dict] are injectable (tests feed oracles); without
+    them the cost matrices are built on the device and never leave it."""
+    dist = np.asarray(distances)
+    size = len(dist)
+    split_size = int(size / 4)
+    if split_size <= 0:
+        raise ValueError("split needs at least 4 stands")
+    run = _stage_runner(dist, solver_batch, lcm_batch)
+
+    def inst(demand, cabs):
+        return (np.array([c[2] for c in cabs], dtype=np.int32), np.array([d[1] for d in demand], dtype=np.int32))
+
+    def picked(ins, col):
+        """cost[i][col[i]] of every row (count_sum / split.py:89 read these cells)"""
+        c, d = ins
+        col = np.asarray(col, dtype=np.int64)
+        rows = np.arange(len(col))
+        out = np.full(len(col), BIG_COST, dtype=np.int64)
+        real = (rows < len(c)) & (col < len(d))
+        out[real] = dist[c[rows[real]].astype(np.int64), d[col[real]].astype(np.int64)]
+        return out
+
+    def real_sum(p):
+        return int(p[p < BIG_COST].sum())
+
+    # ---- stage 1: optimum + greedy_opt LCM (greedy_opt.py:141-146), split LCM on the transpose (split.py:209) ----------
+    full = [inst(dem, cab) for dem, cab in cases]
+    cols, greedy = run(full, True, dict(mask_value=BIG_COST, stop_above=threshold, sum_below=BIG_COST))
+    _, lcm_split = run(full, False, dict(mask_value=BIG_COST, sum_below=BIG_COST), transpose=True)
+    # ---- stage 2: the hybrid rest (greedy_opt.py:147-150) and the ranges of split.py:66-105 ---------------------------
+    stage2, jobs = [], []            # jobs: (case, "rest") or (case, range index, split_demand, split_cabs)
+    rest_n2 = []
+    ranges = []
+    start = 0
+    while start < size:
+        ranges.append(range(start, start + split_size))
+        start += split_size
+    for k, (demand, cabs) in enumerate(cases):
+        rest_demand = filter_out(demand, greedy[k]["cols"].tolist(), 0)
+        rest_cabs = filter_out(cabs, greedy[k]["rows"].tolist(), 0)
+        rest_n2.append(max(len(rest_demand), len(rest_cabs)))
+        if rest_demand and rest_cabs:
+            stage2.append(inst(rest_demand, rest_cabs)); jobs.append((k, "rest"))
+        if demand and cabs:
+            for r in ranges:
+                sd, sc = filter_rows(demand, r, 1), filter_rows(cabs, r, 2)
+                if sd and sc:
+                    stage2.append(inst(sd, sc)); jobs.append((k, "range", sd, sc))
+    cols2, _ = run(stage2, True)
+    hyb_rest = [0] * len(cases)
+    split_sum = [0] * len(cases)
+    rest_cust = [[] for _ in cases]
+    rest_cab_ids = [[] for _ in cases]
+    for ins, col, job in zip(stage2, cols2, jobs):
+        k = job[0]
+        p = picked(ins, col)
+        if job[1] == "rest":
+            hyb_rest[k] = real_sum(p)
+            continue
+        sd, sc = job[2], job[3]
+        split_sum[k] += int(p[p != BIG_COST].sum())
+        for taxi in np.nonzero(p == BIG_COST)[0]:                  # split.py:89 -- not served
+            if len(sc) > len(sd):
+                rest_cab_ids[k].append(sc[taxi][0])
+            else:
+                rest_cust[k].append(sd[int(col[taxi])][0])
+    # ranges with one side only hand all of it to the leftover run (split.py:94-105)
+    for k, (demand, cabs) in enumerate(cases):
+        if not (demand and cabs):
+            continue
+        for r in ranges:
+            sd, sc = filter_rows(demand, r, 1), filter_rows(cabs, r, 2)
+            if sd and not sc:
+                rest_cust[k] += [d[0] for d in sd]
+            elif sc and not sd:
+                rest_cab_ids[k] += [c[0] for c in sc]
+    # ---- stage 3: the split leftovers (split.py:109-119) --------------------------------------------------------------
+    stage3, owners = [], []
+    for k, (demand, cabs) in enumerate(cases):
+        rd, rs = filter_rows(demand, rest_cust[k], 0), filter_rows(cabs, rest_cab_ids[k], 0)
+        if rd and rs:
+            stage3.append(inst(rd, rs)); owners.append(k)
+    cols3, _ = run(stage3, True)
+    for k, ins, col in zip(owners, stage3, cols3):
+        split_sum[k] += real_sum(picked(ins, col))
+    out = []
+    for k, (demand, cabs) in enumerate(cases):
+        opt = real_sum(picked(full[k], cols[k])) if max(len(demand), len(cabs)) else 0
+        split = split_sum[k] if (demand and cabs) else None
+        out.append((opt, split, int(lcm_split[k]["total"]), hyb_rest[k] + int(greedy[k]["total"]), rest_n2[k]))
+    return out
 
 
 def pool_greedy_vs_optimum(instances: Sequence, dist, accept_all: bool = True, max_loss: float = 1.01,
