@@ -318,6 +318,22 @@ int td_pool_pairs_exact_batch(const int32_t *from, const int32_t *to, const int3
                               int32_t *pairs_out /* batch x (n_max/2) x 4 */, int32_t *n_pairs_out /* batch */,
                               int64_t *cost_out /* batch */, void *workspace, size_t workspace_bytes, void *stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Greedy 2-passenger pool, batched: td_pool_pairs over many instances in one launch
+ *
+ * Arguments, layout, argument checks, withdrawal and return codes are those of td_pool_pairs_exact_batch above, without
+ * the workspace (one CTA per instance, everything in shared memory).  pairs_out[b] holds exactly the rows
+ * [custA, custB, plan, cost] that td_pool_pairs returns for instance b with the same dist / accept_all / max_loss, in
+ * its scan order; n_pairs_out[b] is their count and cost_out[b] their total; unused rows are -1.  The greedy under the
+ * strict order (cost, A*n+B) has one answer, so it depends on nothing but the instance.  Unlike td_pool_pairs, an
+ * instance holds at most TD_PAIRS_BATCH_MAX_N customers and every table entry must lie in [0, 2^22].
+ * ------------------------------------------------------------------------------------------ */
+#define TD_PAIRS_BATCH_MAX_N 4096
+int td_pool_pairs_batch(const int32_t *from, const int32_t *to, const int32_t *sizes, const int64_t *offsets,
+                        int batch, int n_max, const int32_t *dist, int n_stands, int accept_all, double max_loss,
+                        int32_t *pairs_out /* batch x (n_max/2) x 4 */, int32_t *n_pairs_out /* batch */,
+                        int64_t *cost_out /* batch */, void *stream);
+
 /* After an ASYNCHRONOUS td_pool_find / td_pool_find_shards call (stats == NULL) on `workspace`: waits for the
  * stream and reads the per-shard counters back (one small copy).  *overflow_out != 0: the record list was too
  * small for a single pass -- counts_out holds -1 and the call has to be repeated synchronously (stats != NULL),
@@ -376,6 +392,10 @@ int tdh_pool_find(const int32_t *demand, int n, const int32_t *dist, int n_stand
  * rows; a live row with a stand outside the table, or a table entry outside [0, 2^22], is TD_ERR_INVALID here */
 int tdh_pool_pairs_exact(const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
                          int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out);
+/* one instance of td_pool_pairs_batch: the Simulator's own greedy (Simulator.findPool) from host buffers, with the checks
+ * of tdh_pool_pairs_exact; pairs_out holds n/2 rows */
+int tdh_pool_pairs(const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
+                   int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out);
 /* all n_shards logical shards + merge, i.e. what `findpool` produces (findpool.c:122-176) */
 int tdh_pool_find_all(const int32_t *demand, int n, const int32_t *dist, int n_stands, int pool_size,
                       int n_shards, int32_t *plans_out, int32_t cap, int32_t *n_plans_out,

@@ -18,6 +18,7 @@ TD_ERR_NOT_CONVERGED = -6
 INT32_MAX = 2**31 - 1
 BIG_COST = 250000
 PAIRS_EXACT_MAX_N = 4096    # TD_PAIRS_EXACT_MAX_N
+PAIRS_BATCH_MAX_N = 4096    # TD_PAIRS_BATCH_MAX_N
 POOL_REC_W = 9
 PROF_COST, PROF_LCM, PROF_ASSIGN, PROF_POOL_ENUM, PROF_POOL_SELECT = range(5)
 
@@ -98,7 +99,9 @@ _SIGNATURES = {
     "td_pool_pairs_exact_workspace_bytes": (ctypes.c_size_t, [_I, _I]),
     "td_pool_pairs_exact_batch": (_I, [c_vp, c_vp, c_vp, c_vp, _I, _I, c_vp, _I, _I, ctypes.c_double, c_vp, c_vp, c_vp, c_vp,
                                        ctypes.c_size_t, c_vp]),
+    "td_pool_pairs_batch": (_I, [c_vp, c_vp, c_vp, c_vp, _I, _I, c_vp, _I, _I, ctypes.c_double, c_vp, c_vp, c_vp, c_vp]),
     "tdh_pool_pairs_exact": (_I, [c_vp, c_vp, _I, c_vp, _I, _I, ctypes.c_double, c_vp, c_vp, c_vp]),
+    "tdh_pool_pairs": (_I, [c_vp, c_vp, _I, c_vp, _I, _I, ctypes.c_double, c_vp, c_vp, c_vp]),
     "tdh_cost_matrix": (_I, [c_vp, _I, c_vp, _I, c_vp, _I, ctypes.c_int32, ctypes.c_int32, c_vp]),
     "tdh_lcm": (_I, [c_vp, _I, ctypes.POINTER(LcmParams), c_vp, c_vp, c_vp, c_vp, c_vp]),
     "tdh_assign_exact": (_I, [c_vp, _I, c_vp, c_vp, c_vp, ctypes.POINTER(AssignStats)]),

@@ -234,8 +234,9 @@ extern "C" int tdh_pool_find(const int32_t *demand, int n, const int32_t *dist, 
     return *n_plans_out > cap ? TD_ERR_CAPACITY : TD_OK;
 }
 
-extern "C" int tdh_pool_pairs_exact(const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
-                                    int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out) {
+// one instance of td_pool_pairs_exact_batch (exact) or td_pool_pairs_batch (greedy) from host buffers
+static int tdh_pool_pairs_one(bool exact, const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
+                              int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out) {
     if (n < 0 || n > TD_PAIRS_EXACT_MAX_N || n_stands < 1 || n_stands > 128 || !n_pairs_out || !cost_out) return TD_ERR_INVALID;
     if (!accept_all && !std::isfinite(max_loss)) return TD_ERR_INVALID;
     if (n > 0 && (!from || !to)) return TD_ERR_INVALID;
@@ -255,18 +256,35 @@ extern "C" int tdh_pool_pairs_exact(const int32_t *from, const int32_t *to, int 
     const int rows = n / 2;
     const size_t out_bytes = 16 + size_t(rows > 0 ? rows : 1) * 16;   // cost (8), count (4), pad, rows
     TDH_TRY(d_out.alloc(out_bytes));
-    const size_t wsb = td_pool_pairs_exact_workspace_bytes(1, n);
-    TDH_TRY(d_ws.alloc(wsb));
     int32_t *in = d_in.as<int32_t>();
     char *out = d_out.as<char>();
-    TDH_RC(td_pool_pairs_exact_batch(in, in + nn, in + 2 * nn, reinterpret_cast<const int64_t *>(in + off_at), 1, n, in + dist_at,
-                                     n_stands, accept_all, max_loss, reinterpret_cast<int32_t *>(out + 16),
-                                     reinterpret_cast<int32_t *>(out + 8), reinterpret_cast<int64_t *>(out), d_ws.p, wsb, nullptr));
+    const int64_t *offs = reinterpret_cast<const int64_t *>(in + off_at);
+    int32_t *rows_d = reinterpret_cast<int32_t *>(out + 16), *count_d = reinterpret_cast<int32_t *>(out + 8);
+    int64_t *cost_d = reinterpret_cast<int64_t *>(out);
+    if (exact) {
+        const size_t wsb = td_pool_pairs_exact_workspace_bytes(1, n);
+        TDH_TRY(d_ws.alloc(wsb));
+        TDH_RC(td_pool_pairs_exact_batch(in, in + nn, in + 2 * nn, offs, 1, n, in + dist_at, n_stands, accept_all, max_loss,
+                                         rows_d, count_d, cost_d, d_ws.p, wsb, nullptr));
+    } else {
+        TDH_RC(td_pool_pairs_batch(in, in + nn, in + 2 * nn, offs, 1, n, in + dist_at, n_stands, accept_all, max_loss, rows_d,
+                                   count_d, cost_d, nullptr));
+    }
     std::vector<char> host(out_bytes);
     TDH_TRY(cudaMemcpy(host.data(), out, out_bytes, cudaMemcpyDeviceToHost));
     memcpy(cost_out, host.data(), 8); memcpy(n_pairs_out, host.data() + 8, 4);
     if (*n_pairs_out > 0) memcpy(pairs_out, host.data() + 16, size_t(*n_pairs_out) * 16);
     return TD_OK;
+}
+
+extern "C" int tdh_pool_pairs_exact(const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
+                                    int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out) {
+    return tdh_pool_pairs_one(true, from, to, n, dist, n_stands, accept_all, max_loss, pairs_out, n_pairs_out, cost_out);
+}
+
+extern "C" int tdh_pool_pairs(const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
+                              int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out) {
+    return tdh_pool_pairs_one(false, from, to, n, dist, n_stands, accept_all, max_loss, pairs_out, n_pairs_out, cost_out);
 }
 
 extern "C" int tdh_pool_find_all(const int32_t *demand, int n, const int32_t *dist, int n_stands, int pool_size,

@@ -1,4 +1,5 @@
-// td_pairs.cu -- exact 2-passenger pool: minimum-cost maximum-cardinality pair matching, batched, one CTA per instance.
+// td_pairs.cu -- exact 2-passenger pool: minimum-cost maximum-cardinality pair matching, batched, one CTA per instance;
+// and the Simulator's greedy 2-passenger pool over the same batch layout and edges (pairs_greedy_kernel, at the end).
 //
 // The greedy of Simulator.findPool (td_pool.cu, pool_pairs_*) stable-sorts the accepted candidates by cost and scans them
 // for disjoint pairs.  Its exact counterpart (the ILP of the reference's pool_optimum.py / pool_opt_min.py, where every
@@ -67,16 +68,21 @@ __host__ __device__ static PairsWs carve_pairs(void *base, int n_max) {
     return w;
 }
 
-struct PairsCtx {
-    PairsWs w;
-    int n, S, accept_all, qn, nfree;
+// what defines the edges of an instance; shared by the exact kernel and the greedy batch kernel
+struct PairsEdges {
+    int S, accept_all;
     double max_loss;
-    long long K;
     const int32_t *dist, *from, *to;   // shared memory
 };
 
+struct PairsCtx : PairsEdges {
+    PairsWs w;
+    int n, qn, nfree;
+    long long K;
+};
+
 // accepted candidate (A first picked up, then B) -> cost, or -1; plan as in pool_pairs_enum_kernel
-__device__ __forceinline__ int candidate(const PairsCtx &m, int A, int B, int *plan) {
+__device__ __forceinline__ int candidate(const PairsEdges &m, int A, int B, int *plan) {
     const int S = m.S, fa = m.from[A], ta = m.to[A], fb = m.from[B], tb = m.to[B];
     const int32_t *d = m.dist;
     const int dab = d[fa * S + fb];
@@ -94,7 +100,7 @@ __device__ __forceinline__ int candidate(const PairsCtx &m, int A, int B, int *p
 }
 
 // edge {i, j}: the cost of the preferred accepted candidate (smallest (cost, A*n+B)), or -1 when there is no edge
-__device__ __forceinline__ int edge_cost(const PairsCtx &m, int i, int j, int *A_out = nullptr, int *plan_out = nullptr) {
+__device__ __forceinline__ int edge_cost(const PairsEdges &m, int i, int j, int *A_out = nullptr, int *plan_out = nullptr) {
     if (i == j || m.from[i] < 0 || m.from[j] < 0) return -1;
     const int lo = i < j ? i : j, hi = i < j ? j : i;
     int p1 = 0, p2 = 0;
@@ -325,7 +331,41 @@ __device__ void augment_matching(PairsCtx &m, int v, int w) {
     }
 }
 
-// ---- the kernel -------------------------------------------------------------------------------------------------------
+// ---- the kernels ------------------------------------------------------------------------------------------------------
+// Stages instance blockIdx.x (the stand table, its from / to) in shared memory and returns its size.  A withdrawn
+// instance (bad size or offset, a live row whose stand lies outside the table, a table entry outside [0, 2^22]) gets its
+// outputs here and -1 back; the neighbours are unaffected.  The `to` of a removed row (from < 0) is never read.
+__device__ int stage_instance(const int32_t *__restrict__ from, const int32_t *__restrict__ to,
+                              const int32_t *__restrict__ sizes, const int64_t *__restrict__ offsets, int n_max,
+                              const int32_t *__restrict__ dist, int S, int32_t *s_dist, int32_t *s_from, int32_t *s_to,
+                              int32_t *rows, int32_t *n_pairs_out, long long *cost_out, int *s_bad) {
+    const int tid = threadIdx.x, inst = blockIdx.x;
+    const int n = sizes[inst];
+    const long long off = offsets[inst];
+    if (tid == 0) *s_bad = (n < 0 || n > n_max || off < 0) ? 1 : 0;
+    __syncthreads();
+    if (!*s_bad) {
+        for (int k = tid; k < S * S; k += blockDim.x) {
+            const int d = dist[k];
+            if (d < 0 || d > kPairsMaxDist) *s_bad = 1;
+            s_dist[k] = d;
+        }
+        for (int i = tid; i < n; i += blockDim.x) {
+            const int f = from[off + i], t = f >= 0 ? to[off + i] : -1;
+            if (f >= 0 && (f >= S || t < 0 || t >= S)) *s_bad = 1;
+            s_from[i] = f; s_to[i] = t;
+        }
+    }
+    __syncthreads();
+    if (*s_bad) {
+        const int rows_cap = n_max / 2;
+        for (int k = tid; k < rows_cap * 4; k += blockDim.x) rows[k] = -1;
+        if (tid == 0) { n_pairs_out[inst] = -1; cost_out[inst] = LLONG_MIN; }
+        return -1;
+    }
+    return n;
+}
+
 // Key layouts of the min-reductions: edge keys (slack << 24 | v << 12 | w), delta keys (delta << 16 | type << 13 | index).
 __device__ __forceinline__ unsigned long long edge_key(long long sl, int v, int w) {
     return (unsigned long long)sl << 24 | (unsigned long long)v << 12 | unsigned(w);
@@ -344,29 +384,9 @@ pairs_exact_kernel(const int32_t *__restrict__ from, const int32_t *__restrict__
     const int rows_cap = n_max / 2;
     int32_t *rows = pairs_out + size_t(inst) * rows_cap * 4;
     int32_t *s_dist = smem, *s_from = smem + S * S, *s_to = s_from + (n_max > 0 ? n_max : 1);
-
-    const int n = sizes[inst];
-    const long long off = offsets[inst];
-    if (tid == 0) s_bad = (n < 0 || n > n_max || off < 0) ? 1 : 0;
-    __syncthreads();
-    if (!s_bad) {
-        for (int k = tid; k < S * S; k += blockDim.x) {
-            const int d = dist[k];
-            if (d < 0 || d > kPairsMaxDist) s_bad = 1;
-            s_dist[k] = d;
-        }
-        for (int i = tid; i < n; i += blockDim.x) {
-            const int f = from[off + i], t = to[off + i];
-            if (f >= 0 && (f >= S || t < 0 || t >= S)) s_bad = 1;
-            s_from[i] = f; s_to[i] = t;
-        }
-    }
-    __syncthreads();
-    if (s_bad) {                                               // withdrawn: the neighbours are unaffected
-        for (int k = tid; k < rows_cap * 4; k += blockDim.x) rows[k] = -1;
-        if (tid == 0) { n_pairs_out[inst] = -1; cost_out[inst] = LLONG_MIN; }
-        return;
-    }
+    const int n = stage_instance(from, to, sizes, offsets, n_max, dist, S, s_dist, s_from, s_to, rows, n_pairs_out, cost_out,
+                                 &s_bad);
+    if (n < 0) return;
 
     PairsCtx m;
     m.w = carve_pairs(workspace + size_t(inst) * stride, n_max);
@@ -563,9 +583,141 @@ pairs_exact_kernel(const int32_t *__restrict__ from, const int32_t *__restrict__
     if (tid == 0) { n_pairs_out[inst] = npairs; cost_out[inst] = s_total; }
 }
 
+// ---- the greedy of Simulator.findPool, batched (see DESIGN.md section 14) ---------------------------------------------
+// td_pool_pairs stable-sorts the accepted ordered candidates by cost and keeps every pair whose customers are both still
+// free.  Per unordered pair only its preferred candidate (smallest (cost, A*n+B), edge_cost) can be kept, so this is the
+// greedy matching under the strict edge order key = cost << 24 | A*n+B (cost <= 3 * 2^22 < 2^24, A*n+B < 2^24).  With
+// distinct keys it equals dominance rounds: an edge that is the smallest live edge at both ends is kept by the scan
+// (every smaller edge misses both ends), and removing its two customers leaves the scan of the rest unchanged.  Every
+// live customer caches its smallest live edge; a round keeps all mutual bests, then rescans only the customers whose
+// cached partner died.  A round that keeps nothing means no live edge is left (the smallest one is always mutual).
+__device__ __forceinline__ unsigned long long greedy_key(const PairsEdges &e, int n, int i, int j) {
+    int A;
+    const int c = edge_cost(e, i, j, &A);
+    return c < 0 ? kNone : (unsigned long long)c << 24 | unsigned(A * n + (A == i ? j : i));
+}
+
+__device__ __forceinline__ int key_partner(unsigned long long key, int n, int i) {
+    const int ab = int(key & 0xffffff), A = ab / n;
+    return A == i ? ab - A * n : A;
+}
+
+__global__ void __launch_bounds__(1024)
+pairs_greedy_kernel(const int32_t *__restrict__ from, const int32_t *__restrict__ to, const int32_t *__restrict__ sizes,
+                    const int64_t *__restrict__ offsets, int n_max, const int32_t *__restrict__ dist, int S, int accept_all,
+                    double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, long long *cost_out) {
+    extern __shared__ unsigned long long smem64[];
+    __shared__ int s_bad, s_m, s_nlive, s_nscan;
+    __shared__ long long s_total;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5, inst = blockIdx.x;
+    const int rows_cap = n_max / 2, N = n_max > 0 ? n_max : 1;
+    int32_t *rows = pairs_out + size_t(inst) * rows_cap * 4;
+    unsigned long long *best = smem64, *kept = best + N;               // kept: n_max / 2 + 1 keys
+    int32_t *s_dist = reinterpret_cast<int32_t *>(kept + N / 2 + 1), *s_from = s_dist + S * S, *s_to = s_from + N;
+    int32_t *live = s_to + N, *live_next = s_to + 2 * N, *scan = s_to + 3 * N;
+    uint8_t *alive = reinterpret_cast<uint8_t *>(s_to + 4 * N);
+    const int n = stage_instance(from, to, sizes, offsets, n_max, dist, S, s_dist, s_from, s_to, rows, n_pairs_out, cost_out,
+                                 &s_bad);
+    if (n < 0) return;
+    PairsEdges e;
+    e.S = S; e.accept_all = accept_all; e.max_loss = max_loss; e.dist = s_dist; e.from = s_from; e.to = s_to;
+
+    // every customer that is not a removed row is live and scans once
+    if (tid == 0) { s_m = 0; s_total = 0; s_nlive = 0; }
+    __syncthreads();
+    for (int i = tid; i < n; i += blockDim.x) {
+        alive[i] = s_from[i] >= 0;
+        if (alive[i]) { const int k = atomicAdd(&s_nlive, 1); live[k] = i; scan[k] = i; }
+    }
+    __syncthreads();
+    int nlive = s_nlive, nscan = nlive, kept_before = 0;
+    for (;;) {
+        // rescan: one warp per customer, min over the live list (its order does not matter to a minimum).  A customer
+        // left out of the list is dead or had no live edge when it last scanned, so it has no edge to anyone live now.
+        for (int k = warp; k < nscan; k += nwarps) {
+            const int i = scan[k];
+            unsigned long long b = kNone;
+            for (int q = lane; q < nlive; q += 32) {
+                const int j = live[q];
+                if (j == i) continue;
+                const unsigned long long key = greedy_key(e, n, i, j);
+                b = key < b ? key : b;
+            }
+            b = warp_min_u64(b);
+            if (lane == 0) best[i] = b;
+        }
+        __syncthreads();
+        // keep every mutual best; the customer with the lower index records the pair
+        if (tid == 0) { s_nlive = 0; s_nscan = 0; }
+        for (int k = tid; k < nlive; k += blockDim.x) {
+            const int i = live[k];
+            const unsigned long long b = best[i];
+            if (b == kNone) continue;
+            const int p = key_partner(b, n, i);
+            if (best[p] != b) continue;
+            alive[i] = 0;
+            if (i < p) kept[atomicAdd(&s_m, 1)] = b;
+        }
+        __syncthreads();
+        if (s_m == kept_before) break;                                 // no mutual best: no live edge is left
+        kept_before = s_m;
+        // next live list: customers that are alive and still have an edge; rescan those whose partner died
+        for (int k = tid; k < nlive; k += blockDim.x) {
+            const int i = live[k];
+            const unsigned long long b = best[i];
+            if (!alive[i] || b == kNone) continue;
+            live_next[atomicAdd(&s_nlive, 1)] = i;
+            if (!alive[key_partner(b, n, i)]) scan[atomicAdd(&s_nscan, 1)] = i;
+        }
+        __syncthreads();
+        int32_t *const t = live; live = live_next; live_next = t;
+        nlive = s_nlive;
+        nscan = s_nscan;
+    }
+
+    // ---- output: the kept pairs in key order (rank counting), i.e. td_pool_pairs' scan order ----
+    const int npairs = s_m;
+    long long part = 0;
+    for (int k = tid; k < npairs; k += blockDim.x) {
+        const unsigned long long me = kept[k];
+        int rank = 0;
+        for (int q = 0; q < npairs; ++q) rank += kept[q] < me;
+        const int ab = int(me & 0xffffff), A = ab / n, B = ab - A * n;
+        int plan = 0;
+        edge_cost(e, A, B, nullptr, &plan);
+        int32_t *r = rows + size_t(rank) * 4;
+        r[0] = A; r[1] = B; r[2] = plan; r[3] = int(me >> 24);
+        part += int(me >> 24);
+    }
+    atomicAdd(reinterpret_cast<unsigned long long *>(&s_total), (unsigned long long)part);
+    for (int k = npairs * 4 + tid; k < rows_cap * 4; k += blockDim.x) rows[k] = -1;
+    __syncthreads();
+    if (tid == 0) { n_pairs_out[inst] = npairs; cost_out[inst] = s_total; }
+}
+
 static size_t pairs_stride(int n_max) { return carve_pairs(nullptr, n_max).bytes; }
 
 static size_t pairs_smem(int n_max, int S) { return (size_t(S) * S + 2 * size_t(n_max > 0 ? n_max : 1)) * sizeof(int32_t); }
+
+// best (n_max keys), kept (n_max / 2 + 1 keys), the stand table, from, to, two live lists, the rescan list, alive bytes
+static size_t greedy_smem(int n_max, int S) {
+    const size_t N = n_max > 0 ? size_t(n_max) : 1;
+    return (N + N / 2 + 1) * sizeof(unsigned long long) + (size_t(S) * S + 5 * N) * sizeof(int32_t) + N;
+}
+
+// the argument checks of both batch entry points, in this order, before any device lookup; kNothingToLaunch for batch 0
+constexpr int kNothingToLaunch = 1;
+static_assert(TD_PAIRS_EXACT_MAX_N == TD_PAIRS_BATCH_MAX_N, "both pair kernels take the same instance sizes");
+static int check_pairs_batch(const int32_t *from, const int32_t *to, const int32_t *sizes, const int64_t *offsets, int batch,
+                             int n_max, const int32_t *dist, int n_stands, int accept_all, double max_loss,
+                             const int32_t *pairs_out, const int32_t *n_pairs_out, const int64_t *cost_out) {
+    if (batch < 0 || n_max < 0 || n_max > TD_PAIRS_BATCH_MAX_N) return TD_ERR_INVALID;
+    if (n_stands < 1 || n_stands > kPairsMaxStands) return TD_ERR_INVALID;
+    if (!accept_all && !std::isfinite(max_loss)) return TD_ERR_INVALID;
+    if (batch == 0) return have_device() ? kNothingToLaunch : TD_ERR_NO_DEVICE;
+    if (!from || !to || !sizes || !offsets || !dist || !n_pairs_out || !cost_out || (n_max >= 2 && !pairs_out)) return TD_ERR_INVALID;
+    return TD_OK;
+}
 
 }  // namespace td
 
@@ -574,16 +726,33 @@ extern "C" size_t td_pool_pairs_exact_workspace_bytes(int batch, int n_max) {
     return size_t(batch) * td::pairs_stride(n_max);
 }
 
+extern "C" int td_pool_pairs_batch(const int32_t *from, const int32_t *to, const int32_t *sizes, const int64_t *offsets,
+                                   int batch, int n_max, const int32_t *dist, int n_stands, int accept_all, double max_loss,
+                                   int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out, void *stream) {
+    using namespace td;
+    const int rc = check_pairs_batch(from, to, sizes, offsets, batch, n_max, dist, n_stands, accept_all, max_loss, pairs_out,
+                                     n_pairs_out, cost_out);
+    if (rc != TD_OK) return rc == kNothingToLaunch ? TD_OK : rc;
+    if (!have_device()) return TD_ERR_NO_DEVICE;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t smem = greedy_smem(n_max, n_stands);
+    // small instances: several CTAs of 256 threads per SM; large ones: one warp per rescanned customer on 32 warps
+    const int threads = n_max > 512 ? 1024 : 256;
+    TD_CUDA_TRY(cudaFuncSetAttribute(pairs_greedy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    pairs_greedy_kernel<<<batch, threads, smem, st>>>(from, to, sizes, offsets, n_max, dist, n_stands, accept_all, max_loss,
+                                                      pairs_out, n_pairs_out, reinterpret_cast<long long *>(cost_out));
+    TD_LAUNCH_CHECK();
+    return TD_OK;
+}
+
 extern "C" int td_pool_pairs_exact_batch(const int32_t *from, const int32_t *to, const int32_t *sizes, const int64_t *offsets,
                                          int batch, int n_max, const int32_t *dist, int n_stands, int accept_all,
                                          double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out,
                                          void *workspace, size_t workspace_bytes, void *stream) {
     using namespace td;
-    if (batch < 0 || n_max < 0 || n_max > TD_PAIRS_EXACT_MAX_N) return TD_ERR_INVALID;
-    if (n_stands < 1 || n_stands > kPairsMaxStands) return TD_ERR_INVALID;
-    if (!accept_all && !std::isfinite(max_loss)) return TD_ERR_INVALID;
-    if (batch == 0) return have_device() ? TD_OK : TD_ERR_NO_DEVICE;
-    if (!from || !to || !sizes || !offsets || !dist || !n_pairs_out || !cost_out || (n_max >= 2 && !pairs_out)) return TD_ERR_INVALID;
+    const int rc = check_pairs_batch(from, to, sizes, offsets, batch, n_max, dist, n_stands, accept_all, max_loss, pairs_out,
+                                     n_pairs_out, cost_out);
+    if (rc != TD_OK) return rc == kNothingToLaunch ? TD_OK : rc;
     if (!workspace || workspace_bytes < td_pool_pairs_exact_workspace_bytes(batch, n_max)) return TD_ERR_WORKSPACE;
     if (!have_device()) return TD_ERR_NO_DEVICE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);

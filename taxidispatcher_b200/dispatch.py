@@ -11,6 +11,7 @@ Host functions mirror the reference's names, argument order and return layouts
   LCM_java(cost)                                   Simulator.java:523-549
   solve_batch(costs) / LCM_batch(costs, ...)       heuristic.py:20-40, python.py:6-25 over many instances
   find_pool(...) / find_pool_all(...) / pool_merge(...)   pool_n.c / findpool.c
+  find_pool_pairs_batch(...)                       Simulator.findPool over many instances in one launch
   find_pool_pairs_exact(...) / find_pool_pairs_exact_batch(...)   the optimum of pool_optimum.py / pool_opt_min.py
 
 PyTorch is used only for device buffers, pinned staging and streams.  All arithmetic runs in the
@@ -31,7 +32,7 @@ from ._lib import BIG_COST, INT32_MAX, PAIRS_EXACT_MAX_N, POOL_REC_W, AssignStat
 
 __all__ = ["BIG_COST", "Engine", "calculate_cost", "solve", "solve_dispatch", "solve_full", "solve_assignment", "LCM", "LCM_heuristic",
            "LCM_split", "LCM_greedy_opt", "LCM_simulate", "LCM_java", "find_pool", "find_pool_all", "find_pool_block",
-           "find_pool_pairs", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "pool_merge", "pack_batch", "pack_cost_matrices", "run_packed", "run_batch", "solve_batch", "LCM_batch",
+           "find_pool_pairs", "find_pool_pairs_batch", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "pool_merge", "pack_batch", "pack_cost_matrices", "run_packed", "run_batch", "solve_batch", "LCM_batch",
            "TaxiDispatchError"]
 
 
@@ -518,6 +519,21 @@ class Engine:
         check(rc, "td_pool_pairs_exact_batch")
         return rows, npairs, cost
 
+    def pool_pairs_batch(self, frm: torch.Tensor, to: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor, n_max: int,
+                         dist: torch.Tensor, accept_all: bool = True, max_loss: float = 1.01, out: Optional[dict] = None):
+        """Simulator.findPool's greedy of every instance (the batch layout of pool_pairs_exact_batch), one launch.  Returns
+        device tensors (rows [B, n_max // 2, 4] int32 = exactly the rows pool_pairs returns, n_pairs [B] int32, cost [B]
+        int64); a withdrawn instance has n_pairs -1.  `out` may supply any of them by name ("rows", "n_pairs", "cost")."""
+        B = int(sizes.numel())
+        rows = self._batch_out(out, "rows", (B, n_max // 2, 4), torch.int32)
+        npairs = self._batch_out(out, "n_pairs", (B,), torch.int32)
+        cost = self._batch_out(out, "cost", (B,), torch.int64)
+        rc = self.lib.td_pool_pairs_batch(_ptr(frm), _ptr(to), _ptr(sizes), _ptr(offsets), B, int(n_max), _ptr(dist),
+                                          int(dist.shape[0]), 1 if accept_all else 0, float(max_loss), _ptr(rows),
+                                          _ptr(npairs), _ptr(cost), _stream())
+        check(rc, "td_pool_pairs_batch")
+        return rows, npairs, cost
+
     def pool_merge(self, shard_plans: torch.Tensor, total: int, n: int, pool_size: int):
         out = torch.empty((max(total, 1), POOL_REC_W), dtype=torch.int32, device=self.device)
         cnt = torch.zeros(1, dtype=torch.int32, device=self.device)
@@ -931,26 +947,46 @@ def pack_pairs_batch(instances: Sequence, dist):
             dev[off_at: off_at + 2 * B].view(torch.int64), n_max, dev[dist_at: dist_at + d.size].reshape(d.shape))
 
 
+def _find_pairs_batches(instances: Sequence, dist, accept_all: bool, max_loss: float, kinds: Sequence[str]):
+    """Every (frm, to) instance through each of the pair kernels named in `kinds` ("greedy": td_pool_pairs_batch,
+    "exact": td_pool_pairs_exact_batch): one pinned upload, one launch per kind and one read-back for all of them.
+    Returns per kind the per-instance rows, or None for an instance the library withdrew."""
+    B = len(instances)
+    if B == 0:
+        return [[] for _ in kinds]
+    eng = engine()
+    frm, to, sizes, offsets, n_max, d = pack_pairs_batch(instances, dist)
+    if n_max > PAIRS_EXACT_MAX_N:
+        raise ValueError("an instance has %d customers; the batched 2-passenger pools take at most %d" % (n_max, PAIRS_EXACT_MAX_N))
+    cap = n_max // 2
+    arena = _Arena(eng.device, [(B * cap * 4, torch.int32), (B, torch.int32), (B, torch.int64)] * len(kinds))
+    for k, kind in enumerate(kinds):
+        rows_v, np_v, cost_v = arena.views[3 * k: 3 * k + 3]
+        launch = {"greedy": eng.pool_pairs_batch, "exact": eng.pool_pairs_exact_batch}[kind]
+        launch(frm, to, sizes, offsets, n_max, d, accept_all, max_loss,
+               out={"rows": rows_v.view(B, cap, 4), "n_pairs": np_v, "cost": cost_v})
+    host = arena.host()                                            # the one read-back of the batch
+    out = []
+    for k in range(len(kinds)):
+        rows, npairs = host[3 * k].reshape(B, cap, 4), host[3 * k + 1]
+        out.append([None if npairs[b] < 0 else rows[b, : int(npairs[b])].copy() for b in range(B)])
+    return out
+
+
+def find_pool_pairs_batch(instances: Sequence, dist, accept_all: bool = True, max_loss: float = 1.01):
+    """Simulator.findPool for every (frm, to) instance over one stand table: one pinned upload, one launch and one
+    read-back.  Returns per instance exactly the array find_pool_pairs returns, or None for an instance the library
+    withdrew (a live row whose stand lies outside the table).  Instances hold at most PAIRS_BATCH_MAX_N customers and
+    every table entry must lie in [0, 2^22]."""
+    return _find_pairs_batches(instances, dist, accept_all, max_loss, ("greedy",))[0]
+
+
 def find_pool_pairs_exact_batch(instances: Sequence, dist, accept_all: bool = True, max_loss: float = 1.01):
     """The exact 2-passenger pool of every (frm, to) instance over one stand table: one pinned upload, one launch and one
     read-back.  Returns per instance the rows (custA, custB, plan, cost) of a minimum-cost maximum-cardinality pairing
     in (cost, A*n+B) order -- the layout find_pool_pairs returns -- or None for an instance the library withdrew (a
     live row whose stand lies outside the table)."""
-    B = len(instances)
-    if B == 0:
-        return []
-    eng = engine()
-    frm, to, sizes, offsets, n_max, d = pack_pairs_batch(instances, dist)
-    if n_max > PAIRS_EXACT_MAX_N:
-        raise ValueError("an instance has %d customers; the exact pool takes at most %d" % (n_max, PAIRS_EXACT_MAX_N))
-    cap = n_max // 2
-    arena = _Arena(eng.device, [(B * cap * 4, torch.int32), (B, torch.int32), (B, torch.int64)])
-    rows_v, np_v, cost_v = arena.views
-    eng.pool_pairs_exact_batch(frm, to, sizes, offsets, n_max, d, accept_all, max_loss,
-                               out={"rows": rows_v.view(B, cap, 4), "n_pairs": np_v, "cost": cost_v})
-    rows, npairs, _ = arena.host()                                 # the one read-back of the batch
-    rows = rows.reshape(B, cap, 4)
-    return [None if npairs[b] < 0 else rows[b, : int(npairs[b])].copy() for b in range(B)]
+    return _find_pairs_batches(instances, dist, accept_all, max_loss, ("exact",))[0]
 
 
 def find_pool_pairs_exact(frm, to, dist, accept_all: bool = True, max_loss: float = 1.01):

@@ -368,15 +368,20 @@ def pool_greedy_vs_optimum(instances: Sequence, dist, accept_all: bool = True, m
     (Simulator.java:681-758) and by the optimal pairing (minimum cost among the pairings of maximum cardinality, the
     reference's ILP where it is feasible).  Returns [(greedy_count, greedy_cost, opt_count, opt_cost)] per case;
     opt_count >= greedy_count, and opt_cost <= greedy_cost where the counts are equal.  greedy(frm, to, dist, accept_all,
-    max_loss) and exact(instances, dist, accept_all, max_loss) -> row arrays are injectable (tests feed oracles); without
-    them the greedy runs per instance and the exact pool is one batched launch."""
+    max_loss) and exact(instances, dist, accept_all, max_loss) -> row arrays are injectable (tests feed oracles).  Without
+    them the whole experiment is one upload, one greedy and one exact batched launch, and one read-back."""
     from . import dispatch
-    greedy = greedy or dispatch.find_pool_pairs
-    exact = exact or dispatch.find_pool_pairs_exact_batch
-    opt = exact(instances, dist, accept_all, max_loss)
+    if greedy is None and exact is None:
+        grd, opt = dispatch._find_pairs_batches(instances, dist, accept_all, max_loss, ("greedy", "exact"))
+    else:
+        opt = (exact or dispatch.find_pool_pairs_exact_batch)(instances, dist, accept_all, max_loss)
+        if greedy is None:
+            grd = dispatch.find_pool_pairs_batch(instances, dist, accept_all, max_loss)
+        else:
+            grd = [greedy(f, t, dist, accept_all, max_loss) if len(f) >= 2 else np.zeros((0, 4), np.int32)
+                   for f, t in instances]
     out = []
-    for (f, t), o in zip(instances, opt):
-        g = greedy(f, t, dist, accept_all, max_loss) if len(f) >= 2 else np.zeros((0, 4), np.int32)
+    for g, o in zip(grd, opt):
         g, o = np.asarray(g).reshape(-1, 4), np.asarray(o).reshape(-1, 4)
         out.append((len(g), int(g[:, 3].astype(np.int64).sum()), len(o), int(o[:, 3].astype(np.int64).sum())))
     return out
