@@ -345,7 +345,9 @@ size_t td_pool_read_stats_bytes(void);
 
 /* findpool.c:83-108: concatenated shard survivors (shard order) -> sort on column 8 -> greedy
  * disjoint scan.  Reference quirk kept: for pool_size < 4 findpool.c sorts on a column it never
- * filled (findpool.c:34-35,70), so the scan runs in concatenation order. */
+ * filled (findpool.c:34-35,70), so the scan runs in concatenation order.
+ * Every merge entry point below checks the first pool_size columns of every valid row: a customer outside [0, n)
+ * makes *n_plans_out -1 and leaves plans_out untouched (the rows may come from the caller). */
 size_t td_pool_merge_workspace_bytes(int total_plans, int n);
 int td_pool_merge(const int32_t *shard_plans /* total x 9 */, int total_plans, int n, int pool_size,
                   int32_t *plans_out /* total x 9 */, int32_t *n_plans_out /* 1 */,

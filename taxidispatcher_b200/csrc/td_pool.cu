@@ -1275,6 +1275,8 @@ pool_emit_kernel(const PoolRec *__restrict__ kept_all, const PoolCtrl *ctrl, int
 // compaction runs in shared memory: a bitonic sort of the 64-bit scan keys, dominance rounds with the SORTED POSITION as
 // a 32-bit key (native shared-memory atomicMin on a per-customer table), a block scan for the output positions.
 // More rows take the general path (ranks by counting, state in the global workspace).
+// The rows may come from a caller, and both paths index a per-customer table with their customers: a valid row with a
+// customer outside [0, n) makes the merge write *n_plans_out = -1 and return before any such indexing.
 constexpr int kMergeSlots = 64;   // pool_merge ranks by binary search when it has at most this many (sorted) slots
 constexpr int kMergeFast = 8192;
 __global__ void __launch_bounds__(1024)
@@ -1294,10 +1296,10 @@ pool_merge_kernel(const int32_t *__restrict__ plans, int n_slots, int n, int K, 
     // rows stay a contiguous run -- the producer (pool_emit) writes them in ascending (cost, rank) order and the merge
     // below then needs no sort, only a rank by binary searches.  More slots: arrival order, sorted afterwards.
     __shared__ int s_off[kMergeSlots + 1];
-    __shared__ int s_unsorted;
+    __shared__ int s_unsorted, s_bad;
     const bool by_slot = n_slots <= kMergeSlots;
     auto count_of = [&](int slot) { return counts ? counts[slot] : (headed ? plans[size_t(slot) * slot_rows * TD_POOL_REC_W] : cap); };
-    if (tid == 0) { s_m = 0; s_unsorted = 0; }
+    if (tid == 0) { s_m = 0; s_unsorted = 0; s_bad = 0; }
     if (by_slot && tid < 32) {   // one warp: exclusive scan of the (clamped) counts
         int run = 0;
         for (int b0 = 0; b0 < n_slots; b0 += 32) {
@@ -1330,11 +1332,15 @@ pool_merge_kernel(const int32_t *__restrict__ plans, int n_slots, int n, int K, 
             const unsigned long long costpart = K == TD_POOL_MAX_IN_POOL ? (unsigned long long)(unsigned)row_ptr(ridx)[8] : 0ull;
             ckey[c] = (costpart << 32) | (unsigned long long)pos;   // pos < 2^32 (total <= 2^24 rows)
             crow[c] = ridx;
+            bool bad = false;
+            for (int q = 0; q < K; ++q) bad = bad || unsigned(row_ptr(ridx)[q]) >= unsigned(n);
+            if (bad) s_bad = 1;
             // a slot whose rows do not ascend (a caller's own rows) sends the merge through the sort
             if (by_slot && K == TD_POOL_MAX_IN_POOL && r > 0 && (unsigned)row_ptr(ridx - 1)[8] > (unsigned)costpart) s_unsorted = 1;
         }
     }
     __syncthreads();
+    if (s_bad) { if (tid == 0) *n_plans_out = -1; return; }   // uniform: read after the barrier
     if (by_slot && tid == 0) s_m = s_off[n_slots];
     __syncthreads();
     const int m = s_m;

@@ -441,8 +441,16 @@ class Engine:
         check(rc, "td_pool_find_shards_headed")
         return out
 
+    @staticmethod
+    def _merged_count(m: int, where: str) -> int:
+        """The merge's count, or TaxiDispatchError when it is -1 (a row names a customer outside [0, n))."""
+        if m < 0:
+            raise TaxiDispatchError(_lib.TD_ERR_INVALID, where, "a plan names a customer outside [0, n)")
+        return m
+
     def pool_merge_headed(self, blocks: torch.Tensor, slot_shard: Optional[torch.Tensor], n: int, pool_size: int):
-        """blocks [n_slots, cap + 1, 9] headed blocks (device).  Returns (plans, count) device tensors."""
+        """blocks [n_slots, cap + 1, 9] headed blocks (device).  Returns (plans, count) device tensors without a host round
+        trip; the count is -1 when a row names a customer outside [0, n)."""
         n_slots, cap = int(blocks.shape[0]), int(blocks.shape[1]) - 1
         total = n_slots * cap
         out = torch.empty((max(total, 1), POOL_REC_W), dtype=torch.int32, device=self.device)
@@ -467,7 +475,7 @@ class Engine:
         check(rc, "td_pool_merge_headed")
         pack[1 + keep: 1 + keep + n_slots] = blocks[:, 0, :]          # the headers ride along (a few hundred bytes)
         host = _d2h(pack[: 1 + keep + n_slots])
-        m = int(host[0, 0])
+        m = self._merged_count(int(host[0, 0]), "td_pool_merge_headed")
         counts, ev, fe = self.headers_host_view(host[1 + keep:])
         return host[1: 1 + m].copy(), counts, ev, fe
 
@@ -542,12 +550,14 @@ class Engine:
         rc = self.lib.td_pool_merge(_ptr(shard_plans), total, n, pool_size, _ptr(out), _ptr(cnt), _ptr(ws), ws.numel(),
                                     _stream())
         check(rc, "td_pool_merge")
+        self._merged_count(_d2h_int(cnt), "td_pool_merge")
         return out, cnt
 
 
     def pool_merge_padded(self, slot_plans: torch.Tensor, slot_counts: torch.Tensor, slot_shard: Optional[torch.Tensor],
                           n: int, pool_size: int):
-        """slot_plans [n_slots, cap, 9], slot_counts [n_slots] (device).  Returns (plans, count) device tensors."""
+        """slot_plans [n_slots, cap, 9], slot_counts [n_slots] (device).  Returns (plans, count) device tensors; waits for
+        the count and raises TaxiDispatchError when a row names a customer outside [0, n)."""
         n_slots, cap = int(slot_plans.shape[0]), int(slot_plans.shape[1])
         total = n_slots * cap
         out = torch.empty((max(total, 1), POOL_REC_W), dtype=torch.int32, device=self.device)
@@ -557,6 +567,7 @@ class Engine:
         rc = self.lib.td_pool_merge_padded(_ptr(slot_plans), _ptr(slot_counts), _ptr(slot_shard), n_slots, cap, n, pool_size,
                                            _ptr(out), _ptr(cnt), _ptr(ws), ws.numel(), _stream())
         check(rc, "td_pool_merge_padded")
+        self._merged_count(_d2h_int(cnt), "td_pool_merge_padded")
         return out, cnt
 
 
