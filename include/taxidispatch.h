@@ -334,6 +334,44 @@ int td_pool_pairs_batch(const int32_t *from, const int32_t *to, const int32_t *s
                         int32_t *pairs_out /* batch x (n_max/2) x 4 */, int32_t *n_pairs_out /* batch */,
                         int64_t *cost_out /* batch */, void *stream);
 
+/* ------------------------------------------------------------------------------------------
+ * The whole findpool job, batched: td_pool_find_shards over every logical shard + td_pool_merge, for many small
+ * demand sets in one launch
+ *
+ * Instance b is sizes[b] demand rows of 5 int32 (id, from, to, maxWait, maxLoss) starting at ROW offsets[b] of `demand`;
+ * the stand table dist (n_stands x n_stands, n_stands <= 128, every entry in [0, 2^22]) serves the whole batch.
+ * pool_size (2..4) and n_shards (1..64) hold for every instance.  Per instance the call does what tdh_pool_find_all does:
+ * the n_shards logical shards of pool_n.c:226-229, each with its own greedy dedup, then the findpool.c:83-108 merge in
+ * shard order with the td_pool_merge quirk (K = 4: scan in (cost, concatenation position) order; K < 4: concatenation
+ * order).  Ties are broken exactly as the reference breaks them, so every result depends on the instance alone: not on
+ * its position, its neighbours or n_max.
+ *   plans_out[b]      n_max / pool_size + 1 rows x 9 in the pool_n.c:123-134 layout (row indices of the instance's own
+ *                     demand rows), merged, in findpool order; unused rows -1
+ *   n_plans_out[b]    merged count; -1: withdrawn; -2: a shard's record slice was too small (rows -1)
+ *   evaluated_out / feasible_out / kept_out [b * n_shards + s]   per logical shard: pool_n.c count_all, pool_count and
+ *                     the survivors of its dedup (kept -1 for a shard whose slice was too small; all 0 when withdrawn)
+ *   needed_out[b]     the largest per-shard count of materialised records (one per pickup tuple with a feasible drop-off
+ *                     order); always written, so a rerun with records_per_shard = needed_out fits
+ * The workspace holds records_per_shard 8-byte records per (instance, shard): td_pool_batch_workspace_bytes(batch,
+ * n_shards, records_per_shard).  A shard that fills its slice stops writing but keeps enumerating and counting; only
+ * its own instance comes back -2.
+ *
+ * One CTA per (instance, shard), one launch, always asynchronous.  An instance with sizes[b] < 0 or > n_max, offsets[b]
+ * < 0 or a stand outside the table is withdrawn without touching its neighbours; a table entry outside [0, 2^22]
+ * withdraws every instance.  The arguments are checked before anything else: TD_ERR_INVALID for batch < 0, n_max outside
+ * [0, TD_POOL_BATCH_MAX_N], pool_size outside 2..4, n_shards outside [1, 64], n_stands outside [1, 128],
+ * records_per_shard outside [0, 2^31) or a NULL pointer with batch > 0; TD_ERR_WORKSPACE for a workspace smaller than
+ * td_pool_batch_workspace_bytes.
+ * ------------------------------------------------------------------------------------------ */
+#define TD_POOL_BATCH_MAX_N 512   /* 9 bits per customer: (cost, pickup tuple) is one exact 64-bit key */
+size_t td_pool_batch_workspace_bytes(int batch, int n_shards, int64_t records_per_shard);
+int td_pool_find_all_batch(const int32_t *demand, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                           const int32_t *dist, int n_stands, int pool_size, int n_shards,
+                           int32_t *plans_out /* batch x (n_max/pool_size + 1) x 9 */, int32_t *n_plans_out /* batch */,
+                           int64_t *evaluated_out /* batch x n_shards */, int64_t *feasible_out /* batch x n_shards */,
+                           int32_t *kept_out /* batch x n_shards */, int64_t *needed_out /* batch */,
+                           void *workspace, size_t workspace_bytes, int64_t records_per_shard, void *stream);
+
 /* After an ASYNCHRONOUS td_pool_find / td_pool_find_shards call (stats == NULL) on `workspace`: waits for the
  * stream and reads the per-shard counters back (one small copy).  *overflow_out != 0: the record list was too
  * small for a single pass -- counts_out holds -1 and the call has to be repeated synchronously (stats != NULL),

@@ -49,7 +49,7 @@
 // Roofline: the enumeration is INT32-issue + shared-memory-lookup bound; compulsory HBM traffic is
 // ~0.4 B per plan.  SURVEY.md section 8(d) defines the logical bytes used for the HBM-fraction
 // figure: 80 B per evaluated plan (4 customers x the 5-int32 demand record) + 36 B per feasible plan.
-#include "td_common.cuh"
+#include "td_pool_common.cuh"
 #include <string.h>
 #include <stdlib.h>
 
@@ -66,7 +66,6 @@ constexpr size_t kEnumWarpBytes = 256 * 4 + 3 * 32 * 16 + 64 * 8;   // histogram
 constexpr int kChunk = 128;       // records reserved per atomic
 constexpr int kSelThreads = 512;
 constexpr int kCustBits = 14;     // TD_POOL_MAX_CUSTOMERS = 16384
-constexpr int kPermBits = 5;
 
 struct PoolRec {                  // 16 bytes
     unsigned long long rank;      // p0 | p1 | p2 | p3 | perm  (unused pickup slots are 0)
@@ -121,7 +120,6 @@ __device__ __forceinline__ void split_rank(unsigned long long r, int p[4], int &
 }
 
 // ---- prep ----------------------------------------------------------------------------------------
-__device__ __forceinline__ int4 scale_cust_rt(int4 c, int sh);
 __device__ __forceinline__ void pool_prep_cust(int c, const int32_t *__restrict__ demand, int n, const int32_t *__restrict__ dist,
                                                int S, int4 *cust, int4 *cust_s, int sh, PoolCtrl *ctrl) {
     if (c >= n) return;
@@ -132,13 +130,7 @@ __device__ __forceinline__ void pool_prep_cust(int c, const int32_t *__restrict_
         f = 0; t = 0;
     }
     const int d = dist[size_t(f) * S + t];
-    // pool_n.c:115-116: ride > d * (1 + l/100.0), evaluated in fp64 with round-to-nearest, no contraction
-    const double lim = __dmul_rn(double(d), __dadd_rn(1.0, __ddiv_rn(double(l), 100.0)));
-    double fl = floor(lim);
-    int thr;
-    if (fl >= 2147483647.0) thr = INT_MAX;
-    else if (fl < -2147483647.0) thr = INT_MIN;
-    else thr = int(fl);
+    const int thr = pool_detour_thr(d, l);
     cust[c] = make_int4(f, t, thr, w);
     cust_s[c] = scale_cust_rt(make_int4(f, t, thr, w), sh);   // the enumeration's staged copy (fixed point of its evaluation)
 }
@@ -218,9 +210,7 @@ pool_build_lists_kernel(const int4 *__restrict__ cust, int n, const int32_t *__r
 
 
 // Stand-table check for every pool size: a negative entry (plan costs could go negative -- a negative cost marks a hole
-// in the record list) or an entry above kDistLimit (K = 4: the x32 fixed point of eval4s needs 7 legs x 32 < 2^31; K = 2, 3:
-// the (cost << 5 | permutation) order key needs 5 legs < 2^26) is refused with TD_ERR_INVALID, never clamped.
-constexpr int kDistLimit = 1 << 22;
+// in the record list) or an entry above kDistLimit is refused with TD_ERR_INVALID, never clamped.
 __device__ __forceinline__ void pool_check_table(int block, int blocks, const int32_t *__restrict__ dist, long long cells,
                                                  PoolCtrl *ctrl, int32_t *dist_s, int sh) {
     int bad = 0;
@@ -350,14 +340,6 @@ __device__ __forceinline__ int4 scale_cust(int4 c) {
     }
     return c;
 }
-__device__ __forceinline__ int4 scale_cust_rt(int4 c, int sh) {
-    if (sh > 0) {
-        const int lim = 1 << 25;
-        const int z = c.z > lim ? lim : (c.z < -lim ? -lim : c.z);
-        c.z = (z << sh) | ((1 << sh) - 1);
-    }
-    return c;
-}
 template <bool kCustSmem, int SH>
 struct CustView {
     const int4 *p;
@@ -405,61 +387,6 @@ __device__ __forceinline__ void emit_records(const EnumArgs &a, WarpOut &wo, boo
         *reinterpret_cast<int4 *>(a.recs + pos) = *reinterpret_cast<int4 *>(&r);
     }
     wo.used += need;
-}
-
-// K = 4, fixed point x32: every distance is pre-multiplied by kSh4 = 32 (the tables are staged that way), the slacks are
-// 32 * slack + 31, and a leaf's key is  32 * (drop legs) + permutation index  -- ONE three-input add per leaf gives both the
-// last partial sum and the (cost, permutation) order key, and  key <= sl  is exactly  legs <= slack  because the index is
-// below 32.  e[i] = D(F3,T_i); t[i][j] = D(T_i,T_j); sl[i] from thr_i - (pickup legs from i to the last pickup).
-constexpr int kSh4 = 5;
-__device__ __forceinline__ void eval4s(const int e[4], const int t[4][4], const int sl[4], int &nfeas, int &best) {
-    nfeas = 0; best = INT_MAX;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int d0 = e[i];
-        const bool ok0 = d0 <= sl[i];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            if (j == i) continue;
-            const int d1 = d0 + t[i][j];
-            const bool ok1 = ok0 && d1 <= sl[j];
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                if (k == i || k == j) continue;
-                const int l = 6 - i - j - k;
-                const int d2 = d1 + t[j][k];
-                // lexicographic permutation index (pool_n.c:137-150 order)
-                const int rj = j - (j > i);
-                const int rk = k - (k > i) - (k > j);
-                const int perm = i * 6 + rj * 2 + rk;
-                const int key = d2 + t[k][l] + perm;
-                const bool ok = ok1 && d2 <= sl[k] && key <= sl[l];
-                nfeas += ok;
-                best = (ok && key < best) ? key : best;
-            }
-        }
-    }
-}
-__device__ __forceinline__ void eval3(const int e[3], const int t[3][3], const int sl[3], int pick_sum, int &nfeas,
-                                      int &best) {
-    nfeas = 0; best = INT_MAX;
-#pragma unroll
-    for (int i = 0; i < 3; ++i) {
-        const int d0 = e[i];
-        const bool ok0 = d0 <= sl[i];
-#pragma unroll
-        for (int j = 0; j < 3; ++j) {
-            if (j == i) continue;
-            const int k = 3 - i - j;
-            const int d1 = d0 + t[i][j];
-            const int d2 = d1 + t[j][k];
-            const bool ok = ok0 && d1 <= sl[j] && d2 <= sl[k];
-            const int perm = i * 2 + (j - (j > i));
-            const int key = ((pick_sum + d2) << kPermBits) | perm;
-            nfeas += ok;
-            best = (ok && key < best) ? key : best;
-        }
-    }
 }
 
 // kPF (K = 4 with the stand table in shared memory): the closure D* is staged next to the table and the lower bound of

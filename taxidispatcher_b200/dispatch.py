@@ -12,6 +12,7 @@ Host functions mirror the reference's names, argument order and return layouts
   solve_batch(costs) / LCM_batch(costs, ...)       heuristic.py:20-40, python.py:6-25 over many instances
   find_pool(...) / find_pool_all(...) / pool_merge(...)   pool_n.c / findpool.c
   find_pool_pairs_batch(...)                       Simulator.findPool over many instances in one launch
+  find_pool_all_batch(...)                         the whole findpool job over many small demand sets in one launch
   find_pool_pairs_exact(...) / find_pool_pairs_exact_batch(...)   the optimum of pool_optimum.py / pool_opt_min.py
 
 PyTorch is used only for device buffers, pinned staging and streams.  All arithmetic runs in the
@@ -32,7 +33,7 @@ from ._lib import BIG_COST, INT32_MAX, PAIRS_EXACT_MAX_N, POOL_REC_W, AssignStat
 
 __all__ = ["BIG_COST", "Engine", "calculate_cost", "solve", "solve_dispatch", "solve_full", "solve_assignment", "LCM", "LCM_heuristic",
            "LCM_split", "LCM_greedy_opt", "LCM_simulate", "LCM_java", "find_pool", "find_pool_all", "find_pool_block",
-           "find_pool_pairs", "find_pool_pairs_batch", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "pool_merge", "pack_batch", "pack_cost_matrices", "run_packed", "run_batch", "solve_batch", "LCM_batch",
+           "find_pool_pairs", "find_pool_pairs_batch", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "find_pool_all_batch", "pack_pool_batch", "pool_merge", "pack_batch", "pack_cost_matrices", "run_packed", "run_batch", "solve_batch", "LCM_batch",
            "TaxiDispatchError"]
 
 
@@ -541,6 +542,28 @@ class Engine:
                                           _ptr(npairs), _ptr(cost), _stream())
         check(rc, "td_pool_pairs_batch")
         return rows, npairs, cost
+
+    def pool_find_all_batch(self, demand: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor, n_max: int,
+                            dist: torch.Tensor, pool_size: int, n_shards: int = 8, records_per_shard: int = 4096,
+                            out: Optional[dict] = None):
+        """The findpool job (every logical shard + the merge) of every instance (sizes[b] demand rows of 5 int32 at row
+        offsets[b] of `demand`), one launch.  Returns device tensors (plans [B, n_max // pool_size + 1, 9] int32, n_plans
+        [B] int32 (-1 withdrawn, -2 records_per_shard too small), evaluated / feasible [B, n_shards] int64, kept
+        [B, n_shards] int32, needed [B] int64).  `out` may supply any of them by name."""
+        B = int(sizes.numel())
+        plans = self._batch_out(out, "plans", (B, n_max // pool_size + 1, POOL_REC_W), torch.int32)
+        n_plans = self._batch_out(out, "n_plans", (B,), torch.int32)
+        evaluated = self._batch_out(out, "evaluated", (B, n_shards), torch.int64)
+        feasible = self._batch_out(out, "feasible", (B, n_shards), torch.int64)
+        kept = self._batch_out(out, "kept", (B, n_shards), torch.int32)
+        needed = self._batch_out(out, "needed", (B,), torch.int64)
+        ws = self._workspace("pool_batch", self.lib.td_pool_batch_workspace_bytes(B, int(n_shards), int(records_per_shard)))
+        rc = self.lib.td_pool_find_all_batch(_ptr(demand), _ptr(sizes), _ptr(offsets), B, int(n_max), _ptr(dist),
+                                             int(dist.shape[0]), int(pool_size), int(n_shards), _ptr(plans), _ptr(n_plans),
+                                             _ptr(evaluated), _ptr(feasible), _ptr(kept), _ptr(needed), _ptr(ws), ws.numel(),
+                                             int(records_per_shard), _stream())
+        check(rc, "td_pool_find_all_batch")
+        return plans, n_plans, evaluated, feasible, kept, needed
 
     def pool_merge(self, shard_plans: torch.Tensor, total: int, n: int, pool_size: int):
         out = torch.empty((max(total, 1), POOL_REC_W), dtype=torch.int32, device=self.device)
@@ -1200,3 +1223,150 @@ def find_pool_all(demand, dist, pool_size: int, n_shards: int = 8):
     m = _d2h_int(cnt)
     stats["kept"] = m
     return _d2h(merged[:m]), stats
+
+
+POOL_BATCH_MAX_N = _lib.POOL_BATCH_MAX_N
+# find_pool_all_batch sends K = 4 instances above this size through find_pool_all.  One CTA per (instance, shard) runs a
+# shard's whole enumeration, while find_pool_all spreads one instance over the GPU.  Measured on one NVIDIA B200 at 1000 W
+# (profiles/pool_batch_b200.json): 8 x 512 customers take 65.7 ms in the batch kernel against 4.5 ms for the loop of
+# find_pool_all; 148 x 300 customers take 30.9 ms against 38.8 ms.  Sizes in between were not measured.
+POOL_BATCH_K4_LOOP_N = 300
+# Record slices one find_pool_all_batch call may allocate (bytes).  A batch whose rerun would need more goes through
+# find_pool_all instance by instance instead.
+POOL_BATCH_RECORD_BUDGET = 4 << 30
+POOL_BATCH_FIRST_RECORDS = 4096      # records per shard of the first call of a shape (1000 x 100 customers, K = 4: 1778)
+_POOL_BATCH_RPS = {}                 # (pool_size, n_shards, n_max rounded up to a power of two) -> largest slice needed so far
+
+
+def pack_pool_batch(instances: Sequence, dist):
+    """[demand n x 5] host arrays + the stand table -> (demand, sizes, offsets, n_max, dist) on the device for
+    Engine.pool_find_all_batch: instance b is sizes[b] rows at row offsets[b] of `demand`.  Every part travels in ONE
+    pinned buffer and ONE host->device copy."""
+    dems = [np.asarray(d, dtype=np.int32).reshape(-1, 5) for d in instances]
+    d = np.ascontiguousarray(np.asarray(dist, dtype=np.int32))
+    B = len(dems)
+    sizes = np.array([len(x) for x in dems], dtype=np.int32)
+    offsets = np.zeros(B, dtype=np.int64)
+    rows = 0
+    for b, x in enumerate(dems):
+        offsets[b] = rows
+        rows += len(x)
+    meta = (rows * 5 + 1) & ~1                            # sizes start here; offsets at an even int32 index (int64 view)
+    off_at = (meta + B + 1) & ~1
+    dist_at = (off_at + 2 * B + 3) & ~3
+    words = max(dist_at + d.size, 4)
+    COPIED["h2d"] += words * 4
+    bucket = 1 << max(8, int(words - 1).bit_length())
+    key = ("pool_batch", bucket)
+    slot = _PINNED.get(key) if bucket <= (1 << 24) else None
+    if slot is None:
+        slot = {"buf": torch.empty(bucket, dtype=torch.int32).pin_memory(), "ev": None}
+        if bucket <= (1 << 24):
+            _PINNED[key] = slot
+    if slot["ev"] is not None:
+        slot["ev"].synchronize()
+    host = slot["buf"].numpy()
+    for x, o in zip(dems, offsets):
+        host[5 * o: 5 * o + x.size] = x.reshape(-1)
+    host[meta: meta + B] = sizes
+    host[off_at: off_at + 2 * B] = offsets.view(np.int32)
+    host[dist_at: dist_at + d.size] = d.reshape(-1)
+    dev = slot["buf"][:words].to("cuda", non_blocking=True)
+    ev = torch.cuda.Event()
+    ev.record()
+    slot["ev"] = ev
+    n_max = int(sizes.max()) if B else 0
+    return (dev[: max(rows, 1) * 5].view(-1, 5), dev[meta: meta + B], dev[off_at: off_at + 2 * B].view(torch.int64), n_max,
+            dev[dist_at: dist_at + d.size].reshape(d.shape))
+
+
+def pool_batch_routes(sizes: Sequence[int], pool_size: int):
+    """Indices of the instances find_pool_all_batch runs in the batched kernel and of those it sends through
+    find_pool_all: above POOL_BATCH_MAX_N customers, or above POOL_BATCH_K4_LOOP_N at K = 4."""
+    limit = POOL_BATCH_K4_LOOP_N if pool_size == 4 else POOL_BATCH_MAX_N
+    small = [i for i, n in enumerate(sizes) if n <= limit]
+    large = [i for i, n in enumerate(sizes) if n > limit]
+    return small, large
+
+
+def pool_batch_records(batch: int, n_shards: int, needed: int, budget: int = POOL_BATCH_RECORD_BUDGET):
+    """Records per shard for a batch call whose largest shard materialises `needed` records, or None when the record
+    slices of `batch` instances would exceed `budget` bytes."""
+    rps = max(int(needed), 1)
+    return rps if batch * n_shards * rps * 8 <= budget else None
+
+
+def _pool_batch_call(dems: Sequence, dist_np: np.ndarray, pool_size: int, n_shards: int, rps: int):
+    """One upload, one launch, one read-back.  Per instance (n_plans, plans, stats, needed)."""
+    eng = engine()
+    B = len(dems)
+    demand, sizes, offsets, n_max, d = pack_pool_batch(dems, dist_np)
+    rows = n_max // pool_size + 1
+    arena = _Arena(eng.device, [(B * rows * POOL_REC_W, torch.int32), (B, torch.int32), (B * n_shards, torch.int64),
+                                (B * n_shards, torch.int64), (B * n_shards, torch.int32), (B, torch.int64)])
+    v = arena.views
+    eng.pool_find_all_batch(demand, sizes, offsets, n_max, d, pool_size, n_shards, rps,
+                            out={"plans": v[0].view(B, rows, POOL_REC_W), "n_plans": v[1], "evaluated": v[2].view(B, n_shards),
+                                 "feasible": v[3].view(B, n_shards), "kept": v[4].view(B, n_shards), "needed": v[5]})
+    plans, n_plans, ev, fe, kept, needed = arena.host()
+    plans, ev, fe, kept = plans.reshape(B, rows, POOL_REC_W), ev.reshape(B, n_shards), fe.reshape(B, n_shards), \
+        kept.reshape(B, n_shards)
+    out = []
+    for b in range(B):
+        m = int(n_plans[b])
+        stats = {"evaluated": int(ev[b].sum()), "feasible": int(fe[b].sum()), "kept_per_shard": [int(c) for c in kept[b]],
+                 "kept": m}
+        out.append((m, plans[b, : max(m, 0)].copy(), stats, int(needed[b])))
+    return out
+
+
+def _find_pool_all_or_none(dem, dist_np, pool_size: int, n_shards: int):
+    try:
+        plans, stats = find_pool_all(dem, dist_np, pool_size, n_shards)
+    except TaxiDispatchError as e:
+        if e.code != _lib.TD_ERR_INVALID:
+            raise
+        return None
+    stats.pop("rounds", None)
+    return plans, stats
+
+
+def find_pool_all_batch(instances: Sequence, dist, pool_size: int, n_shards: int = 8):
+    """find_pool_all for every demand set (n x 5 rows) over one stand table.  Returns per instance exactly the plans and
+    the evaluated / feasible / kept_per_shard / kept counters find_pool_all gives (its internal `rounds` is not
+    reported), or None for an instance the library withdrew (a stand outside the table, or a table entry outside
+    [0, 2^22]).  Instances of up to POOL_BATCH_MAX_N customers (POOL_BATCH_K4_LOOP_N at K = 4) run in one batched launch;
+    larger ones, and a rerun that would exceed POOL_BATCH_RECORD_BUDGET, go through find_pool_all.  The result does not
+    depend on the route."""
+    if not 1 <= n_shards <= 64:
+        raise ValueError("find_pool_all_batch takes 1 to 64 shards, got %d" % n_shards)
+    dist_np = np.ascontiguousarray(np.asarray(dist, dtype=np.int32))
+    dems = [np.asarray(d, dtype=np.int32).reshape(-1, 5) for d in instances]
+    results = [None] * len(dems)
+    small, large = pool_batch_routes([len(x) for x in dems], pool_size)
+    for i in large:
+        results[i] = _find_pool_all_or_none(dems[i], dist_np, pool_size, n_shards)
+    if not small:
+        return results
+    n_max = max(len(dems[i]) for i in small)
+    key = (pool_size, n_shards, 1 << max(n_max - 1, 0).bit_length())
+    rps = _POOL_BATCH_RPS.get(key, POOL_BATCH_FIRST_RECORDS)
+    rps = max(1, min(rps, POOL_BATCH_RECORD_BUDGET // (8 * n_shards * len(small))))
+    redo = []
+    for i, (m, plans, stats, needed) in zip(small, _pool_batch_call([dems[i] for i in small], dist_np, pool_size, n_shards, rps)):
+        if m == -2:
+            redo.append((i, needed))
+        elif m >= 0:
+            results[i] = (plans, stats)
+    if redo:
+        need = max(nd for _, nd in redo)
+        _POOL_BATCH_RPS[key] = max(_POOL_BATCH_RPS.get(key, 0), need)
+        rps = pool_batch_records(len(redo), n_shards, need)
+        if rps is None:
+            for i, _ in redo:
+                results[i] = _find_pool_all_or_none(dems[i], dist_np, pool_size, n_shards)
+        else:
+            idx = [i for i, _ in redo]
+            for i, (m, plans, stats, _) in zip(idx, _pool_batch_call([dems[i] for i in idx], dist_np, pool_size, n_shards, rps)):
+                results[i] = (plans, stats) if m >= 0 else None
+    return results
