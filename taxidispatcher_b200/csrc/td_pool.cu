@@ -42,7 +42,11 @@
 //                      Records are processed in ascending cost bands (the cheap plans kill most customers before the
 //                      bulk of the list is looked at), the active list is fragmented over the CTAs, and a warp folds
 //                      the keys of consecutive records that share a customer into ONE atomicMin (per-run minima).
-//   pool_emit          kept plans in key order -> 9-int records of pool_n.c:123-134
+//                      Record format: when every plan cost provably fits beside the customers packed with
+//                      cb = ceil(log2 n) bits each (key64_fits, decided on the device from max W + max thr before the
+//                      enumeration), a record IS its 8-byte single-level key (cost | p0 | p1 | p2 | p3 | perm); otherwise
+//                      it is a 16-byte PoolRec and the keys come from rec_key1 / rec_hi.  Kept plans are PoolRec either way.
+//   pool_emit         kept plans in key order -> 9-int records of pool_n.c:123-134
 //   pool_merge         findpool.c:83-108: the shard outputs are sorted runs, so the global order is a rank by binary
 //                      searches (bitonic sort for rows in any other order), then the same dominance rounds in shared memory
 //
@@ -104,7 +108,32 @@ struct PoolCtrl {
     unsigned int act_cnt[kMaxBands][2];          // live in-band records, ping-pong between rounds
     unsigned long long hist[kMaxSlots][kBuckets];   // plans per min(cost, kBuckets-1), filled by pool_enum (64-bit: the
                                                     // counts include plans beyond the materialised cost window)
+    // ---- set once per call by pool_prepare / pool_build_lists, outside the per-pass reset (see key64_fits) ----
+    int max_wait, max_thr;        // max(W, 0) and max(thr, 0) over the customers
+    unsigned int key64;           // 1: the record list holds 8-byte keys, 0 (a zeroed block, td_pool_pairs): PoolRec
 };
+
+// Bits per customer index in the single-level key (selection) and in the 8-byte records: cb = ceil(log2 n), at least 1.
+__host__ __device__ __forceinline__ int key_cb(int n) {
+    int cb = 1;
+    while ((1 << cb) < n) ++cb;
+    return cb;
+}
+
+// The 8-byte record format: (cost, p0, p1, p2, p3, perm) packed as cost | cb bits x 4 | kPermBits, i.e. the single-level key
+// of the selection itself.  It is exact when every materialised cost is below 2^(64 - 4 cb - kPermBits), and that follows
+// from the input alone.  A plan's cost is its pickup legs plus its drop-off legs.  The pickup legs are at most W of its last
+// pickup: the wait rule admits a pickup only while the cumulative pickup distance is within its W.  The drop-off legs are at
+// most the ride of the passenger dropped last, which the detour rule bounds by its thr.  So every feasible plan costs at
+// most max(W, 0) + max(thr, 0) over the customers, and costs are never negative (pool_check_table refuses negative table
+// entries for every K), so the cost field needs no sign.  n <= 16384 leaves at least 3 cost bits.
+__device__ __forceinline__ unsigned key64_fits(int n, int max_wait, int max_thr) {
+    const int cost_bits = 64 - 4 * key_cb(n) - kPermBits;
+    if (cost_bits < 1) return 0u;
+    if (cost_bits >= 33) return 1u;
+    return (unsigned long long)max_wait + (unsigned long long)max_thr < (1ull << cost_bits) ? 1u : 0u;
+}
+constexpr unsigned long long kKeyHole = ~0ull;   // no valid key: perm <= 23 never fills the permutation field
 
 __device__ __forceinline__ unsigned long long make_rank(int p0, int p1, int p2, int p3, int perm) {
     return ((((((unsigned long long)p0 << kCustBits) | (unsigned)p1) << kCustBits | (unsigned)p2) << kCustBits |
@@ -118,21 +147,45 @@ __device__ __forceinline__ void split_rank(unsigned long long r, int p[4], int &
     p[1] = int(r & m); r >>= kCustBits;
     p[0] = int(r & m);
 }
+// Single-level key: (cost, rank) in ONE 64-bit word, rank repacked with cb = key_cb(n) bits per customer.  Exact when
+// cost < 2^(64 - 4 cb - kPermBits).  Order-preserving: lexicographic (cost, p0, p1, p2, p3, perm).
+__device__ __forceinline__ unsigned long long pack_key1(int cost, unsigned long long rank, int cb) {
+    const unsigned m = (1u << kCustBits) - 1;
+    const unsigned perm = unsigned(rank) & ((1u << kPermBits) - 1); rank >>= kPermBits;
+    const unsigned p3 = unsigned(rank) & m; rank >>= kCustBits;
+    const unsigned p2 = unsigned(rank) & m; rank >>= kCustBits;
+    const unsigned p1 = unsigned(rank) & m; rank >>= kCustBits;
+    const unsigned p0 = unsigned(rank) & m;
+    unsigned long long k = (unsigned long long)(unsigned)cost;
+    k = (k << cb) | p0; k = (k << cb) | p1; k = (k << cb) | p2; k = (k << cb) | p3;
+    return (k << kPermBits) | perm;
+}
 
 // ---- prep ----------------------------------------------------------------------------------------
 __device__ __forceinline__ void pool_prep_cust(int c, const int32_t *__restrict__ demand, int n, const int32_t *__restrict__ dist,
                                                int S, int4 *cust, int4 *cust_s, int sh, PoolCtrl *ctrl) {
-    if (c >= n) return;
-    int f = demand[c * 5 + 1], t = demand[c * 5 + 2];
-    const int w = demand[c * 5 + 3], l = demand[c * 5 + 4];
-    if (f < 0 || f >= S || t < 0 || t >= S) {   // pool_n.c:106-134 would index cost[][] out of bounds: refuse the input
-        ctrl->bad_input = 1;
-        f = 0; t = 0;
+    int w_pos = 0, thr_pos = 0;
+    if (c < n) {
+        int f = demand[c * 5 + 1], t = demand[c * 5 + 2];
+        const int w = demand[c * 5 + 3], l = demand[c * 5 + 4];
+        if (f < 0 || f >= S || t < 0 || t >= S) {   // pool_n.c:106-134 would index cost[][] out of bounds: refuse the input
+            ctrl->bad_input = 1;
+            f = 0; t = 0;
+        }
+        const int d = dist[size_t(f) * S + t];
+        const int thr = pool_detour_thr(d, l);
+        cust[c] = make_int4(f, t, thr, w);
+        cust_s[c] = scale_cust_rt(make_int4(f, t, thr, w), sh);   // the enumeration's staged copy (fixed point of its evaluation)
+        w_pos = w > 0 ? w : 0;
+        thr_pos = thr > 0 ? thr : 0;
     }
-    const int d = dist[size_t(f) * S + t];
-    const int thr = pool_detour_thr(d, l);
-    cust[c] = make_int4(f, t, thr, w);
-    cust_s[c] = scale_cust_rt(make_int4(f, t, thr, w), sh);   // the enumeration's staged copy (fixed point of its evaluation)
+    // the cost bound of the 8-byte records (key64_fits); the whole CTA prepares customers, so every lane is here
+    w_pos = __reduce_max_sync(0xffffffffu, w_pos);
+    thr_pos = __reduce_max_sync(0xffffffffu, thr_pos);
+    if ((threadIdx.x & 31) == 0) {
+        if (w_pos) atomicMax(&ctrl->max_wait, w_pos);
+        if (thr_pos) atomicMax(&ctrl->max_thr, thr_pos);
+    }
 }
 
 // one CTA per stand: counting sort of the customers reachable from this stand by slack, descending
@@ -201,7 +254,10 @@ pool_build_lists_kernel(const int4 *__restrict__ cust, int n, const int32_t *__r
         for (int o = 1; o < 32; o <<= 1) { const unsigned v = __shfl_up_sync(0xffffffffu, incl, o); if (threadIdx.x >= o) incl += v; }
         unsigned acc = incl - mine;
         for (int k = 0; k < 8; ++k) { const unsigned v = s_part[threadIdx.x * 8 + k]; s_part[threadIdx.x * 8 + k] = acc; acc += v; }
-        if (threadIdx.x == 31) { item_off[nl] = incl; ctrl->n_items = incl; }
+        if (threadIdx.x == 31) {
+            item_off[nl] = incl; ctrl->n_items = incl;
+            ctrl->key64 = key64_fits(n, ctrl->max_wait, ctrl->max_thr);   // pool_prepare has ended: the maxima are final
+        }
     }
     __syncthreads();
     unsigned run = s_part[threadIdx.x];
@@ -309,8 +365,9 @@ pool_prepare_kernel(const int32_t *__restrict__ demand, int n, const int32_t *__
 struct EnumArgs {
     // cust_s, dist_s, dclose: copies in the fixed point of the evaluation (staged by bulk copy)
     const int4 *cust; const int4 *cust_s; const int32_t *dist; const int32_t *dist_s; const int32_t *dclose; const int32_t *list; const int32_t *slack; const int32_t *cnt;
-    const unsigned int *item_off; PoolRec *recs; PoolCtrl *ctrl;
-    int n, S, start, stop; unsigned int cap;
+    const unsigned int *item_off; PoolRec *recs; PoolCtrl *ctrl;   // recs: PoolRec or, when ctrl->key64, 8-byte keys
+    int n, S, start, stop; unsigned int cap;                       // cap: records of either format
+    int cb;                       // key_cb(n)
     int step, shard_begin;        // leader p0 belongs to call slot p0 / step - shard_begin
     // multi-pass support (large inputs): only plans with cost in [cost_lo, cost_hi) are materialised, customers
     // whose alive flag is 0 (taken by an earlier cost window) are pruned at every pickup level
@@ -356,6 +413,14 @@ struct WarpOut {  // per-warp slice of the record list
     bool dead;    // the list overflowed: this warp stops materialising (counters and histogram stay exact)
 };
 
+// The record format (key64_fits), set by pool_build_lists before the enumeration and constant during it: loaded where a
+// record is written (read-only path, an L1 hit) rather than kept in a register across the enumeration loops.
+__device__ __forceinline__ bool rec_key64(const EnumArgs &a) { return __ldg(&a.ctrl->key64) != 0u; }
+__device__ __forceinline__ void mark_hole(const EnumArgs &a, bool k64, unsigned pos) {
+    if (k64) reinterpret_cast<unsigned long long *>(a.recs)[pos] = kKeyHole;
+    else a.recs[pos].cost = -1;
+}
+
 __device__ __forceinline__ void emit_records(const EnumArgs &a, WarpOut &wo, bool has, unsigned long long rank, int cost,
                                              int lane, unsigned *whist) {
     has = has && cost >= a.cost_lo;                 // earlier windows are done
@@ -367,7 +432,7 @@ __device__ __forceinline__ void emit_records(const EnumArgs &a, WarpOut &wo, boo
     if (wo.used + need > kChunk) {
         // abandon the rest of the current chunk (mark holes) and reserve a new one
         if (wo.base != 0xffffffffu)
-            for (unsigned t = wo.used + lane; t < kChunk; t += 32) a.recs[wo.base + t].cost = -1;
+            for (unsigned t = wo.used + lane; t < kChunk; t += 32) mark_hole(a, rec_key64(a), wo.base + t);
         unsigned nb = 0xffffffffu;
         // once the list has overflowed nobody reserves any more (the counter must not run away and wrap)
         if (lane == 0 && *reinterpret_cast<volatile unsigned *>(&a.ctrl->overflow) == 0)
@@ -383,8 +448,12 @@ __device__ __forceinline__ void emit_records(const EnumArgs &a, WarpOut &wo, boo
     if (wo.base == 0xffffffffu) return;
     if (has) {
         const unsigned pos = wo.base + wo.used + __popc(ball & ((1u << lane) - 1));
-        PoolRec r; r.rank = rank; r.cost = cost; r.pad = 0;
-        *reinterpret_cast<int4 *>(a.recs + pos) = *reinterpret_cast<int4 *>(&r);
+        if (rec_key64(a)) {
+            reinterpret_cast<unsigned long long *>(a.recs)[pos] = pack_key1(cost, rank, a.cb);
+        } else {
+            PoolRec r; r.rank = rank; r.cost = cost; r.pad = 0;
+            *reinterpret_cast<int4 *>(a.recs + pos) = *reinterpret_cast<int4 *>(&r);
+        }
     }
     wo.used += need;
 }
@@ -728,7 +797,7 @@ pool_enum_kernel(EnumArgs a) {
     }
     // close the last chunk (the queue was drained and the counters published when the item loop ended)
     if (wo.base != 0xffffffffu)
-        for (unsigned t = wo.used + lane; t < kChunk; t += 32) a.recs[wo.base + t].cost = -1;
+        for (unsigned t = wo.used + lane; t < kChunk; t += 32) mark_hole(a, rec_key64(a), wo.base + t);
 }
 
 // ---- selection -----------------------------------------------------------------------------------
@@ -777,21 +846,50 @@ __device__ __forceinline__ bool sel_run_min(int cell, unsigned long long &key, b
 __device__ __forceinline__ unsigned long long rec_hi(const PoolRec &r) {
     return ((unsigned long long)(unsigned)r.cost << 32) | (r.rank >> 32);
 }
-// Single-level key: (cost, rank) in ONE 64-bit word, rank repacked with cb = ceil(log2 n) bits per customer.  Usable when
-// max cost < 2^(64 - 4 cb - 5) (config 3: cb = 10, costs below 2^19); it removes the second-level pass, one grid barrier
-// and the best_lo lookups from every dominance round.  Order-preserving: lexicographic (cost, p0, p1, p2, p3, perm).
-__device__ __forceinline__ unsigned long long rec_key1(const PoolRec &r, int cb) {
-    const unsigned m = (1u << kCustBits) - 1;
-    unsigned long long rk = r.rank;
-    const unsigned perm = unsigned(rk) & ((1u << kPermBits) - 1); rk >>= kPermBits;
-    const unsigned p3 = unsigned(rk) & m; rk >>= kCustBits;
-    const unsigned p2 = unsigned(rk) & m; rk >>= kCustBits;
-    const unsigned p1 = unsigned(rk) & m; rk >>= kCustBits;
-    const unsigned p0 = unsigned(rk) & m;
-    unsigned long long k = (unsigned long long)(unsigned)r.cost;
-    k = (k << cb) | p0; k = (k << cb) | p1; k = (k << cb) | p2; k = (k << cb) | p3;
-    return (k << kPermBits) | perm;
-}
+// Single-level key of a PoolRec (pack_key1).  Usable when every materialised cost is below 2^(64 - 4 cb - 5) (config 3:
+// cb = 10, costs below 2^19); it removes the second-level pass, one grid barrier and the best_lo lookups from every
+// dominance round.
+__device__ __forceinline__ unsigned long long rec_key1(const PoolRec &r, int cb) { return pack_key1(r.cost, r.rank, cb); }
+
+// The two formats of the record list, for the passes of pool_select_body.  Both give a record's cost, customers and
+// first-level key; kept plans are stored as PoolRec either way (pool_emit reads those).
+struct RecFmt16 {                  // PoolRec: any cost; single-level or two-level keys, decided from the histogram
+    using R = PoolRec;
+    static constexpr bool kSingle = false;
+    static constexpr int kPartPer = 4, kFiltPer = 4;
+    __device__ static bool hole(const R &r) { return r.cost < 0; }
+    __device__ static R make_hole() { PoolRec r; r.rank = 0; r.cost = -1; r.pad = 0; return r; }
+    __device__ static int cost(const R &r, int) { return r.cost; }
+    __device__ static int lead(const R &r, int) { return int(r.rank >> (3 * kCustBits + kPermBits)); }
+    __device__ static void cust(const R &r, int, int p[4]) { int perm; split_rank(r.rank, p, perm); }
+    __device__ static unsigned long long key(const R &r, int cb, bool single) { return single ? rec_key1(r, cb) : rec_hi(r); }
+    __device__ static unsigned key_lo(const R &r) { return unsigned(r.rank); }
+    __device__ static PoolRec rec(const R &r, int) { return r; }
+};
+struct RecFmt8 {                   // the single-level key itself (key64_fits): no repacking, no second level
+    using R = unsigned long long;
+    static constexpr bool kSingle = true;
+    static constexpr int kPartPer = 4, kFiltPer = 4;
+    __device__ static bool hole(const R &r) { return r == kKeyHole; }
+    __device__ static R make_hole() { return kKeyHole; }
+    __device__ static int cost(const R &r, int cb) { return int(r >> (4 * cb + kPermBits)); }
+    __device__ static int lead(const R &r, int cb) { return int(r >> (3 * cb + kPermBits)) & ((1 << cb) - 1); }
+    __device__ static void cust(const R &r, int cb, int p[4]) {
+        const unsigned m = (1u << cb) - 1;
+        p[3] = int(unsigned(r >> kPermBits) & m);
+        p[2] = int(unsigned(r >> (cb + kPermBits)) & m);
+        p[1] = int(unsigned(r >> (2 * cb + kPermBits)) & m);
+        p[0] = int(unsigned(r >> (3 * cb + kPermBits)) & m);
+    }
+    __device__ static unsigned long long key(const R &r, int, bool) { return r; }
+    __device__ static unsigned key_lo(const R &) { return 0u; }
+    __device__ static PoolRec rec(const R &r, int cb) {
+        int p[4];
+        cust(r, cb, p);
+        PoolRec o; o.rank = make_rank(p[0], p[1], p[2], p[3], int(unsigned(r) & ((1u << kPermBits) - 1))); o.cost = cost(r, cb); o.pad = 0;
+        return o;
+    }
+};
 
 // Selection = the reference's sort-by-cost + greedy scan (pool_n.c:187-207), done as dominance rounds.
 // Cost is the leading key, so the scan over records with cost < t is a prefix of the whole scan:
@@ -804,8 +902,10 @@ __device__ __forceinline__ unsigned long long rec_key1(const PoolRec &r, int cb)
 //                   different shards never interact because their state is indexed by shard).
 // Each record is read ~3 times in total; the rounds touch only the live in-band records
 // (config 3: ~0.3 M record visits per shard instead of ~7.5 M x 3 passes on the unbanded list).
-__global__ void __launch_bounds__(kSelThreads, 2)   // 64 registers: two CTAs per SM keep the streaming passes fed
-pool_select_kernel(SelArgs a) {
+// F: the record format (RecFmt16 / RecFmt8) of list[], act[]; kept[] is PoolRec either way.
+template <class F>
+__device__ __forceinline__ void pool_select_body(const SelArgs &a) {
+    using R = typename F::R;
     cg::grid_group grid = cg::this_grid();
     const unsigned tid = blockIdx.x * blockDim.x + threadIdx.x;
     const unsigned nthreads = gridDim.x * blockDim.x;
@@ -813,10 +913,6 @@ pool_select_kernel(SelArgs a) {
     const int K = a.K;
     const int n = a.n;
     PoolCtrl *ctrl = a.ctrl;
-    // The record list overflowed (asynchronous single pass) or the input was refused: the histogram kept counting, so the
-    // band sizes exceed what was materialised -- nothing below may run.  Both flags are final when the enumeration has
-    // ended, every thread of the grid sees the same values and leaves before the first barrier; pool_emit reports -1.
-    if (ctrl->overflow || ctrl->bad_input) return;
     if (tid == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); ctrl->tstamp[31] = t; }
     __shared__ int s_band_hi[kMaxSlots][kMaxBands];
     const unsigned n_state = unsigned(n) * unsigned(a.n_slots);
@@ -865,12 +961,12 @@ pool_select_kernel(SelArgs a) {
     __syncthreads();
     // p0 / step without a division per record (step_inv == 0: step is 1)
     auto slot_of = [&](int p0) -> int { return (a.step_inv ? int(__umulhi(unsigned(p0), a.step_inv)) : p0) - a.shard_begin; };
-    // single-level keys when every materialised cost fits beside the repacked rank (uniform: from the histogram)
-    int cb = 1;
-    while ((1 << cb) < n) ++cb;
+    // single-level keys when every materialised cost fits beside the repacked rank (8-byte records: always; PoolRec:
+    // uniform, from the histogram)
+    const int cb = key_cb(n);
     const int cost_bits = 64 - 4 * cb - kPermBits;
-    bool single_key = cost_bits >= 1;
-    if (single_key) {
+    bool single_key = F::kSingle || cost_bits >= 1;
+    if (!F::kSingle && single_key) {
         const int lim = cost_bits >= 31 ? kBuckets - 1 : (int)min((long long)kBuckets - 1, 1ll << cost_bits);
         // every bucket at or above the limit (and the open-ended last bucket) must be empty
         for (int sl = 0; sl < a.n_slots && single_key; ++sl)
@@ -891,30 +987,31 @@ pool_select_kernel(SelArgs a) {
     // Block-aggregated: a CTA classifies kPartPer records per thread, counts them per band in shared memory,
     // reserves one contiguous range per band with ONE global atomic each, then scatters.
     {
-        constexpr int kPartPer = 4;
+        constexpr int kPartPer = F::kPartPer;
         __shared__ unsigned s_bcnt[kMaxBands], s_bbase[kMaxBands];
         const unsigned cnt = ctrl->overflow ? 0u : ctrl->n_records;
-        const PoolRec *src = a.list[0];
-        PoolRec *dst = a.list[1];
+        const R *src = reinterpret_cast<const R *>(a.list[0]);
+        R *dst = reinterpret_cast<R *>(a.list[1]);
         const unsigned chunk = blockDim.x * kPartPer;
         for (unsigned base = blockIdx.x * chunk; base < cnt; base += gridDim.x * chunk) {
             if (threadIdx.x < kMaxBands) s_bcnt[threadIdx.x] = 0;
             __syncthreads();
-            PoolRec r[kPartPer];
+            R r[kPartPer];
             int band[kPartPer];
             unsigned lrank[kPartPer];
 #pragma unroll
             for (int u = 0; u < kPartPer; ++u) {
                 const unsigned i = base + u * blockDim.x + threadIdx.x;
                 band[u] = -1;
-                if (i < cnt) r[u] = src[i]; else r[u].cost = -1;
+                r[u] = i < cnt ? src[i] : F::make_hole();
             }
 #pragma unroll
             for (int u = 0; u < kPartPer; ++u) {
-                if (r[u].cost < 0) continue;
-                const int slot = slot_of(int(r[u].rank >> (3 * kCustBits + kPermBits)));
+                if (F::hole(r[u])) continue;
+                const int slot = slot_of(F::lead(r[u], cb));
+                const int cost = F::cost(r[u], cb);
                 int bsel = 0;
-                while (r[u].cost >= s_band_hi[slot][bsel]) ++bsel;
+                while (cost >= s_band_hi[slot][bsel]) ++bsel;
                 band[u] = bsel;
             }
 #pragma unroll
@@ -948,12 +1045,13 @@ pool_select_kernel(SelArgs a) {
         // later pass of the band works on that fragment.  Only the totals (termination test), alive[] and the
         // per-customer minima are shared through global memory.
         __shared__ unsigned s_cnt;               // records in this CTA's fragment of the list being written
-        const size_t frag = size_t(blockIdx.x) * a.frag_cap;
+        // frag_cap counts PoolRec: an 8-byte fragment starts at the same byte and holds twice the records
+        const size_t frag = size_t(blockIdx.x) * a.frag_cap * (sizeof(PoolRec) / sizeof(R));
         unsigned my_cnt = 0;
         {
-            constexpr int kFiltPer = 4;
-            const PoolRec *src = a.list[1];
-            PoolRec *act = a.act[0] + frag;
+            constexpr int kFiltPer = F::kFiltPer;
+            const R *src = reinterpret_cast<const R *>(a.list[1]);
+            R *act = reinterpret_cast<R *>(a.act[0]) + frag;
             // records per thread and chunk: fewer for a small band, so that its live records (and with them the work of
             // the rounds, which stay on the fragments) spread over more CTAs
             const unsigned want = (b1 - b0 + nthreads - 1) / nthreads;
@@ -963,7 +1061,7 @@ pool_select_kernel(SelArgs a) {
             if (threadIdx.x == 0) s_cnt = 0;
             __syncthreads();
             for (unsigned base = b0 + blockIdx.x * chunk; base < b1; base += gridDim.x * chunk) {
-                PoolRec r[kFiltPer];
+                R r[kFiltPer];
                 bool live[kFiltPer];
                 int p[kFiltPer][4];
 #pragma unroll
@@ -975,8 +1073,7 @@ pool_select_kernel(SelArgs a) {
 #pragma unroll
                 for (int u = 0; u < kFiltPer; ++u) {
                     if (!live[u]) continue;
-                    int perm;
-                    split_rank(r[u].rank, p[u], perm);
+                    F::cust(r[u], cb, p[u]);
                     const int so = slot_of(p[u][0]) * n;
                     uint8_t fl[4];                       // the four flags are loaded together (no short-circuit chain)
 #pragma unroll
@@ -990,7 +1087,7 @@ pool_select_kernel(SelArgs a) {
                     unsigned wbase = 0;
                     if (lane == 0) wbase = atomicAdd(&s_cnt, __popc(ball));
                     wbase = __shfl_sync(0xffffffffu, wbase, 0);
-                    const unsigned long long hi = live[u] ? (single_key ? rec_key1(r[u], cb) : rec_hi(r[u])) : ~0ull;
+                    const unsigned long long hi = live[u] ? F::key(r[u], cb, single_key) : ~0ull;
                     unsigned long long rmin[3];
                     bool head[3];
 #pragma unroll
@@ -1034,19 +1131,19 @@ pool_select_kernel(SelArgs a) {
         unsigned al = 0;
         for (unsigned r = 0;; ++r) {
             if (r > 0) {   // pass A: drop the plans killed by the previous round, compact, first-level minima
-                const PoolRec *src = a.act[al] + frag;
-                PoolRec *dst = a.act[al ^ 1] + frag;
+                const R *src = reinterpret_cast<const R *>(a.act[al]) + frag;
+                R *dst = reinterpret_cast<R *>(a.act[al ^ 1]) + frag;
                 __syncthreads();
                 if (threadIdx.x == 0) s_cnt = 0;
                 __syncthreads();
                 for (unsigned base = 0; base < my_cnt; base += blockDim.x) {
                     const unsigned i = base + threadIdx.x;
                     bool live = false;
-                    PoolRec rec;
-                    int p[4], perm;
+                    R rec;
+                    int p[4];
                     if (i < my_cnt) {
                         rec = src[i];
-                        split_rank(rec.rank, p, perm);
+                        F::cust(rec, cb, p);
                         const int so = slot_of(p[0]) * n;
                         uint8_t fl[4];
 #pragma unroll
@@ -1058,7 +1155,7 @@ pool_select_kernel(SelArgs a) {
                     unsigned wbase = 0;
                     if (lane == 0) wbase = atomicAdd(&s_cnt, __popc(ball));
                     wbase = __shfl_sync(0xffffffffu, wbase, 0);
-                    const unsigned long long hi = live ? (single_key ? rec_key1(rec, cb) : rec_hi(rec)) : ~0ull;
+                    const unsigned long long hi = live ? F::key(rec, cb, single_key) : ~0ull;
                     unsigned long long rmin[3];
                     bool head[3];
 #pragma unroll
@@ -1086,16 +1183,16 @@ pool_select_kernel(SelArgs a) {
             }
             const unsigned n_act = ctrl->act_cnt[band][al];
             if (n_act == 0) break;
-            const PoolRec *cur = a.act[al] + frag;
+            const R *cur = reinterpret_cast<const R *>(a.act[al]) + frag;
             // pass B: second-level minimum among the plans that tie on the first level (two-level keys only)
             if (!single_key)
             for (unsigned i = threadIdx.x; i < my_cnt; i += blockDim.x) {
-                const PoolRec rec = cur[i];
-                int p[4], perm;
-                split_rank(rec.rank, p, perm);
+                const R rec = cur[i];
+                int p[4];
+                F::cust(rec, cb, p);
                 const int so = slot_of(p[0]) * n;
-                const unsigned long long hi = rec_hi(rec);
-                const unsigned lo = unsigned(rec.rank);
+                const unsigned long long hi = F::key(rec, cb, false);
+                const unsigned lo = F::key_lo(rec);
                 for (int q = 0; q < K; ++q)
                     if (a.best_hi[par][so + p[q]] == hi && lo < a.best_lo[par][so + p[q]]) atomicMin(&a.best_lo[par][so + p[q]], lo);
             }
@@ -1103,13 +1200,13 @@ pool_select_kernel(SelArgs a) {
             if (!single_key) grid.sync();
             // pass C: keep the plans that hold the minimum at every one of their customers
             for (unsigned i = threadIdx.x; i < my_cnt; i += blockDim.x) {
-                const PoolRec rec = cur[i];
-                int p[4], perm;
-                split_rank(rec.rank, p, perm);
+                const R rec = cur[i];
+                int p[4];
+                F::cust(rec, cb, p);
                 const int slot = slot_of(p[0]);
                 const int so = slot * n;
-                const unsigned long long hi = single_key ? rec_key1(rec, cb) : rec_hi(rec);
-                const unsigned lo = unsigned(rec.rank);
+                const unsigned long long hi = F::key(rec, cb, single_key);
+                const unsigned lo = F::key_lo(rec);
                 unsigned long long bh[4];
                 unsigned bl[4];
 #pragma unroll
@@ -1121,7 +1218,7 @@ pool_select_kernel(SelArgs a) {
                                  bl[0] == lo && bl[1] == lo && bl[2] == lo && bl[3] == lo;
                 if (dom) {
                     const unsigned pos = atomicAdd(&ctrl->n_kept[slot], 1u);
-                    a.kept[size_t(slot) * a.keep_cap + pos] = rec;
+                    a.kept[size_t(slot) * a.keep_cap + pos] = F::rec(rec, cb);
                     for (int q = 0; q < K; ++q) a.alive[so + p[q]] = 0;
                 }
             }
@@ -1134,6 +1231,17 @@ pool_select_kernel(SelArgs a) {
         stamp();
     }
     if (tid == 0) { ctrl->rounds = rounds; ctrl->total_rounds += rounds; }
+}
+
+__global__ void __launch_bounds__(kSelThreads, 2)   // 64 registers: two CTAs per SM keep the streaming passes fed
+pool_select_kernel(SelArgs a) {
+    // The record list overflowed (asynchronous single pass) or the input was refused: the histogram kept counting, so the
+    // band sizes exceed what was materialised -- nothing below may run.  Both flags are final when the enumeration has
+    // ended, every thread of the grid sees the same values and leaves before the first barrier; pool_emit reports -1.
+    // The record format is uniform as well (set by pool_build_lists; 0 in td_pool_pairs' zeroed block).
+    if (a.ctrl->overflow || a.ctrl->bad_input) return;
+    if (a.ctrl->key64) pool_select_body<RecFmt8>(a);
+    else pool_select_body<RecFmt16>(a);
 }
 
 // kept plans -> ascending (cost, rank) -> pool_n.c:123-134 records
@@ -1714,17 +1822,17 @@ static int pool_find_shards_impl(const int32_t *demand, int n, const int32_t *di
     while (sel_per_sm > 1 && sms * sel_per_sm > kSelMaxGrid) --sel_per_sm;
     if (sms * sel_per_sm < shard_count || sms * sel_per_sm > kSelMaxGrid) return TD_ERR_INVALID;
 
-    // the per-pass part of the control block (everything after pass_begin_marker)
+    // the per-pass part of the control block (from pass_begin_marker to the per-call tail that starts at max_wait)
     const size_t pass_off = offsetof(PoolCtrl, pass_begin_marker);
     auto reset_pass = [&]() -> int {
-        TD_CUDA_TRY(cudaMemsetAsync(reinterpret_cast<char *>(w.ctrl) + pass_off, 0, sizeof(PoolCtrl) - pass_off, st));
+        TD_CUDA_TRY(cudaMemsetAsync(reinterpret_cast<char *>(w.ctrl) + pass_off, 0, offsetof(PoolCtrl, max_wait) - pass_off, st));
         return TD_OK;
     };
     auto run_enum = [&](int cost_lo, int cost_hi, bool use_alive, bool count_stats, int stride) -> int {
         EnumArgs ea;
         ea.cust = w.cust; ea.cust_s = w.cust_s; ea.dist = dist; ea.dist_s = w.dist_s; ea.dclose = w.dclose; ea.list = w.list; ea.slack = w.slack; ea.cnt = w.cnt; ea.item_off = w.item_off;
         ea.recs = w.recs[0]; ea.ctrl = w.ctrl; ea.n = n; ea.S = n_stands; ea.start = start; ea.stop = stop;
-        ea.cap = unsigned(rec_cap64); ea.step = step; ea.shard_begin = shard_begin;
+        ea.cap = unsigned(rec_cap64); ea.step = step; ea.shard_begin = shard_begin; ea.cb = key_cb(n);
         ea.cost_lo = cost_lo; ea.cost_hi = cost_hi; ea.alive = use_alive ? w.alive : nullptr;
         ea.count_stats = count_stats ? 1 : 0; ea.item_stride = stride;
         ProfScope prof(TD_PROF_POOL_ENUM, st);
