@@ -238,7 +238,37 @@ int td_lcm_batch_cluster(const int32_t *costs, const int32_t *sizes, const int64
                          int32_t *last_min_out /* batch, may be NULL */, void *stream);
 
 /* ------------------------------------------------------------------------------------------
- * K4  pool finder           replaces one `pool_n <pool-size> <thread> <file> <n> <out>` process
+ * Batches of large instances (n <= TD_BATCH_LARGE_MAX_N)   heuristic.py's 2000 x 2000 LCM-vs-
+ *     optimum experiment, Simulator.java's 1300-row LCM model and perf.jl's 1000 x 1000 solve,
+ *     over many instances.
+ *
+ * Exactly the arguments, layout and semantics of the *_batch_cluster pair above (packed
+ * instances, output stride n_max, -1 / 0 fill, withdrawal of an instance with a bad size or
+ * offset, batch == 0 launches nothing, no workspace, always asynchronous), for 0 <= n_max <= 2048,
+ * small n_max included.  One launch per call; every instance runs on one thread-block cluster of
+ * K CTAs (K = 4 up to n_max 1024, 8 above: at most 256 columns / rows per CTA, one per thread)
+ * that keeps only the O(n) state in shared memory and reads the matrix from global memory.
+ * Returns TD_ERR_CUDA when no such cluster fits the device.
+ *
+ * The same algorithms as the *_batch_cluster pair, step for step: td_assign_exact_batch_large
+ * returns, for every instance of n <= 640, the identical col_of_row, u, v and objective as
+ * td_assign_exact_batch_cluster (and for n <= 232 as td_assign_exact_batch), an exact optimum with
+ * valid duals for every n, and results that do not depend on n_max or on the position in the
+ * batch.  td_lcm_batch_large returns the literal trace of td_lcm for every params.
+ * ------------------------------------------------------------------------------------------ */
+#define TD_BATCH_LARGE_MAX_N 2048    /* 8 CTAs x 256 columns / rows: one per thread */
+int td_assign_exact_batch_large(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                                int32_t *col_of_row_out /* batch x n_max */, int64_t *objective_out /* batch */,
+                                int64_t *u_out /* batch x n_max or NULL */, int64_t *v_out /* batch x n_max or NULL */,
+                                void *stream);
+int td_lcm_batch_large(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                       const td_lcm_params *params /* host, same for every instance */,
+                       int32_t *rows_out /* batch x n_max */, int32_t *cols_out /* batch x n_max */,
+                       int32_t *n_pairs_out /* batch */, int64_t *total_out /* batch */,
+                       int32_t *last_min_out /* batch, may be NULL */, void *stream);
+
+/* ------------------------------------------------------------------------------------------
+ * K4  pool finder          replaces one `pool_n <pool-size> <thread> <file> <n> <out>` process
  *     (pool_n.c:209-238): findPool :153-177, drop_customers :101-151, removeDuplicates :187-207,
  *     shard rule :226-229.
  *

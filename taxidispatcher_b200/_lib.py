@@ -20,6 +20,7 @@ BIG_COST = 250000
 PAIRS_EXACT_MAX_N = 4096    # TD_PAIRS_EXACT_MAX_N
 PAIRS_BATCH_MAX_N = 4096    # TD_PAIRS_BATCH_MAX_N
 POOL_BATCH_MAX_N = 512      # TD_POOL_BATCH_MAX_N
+BATCH_LARGE_MAX_N = 2048    # TD_BATCH_LARGE_MAX_N
 POOL_REC_W = 9
 PROF_COST, PROF_LCM, PROF_ASSIGN, PROF_POOL_ENUM, PROF_POOL_SELECT = range(5)
 
@@ -81,6 +82,8 @@ _SIGNATURES = {
     "td_lcm_batch": (_I, [c_vp, c_vp, c_vp, _I, _I, ctypes.POINTER(LcmParams), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "td_assign_exact_batch_cluster": (_I, [c_vp, c_vp, c_vp, _I, _I, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "td_lcm_batch_cluster": (_I, [c_vp, c_vp, c_vp, _I, _I, ctypes.POINTER(LcmParams), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "td_assign_exact_batch_large": (_I, [c_vp, c_vp, c_vp, _I, _I, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "td_lcm_batch_large": (_I, [c_vp, c_vp, c_vp, _I, _I, ctypes.POINTER(LcmParams), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "td_pool_workspace_bytes":(ctypes.c_size_t, [_I, _I, _I, ctypes.c_int64]),
     "td_pool_find": (_I, [c_vp, _I, c_vp, _I, _I, _I, _I, c_vp, ctypes.c_int32, c_vp, ctypes.POINTER(PoolStats),
                           c_vp, ctypes.c_size_t, ctypes.c_int64, c_vp]),

@@ -1,16 +1,31 @@
-// td_batch_cluster.cu -- batches of mid-size assignment and LCM instances (n <= TD_BATCH_CLUSTER_MAX_N = 640), one
-// thread-block cluster of K CTAs per instance, the instance held in the cluster's shared memory (DSMEM).
+// td_batch_cluster.cu -- batches of mid-size and large assignment and LCM instances, one thread-block cluster of K CTAs
+// per instance.  Two storage forms of the same two kernels (template parameter kGlobal):
 //
-// td_assign_exact_batch / td_lcm_batch (td_assign.cu, td_lcm.cu) keep one instance in ONE CTA's shared memory and stop at
-// 232 rows.  Here the n x n matrix is cut into K blocks, one per CTA of a portable cluster (K in {1, 2, 4, 8}); what the
-// single-CTA routines read from their own shared memory -- the row minima, the lowest asking column of a row, the level
-// minimum of a Dijkstra step, the rows that join the tree, the LCM arg-min -- is reduced or gathered across the cluster
-// through distributed shared memory.  K is the smallest count whose block fits one CTA next to its O(n) state, and it
-// depends on n_max only: 232 -> 1, 300 -> 2, 400 -> 4, 640 -> 8.
+//   DSMEM form   (td_*_batch_cluster, n <= TD_BATCH_CLUSTER_MAX_N = 640): the n x n matrix is cut into K blocks, one per
+//                CTA of a portable cluster (K in {1, 2, 4, 8}), and staged in the CTAs' shared memory.  K is the smallest
+//                count whose block fits one CTA next to its O(n) state: 232 -> 1, 300 -> 2, 400 -> 4, 640 -> 8.
+//   global form  (td_*_batch_large, n <= TD_BATCH_LARGE_MAX_N = 2048): the matrix stays in global memory (L2 / HBM) and
+//                only the O(n) state is on chip.  K is the smallest of {4, 8} with ceil(n_max / K) <= 256, so a thread
+//                owns at most one column (assignment) or one row (LCM): 4 up to 1024, 8 up to 2048.
 //
-// Both kernels run the SAME algorithm as the single-CTA ones, step for step, so they return the same results:
+// What the single-CTA routines read from their own shared memory -- the row minima, the lowest asking column of a row,
+// the level minimum of a Dijkstra step, the rows that join the tree, the LCM arg-min -- is reduced or gathered across the
+// cluster through distributed shared memory in both forms.  K depends on n_max only.
+//
+// What one CTA of the global form reads from the matrix per step:
+//   assignment  row minima: one warp per row over the CTA's columns (coalesced row segments); column minima and the
+//               greedy: thread t walks down its column j0 + t (one coalesced row segment per row across the CTA); a
+//               Dijkstra step: the row segment [j0, j0 + B) of every row that joined the tree in the previous step.
+//   LCM         the initial row minima: one warp per owned row, the whole row; per iteration: the whole row of every
+//               owned row whose cached minimum sat in the picked column (one warp per row).  The mask is not written:
+//               a cell reads as mask_value when its row or its column has been picked (flags in shared memory), which is
+//               exactly the value the literal algorithm wrote there.
+//
+// Both kernels run the SAME algorithm as the single-CTA ones, step for step, in both forms, so they return the same
+// results:
 //   assignment  the matching, both potential vectors and the objective of assign_small_solve (td_assign.cu) for every
-//               n <= 232, and results that depend neither on K, nor on n_max, nor on the instance's slot in the batch;
+//               n <= 232, and results that depend neither on K, nor on the storage form, nor on n_max, nor on the
+//               instance's slot in the batch;
 //   LCM         the literal trace (rows, cols, n_pairs, total, last_min) of td_lcm / td_lcm_batch for every params.
 //
 // Every CTA of a cluster takes the same path (also when an instance is withdrawn) and ends with cluster.sync(), so no
@@ -33,7 +48,7 @@ __host__ __device__ constexpr size_t cl_align16(size_t b) { return (b + 15) & ~s
 
 // ---- exact assignment: CTA k owns the columns [k*B, min(n, (k+1)*B)) ------------------------------------------------
 // Shared memory of one CTA (n_max rows, B columns):
-//   c      [n_max][B] int32   the cost block of the CTA's columns
+//   c      [n_max][B] int32   the cost block of the CTA's columns (DSMEM form only; the global form reads the matrix)
 //   u      [n_max]    int64   row potentials (replicated)
 //   mate   [n_max]    int32   column of row i, -1: free (replicated)
 //   tr     [n_max]    int32   rows of the current tree in join order; the rows of one level are a contiguous run (replicated)
@@ -44,10 +59,10 @@ __host__ __device__ constexpr size_t cl_align16(size_t b) { return (b + 15) & ~s
 struct AsgClLayout {
     size_t c, u, mate, tr, xa, xb, p, way, stage, slots, bytes;
 };
-__host__ __device__ inline AsgClLayout asg_cl_layout(int n_max, int B) {
+__host__ __device__ inline AsgClLayout asg_cl_layout(int n_max, int B, bool global) {
     AsgClLayout L;
     size_t o = 0;
-    L.c = o; o = cl_align16(o + size_t(n_max) * B * 4);
+    L.c = o; o = cl_align16(o + (global ? 0 : size_t(n_max) * B * 4));
     L.u = o; o = cl_align16(o + size_t(n_max) * 8);
     L.mate = o; o = cl_align16(o + size_t(n_max) * 4);
     L.tr = o; o = cl_align16(o + size_t(n_max) * 4);
@@ -87,6 +102,7 @@ __device__ __forceinline__ long long block_sum_ll(long long x, long long *s_red)
     return s;
 }
 
+template <bool kGlobal>
 __global__ void __launch_bounds__(kClThreads, 1)
 assign_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict__ sizes, const int64_t *__restrict__ offsets,
                       int n_max, int B, int32_t *col_of_row_out, long long *objective_out, long long *u_out, long long *v_out) {
@@ -116,7 +132,7 @@ assign_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restri
         cluster.sync();
         return;
     }
-    const AsgClLayout L = asg_cl_layout(n_max, B);
+    const AsgClLayout L = asg_cl_layout(n_max, B, kGlobal);
     int32_t *c = reinterpret_cast<int32_t *>(csm + L.c);
     long long *u = reinterpret_cast<long long *>(csm + L.u);
     int *mate = reinterpret_cast<int *>(csm + L.mate);
@@ -135,16 +151,31 @@ assign_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restri
     const int nloc = n - j0 < 0 ? 0 : (n - j0 < B ? n - j0 : B);
     const bool own = t < nloc;               // thread t owns column j0 + t
     const int32_t *src = costs + off;
-    for (int e = t; e < n * nloc; e += kClThreads) {
-        const int i = e / nloc, jl = e - i * nloc;
-        c[i * B + jl] = __ldg(src + size_t(i) * n + j0 + jl);
-    }
-    __syncthreads();
+    // cost[i][j0 + jl]: the staged block, or the matrix itself
+    auto cst = [&](int i, int jl) -> int32_t {
+        if constexpr (kGlobal) return __ldg(src + size_t(i) * n + j0 + jl);
+        else return c[i * B + jl];
+    };
     // row minima: partial over the CTA's columns -> xa, then the minimum of the K partials (order-free: the same value)
-    for (int i = t; i < n; i += kClThreads) {
-        int m = INT_MAX;
-        for (int jl = 0; jl < nloc; ++jl) { const int v0 = c[i * B + ((jl + i) % nloc)]; m = v0 < m ? v0 : m; }
-        xa[i] = m;
+    if constexpr (kGlobal) {
+        for (int i = w; i < n; i += kClWarps) {
+            int m = INT_MAX;
+            for (int jl = lane; jl < nloc; jl += 32) { const int v0 = cst(i, jl); m = v0 < m ? v0 : m; }
+#pragma unroll
+            for (int s = 16; s > 0; s >>= 1) { const int y = __shfl_xor_sync(0xffffffffu, m, s); m = y < m ? y : m; }
+            if (lane == 0) xa[i] = m;
+        }
+    } else {
+        for (int e = t; e < n * nloc; e += kClThreads) {
+            const int i = e / nloc, jl = e - i * nloc;
+            c[i * B + jl] = __ldg(src + size_t(i) * n + j0 + jl);
+        }
+        __syncthreads();
+        for (int i = t; i < n; i += kClThreads) {
+            int m = INT_MAX;
+            for (int jl = 0; jl < nloc; ++jl) { const int v0 = c[i * B + ((jl + i) % nloc)]; m = v0 < m ? v0 : m; }
+            xa[i] = m;
+        }
     }
     cluster.sync();
     for (int i = t; i < n; i += kClThreads) {
@@ -159,7 +190,7 @@ assign_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restri
     long long v = 0;
     if (own) {
         long long m = kInf;
-        for (int i = 0; i < n; ++i) { const long long r = (long long)c[i * B + t] - u[i]; m = r < m ? r : m; }
+        for (int i = 0; i < n; ++i) { const long long r = (long long)cst(i, t) - u[i]; m = r < m ? r : m; }
         v = m;
     }
     // greedy matching on tight cells, as assign_small_solve: every free column asks for the lowest free row that is tight
@@ -175,7 +206,7 @@ assign_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restri
         if (own && p[t] < 0) {
             int pick = -1;
             for (int i = 0; i < n && pick < 0; ++i)
-                if (mate[i] < 0 && (long long)c[i * B + t] - u[i] - v == 0) pick = i;
+                if (mate[i] < 0 && (long long)cst(i, t) - u[i] - v == 0) pick = i;
             if (pick >= 0) atomicMin(&ask[pick], j0 + t);
         }
         cluster.sync();
@@ -212,7 +243,7 @@ assign_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restri
             if (own && !used) {
                 for (int k = lo; k < hi; ++k) {
                     const int r = tr[k];
-                    const long long cur = (long long)c[r * B + t] - u[r] - v;
+                    const long long cur = (long long)cst(r, t) - u[r] - v;
                     if (cur < minv) { minv = cur; way[t] = r == i ? -1 : mate[r]; }
                 }
                 key = minv;
@@ -301,7 +332,7 @@ assign_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restri
             if (u_out) u_out[o + k] = 0;
             if (v_out) v_out[o + k] = 0;
         }
-    const long long part = block_sum_ll(own ? (long long)c[p[t] * B + t] : 0, s_red);
+    const long long part = block_sum_ll(own ? (long long)cst(p[t], t) : 0, s_red);
     if (t == 0) cluster.map_shared_rank(slot_obj, 0)[rank] = part;
     cluster.sync();                          // the last remote access of the cluster
     if (rank == 0 && t == 0) {
@@ -312,19 +343,16 @@ assign_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restri
 }
 
 // ---- LCM: CTA k owns the rows [k*R, min(n, (k+1)*R)) of the working array ---------------------------------------------
-// Shared memory: rk [R] uint64 (cached row minimum keys), d [R][n_max] int32 (the CTA's rows, overwritten with the mask
-// like the reference does), stale [R] int32, slots [2][8] uint64 (every CTA's local arg-min, double-buffered by iteration
-// parity: one cluster.sync per iteration).
-__host__ __device__ inline size_t lcm_cl_bytes(int n_max, int R) {
-    return cl_align16(size_t(R) * 8) + cl_align16(size_t(R) * n_max * 4) + cl_align16(size_t(R) * 4) + 2 * kClMaxK * 8;
+// Shared memory: rk [R] uint64 (cached row minimum keys), d [R][n_max] int32 (DSMEM form: the CTA's rows, overwritten with
+// the mask like the reference does), stale [R] int32, slots [2][8] uint64 (every CTA's local arg-min, double-buffered by
+// iteration parity: one cluster.sync per iteration), and in the global form the picked flags cpick [n_max] and rpick [R]
+// uint8 (column / owned row picked: its cells read as mask_value).
+__host__ __device__ inline size_t lcm_cl_bytes(int n_max, int R, bool global) {
+    return cl_align16(size_t(R) * 8) + cl_align16(global ? 0 : size_t(R) * n_max * 4) + cl_align16(size_t(R) * 4) +
+           2 * kClMaxK * 8 + (global ? cl_align16(size_t(n_max)) + cl_align16(size_t(R)) : 0);
 }
 
-__device__ __forceinline__ uint64_t lcm_cl_row_min(const int32_t *row, int n, int ig, int lane) {
-    uint64_t best = kKeyInf;
-    for (int j = lane; j < n; j += 32) { const uint64_t k = pack_key(row[j], uint32_t(ig * n + j)); best = k < best ? k : best; }
-    return warp_min_u64(best);
-}
-
+template <bool kGlobal>
 __global__ void __launch_bounds__(kClThreads, 1)
 lcm_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict__ sizes, const int64_t *__restrict__ offsets,
                    int n_max, int R, td_lcm_params prm, int32_t *rows_out, int32_t *cols_out, int32_t *n_pairs_out,
@@ -354,15 +382,37 @@ lcm_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict_
     }
     unsigned long long *rk = reinterpret_cast<unsigned long long *>(csm);                          // [R]
     int32_t *d = reinterpret_cast<int32_t *>(csm + cl_align16(size_t(R) * 8));                     // [R][n]
-    int *stale = reinterpret_cast<int *>(reinterpret_cast<unsigned char *>(d) + cl_align16(size_t(R) * n_max * 4));   // [R]
+    int *stale = reinterpret_cast<int *>(reinterpret_cast<unsigned char *>(d) +
+                                         cl_align16(kGlobal ? 0 : size_t(R) * n_max * 4));          // [R]
     unsigned long long *slot = reinterpret_cast<unsigned long long *>(reinterpret_cast<unsigned char *>(stale) +
                                                                       cl_align16(size_t(R) * 4));   // [2][8]
+    unsigned char *cpick = reinterpret_cast<unsigned char *>(slot + 2 * kClMaxK);                    // [n_max]
+    unsigned char *rpick = cpick + cl_align16(size_t(n_max));                                        // [R]
     const int i0 = rank * R;
     const int nloc = n - i0 < 0 ? 0 : (n - i0 < R ? n - i0 : R);
     const int32_t *src = costs + off + size_t(i0) * n;
-    for (int k = t; k < nloc * n; k += kClThreads) d[k] = __ldg(src + k);
+    // the minimum key of owned row il (one warp): the working array's cells, or the matrix with the picked rows and
+    // columns reading as mask_value
+    auto row_min = [&](int il) -> uint64_t {
+        const int ig = i0 + il;
+        uint64_t best = kKeyInf;
+        for (int j = lane; j < n; j += 32) {
+            int32_t x;
+            if constexpr (kGlobal) x = (rpick[il] || cpick[j]) ? prm.mask_value : __ldg(src + size_t(il) * n + j);
+            else x = d[il * n + j];
+            const uint64_t k = pack_key(x, uint32_t(ig * n + j));
+            best = k < best ? k : best;
+        }
+        return warp_min_u64(best);
+    };
+    if constexpr (kGlobal) {
+        for (int k = t; k < n; k += kClThreads) cpick[k] = 0;
+        for (int k = t; k < nloc; k += kClThreads) rpick[k] = 0;
+    } else {
+        for (int k = t; k < nloc * n; k += kClThreads) d[k] = __ldg(src + k);
+    }
     __syncthreads();
-    for (int il = w; il < nloc; il += kClWarps) { const uint64_t k = lcm_cl_row_min(d + il * n, n, i0 + il, lane); if (lane == 0) rk[il] = k; }
+    for (int il = w; il < nloc; il += kClWarps) { const uint64_t k = row_min(il); if (lane == 0) rk[il] = k; }
     const int iters = (prm.max_iters < 0 || prm.max_iters > n) ? n : prm.max_iters;
     long long total = 0;
     int pairs = 0;
@@ -392,11 +442,17 @@ lcm_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict_
         if (rank == 0 && t == 0) { rows_out[o + pairs] = r; cols_out[o + pairs] = cc; }
         ++pairs;
         if (prm.sum_below == INT32_MAX || v < prm.sum_below) total += v;
-        if (r >= i0 && r < i0 + nloc)                     // the owner masks row r
+        if constexpr (kGlobal) {                          // flag row r (its owner) and column cc (every CTA)
+            if (t == 0) {
+                cpick[cc] = 1;
+                if (r >= i0 && r < i0 + nloc) rpick[r - i0] = 1;
+            }
+        } else if (r >= i0 && r < i0 + nloc) {            // the owner masks row r
             for (int j = t; j < n; j += kClThreads) d[(r - i0) * n + j] = prm.mask_value;
+        }
         if (t < nloc) {                                   // every CTA masks column cc in its rows
             const int ig = i0 + t;
-            d[t * n + cc] = prm.mask_value;
+            if constexpr (!kGlobal) d[t * n + cc] = prm.mask_value;
             const uint64_t k = rk[t];
             if (ig == r) rk[t] = pack_key(prm.mask_value, uint32_t(r * n));
             else if (int(key_index(k)) - ig * n == cc) stale[atomicAdd(&s_nstale, 1)] = t;
@@ -406,7 +462,7 @@ lcm_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict_
         const int ns = s_nstale;
         for (int s = w; s < ns; s += kClWarps) {
             const int il = stale[s];
-            const uint64_t k = lcm_cl_row_min(d + il * n, n, i0 + il, lane);
+            const uint64_t k = row_min(il);
             if (lane == 0) rk[il] = k;
         }
         if (prm.residual_size > 0 && n - pairs == prm.residual_size) break;
@@ -422,14 +478,16 @@ lcm_cluster_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict_
 }
 
 // ---- host side ----------------------------------------------------------------------------------------------------------
-// The smallest cluster whose per-CTA block fits next to its O(n) state; depends on n_max only.
+// DSMEM form: the smallest cluster whose per-CTA block fits next to its O(n) state.  Global form: the smallest of {4, 8}
+// that leaves at most one column / row per thread.  Both depend on n_max only.
 template <typename Bytes>
-static int cluster_ctas(int n_max, Bytes bytes) {
+static int cluster_ctas(int n_max, bool global, Bytes bytes) {
+    if (global) return cl_block(n_max, 4) <= kClThreads ? 4 : 8;
     for (int k = 1; k <= kClMaxK; k *= 2)
-        if (bytes(n_max, cl_block(n_max, k)) + kClStaticReserve <= kClSmemLimit) return k;
+        if (bytes(n_max, cl_block(n_max, k), false) + kClStaticReserve <= kClSmemLimit) return k;
     return 0;
 }
-static size_t asg_cl_bytes(int n_max, int B) { return asg_cl_layout(n_max, B).bytes; }
+static size_t asg_cl_bytes(int n_max, int B, bool global) { return asg_cl_layout(n_max, B, global).bytes; }
 
 template <typename... Exp, typename... Act>
 static int launch_clusters(void (*kernel)(Exp...), const char *name, int batch, int k, size_t smem, cudaStream_t st,
@@ -461,37 +519,66 @@ static int launch_clusters(void (*kernel)(Exp...), const char *name, int batch, 
     return TD_OK;
 }
 
-}  // namespace td
-
-extern "C" int td_assign_exact_batch_cluster(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch,
-                                             int n_max, int32_t *col_of_row_out, int64_t *objective_out, int64_t *u_out,
-                                             int64_t *v_out, void *stream) {
-    using namespace td;
-    if (batch < 0 || n_max < 0 || n_max > TD_BATCH_CLUSTER_MAX_N) return TD_ERR_INVALID;
+// The argument rules of the four entry points; they differ in the storage form and its size limit only.
+template <bool kGlobal>
+static int assign_batch(const char *name, int max_n, const int32_t *costs, const int32_t *sizes, const int64_t *offsets,
+                        int batch, int n_max, int32_t *col_of_row_out, int64_t *objective_out, int64_t *u_out,
+                        int64_t *v_out, void *stream) {
+    if (batch < 0 || n_max < 0 || n_max > max_n) return TD_ERR_INVALID;
     if (batch == 0) return TD_OK;
     if (!costs || !sizes || !offsets || !col_of_row_out || !objective_out) return TD_ERR_INVALID;
     if ((reinterpret_cast<uintptr_t>(costs) & 15) != 0) return TD_ERR_INVALID;
     if (!have_device()) return TD_ERR_NO_DEVICE;
-    const int k = cluster_ctas(n_max, asg_cl_bytes);
+    const int k = cluster_ctas(n_max, kGlobal, asg_cl_bytes);
     const int B = k ? cl_block(n_max, k) : 0;
-    return launch_clusters(assign_cluster_kernel, "td_assign_exact_batch_cluster", batch, k, asg_cl_bytes(n_max, B),
+    return launch_clusters(assign_cluster_kernel<kGlobal>, name, batch, k, asg_cl_bytes(n_max, B, kGlobal),
                            static_cast<cudaStream_t>(stream), costs, sizes, offsets, n_max, B, col_of_row_out,
                            reinterpret_cast<long long *>(objective_out), reinterpret_cast<long long *>(u_out),
                            reinterpret_cast<long long *>(v_out));
 }
 
-extern "C" int td_lcm_batch_cluster(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
-                                    const td_lcm_params *params, int32_t *rows_out, int32_t *cols_out, int32_t *n_pairs_out,
-                                    int64_t *total_out, int32_t *last_min_out, void *stream) {
-    using namespace td;
-    if (batch < 0 || n_max < 0 || n_max > TD_BATCH_CLUSTER_MAX_N) return TD_ERR_INVALID;
+template <bool kGlobal>
+static int lcm_batch(const char *name, int max_n, const int32_t *costs, const int32_t *sizes, const int64_t *offsets,
+                     int batch, int n_max, const td_lcm_params *params, int32_t *rows_out, int32_t *cols_out,
+                     int32_t *n_pairs_out, int64_t *total_out, int32_t *last_min_out, void *stream) {
+    if (batch < 0 || n_max < 0 || n_max > max_n) return TD_ERR_INVALID;
     if (batch == 0) return TD_OK;
     if (!costs || !sizes || !offsets || !params || !rows_out || !cols_out || !n_pairs_out || !total_out) return TD_ERR_INVALID;
     if ((reinterpret_cast<uintptr_t>(costs) & 15) != 0) return TD_ERR_INVALID;
     if (!have_device()) return TD_ERR_NO_DEVICE;
-    const int k = cluster_ctas(n_max, lcm_cl_bytes);
+    const int k = cluster_ctas(n_max, kGlobal, lcm_cl_bytes);
     const int R = k ? cl_block(n_max, k) : 0;
-    return launch_clusters(lcm_cluster_kernel, "td_lcm_batch_cluster", batch, k, lcm_cl_bytes(n_max, R),
+    return launch_clusters(lcm_cluster_kernel<kGlobal>, name, batch, k, lcm_cl_bytes(n_max, R, kGlobal),
                            static_cast<cudaStream_t>(stream), costs, sizes, offsets, n_max, R, *params, rows_out, cols_out,
                            n_pairs_out, reinterpret_cast<long long *>(total_out), last_min_out);
+}
+
+}  // namespace td
+
+extern "C" int td_assign_exact_batch_cluster(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch,
+                                             int n_max, int32_t *col_of_row_out, int64_t *objective_out, int64_t *u_out,
+                                             int64_t *v_out, void *stream) {
+    return td::assign_batch<false>("td_assign_exact_batch_cluster", TD_BATCH_CLUSTER_MAX_N, costs, sizes, offsets, batch,
+                                   n_max, col_of_row_out, objective_out, u_out, v_out, stream);
+}
+
+extern "C" int td_lcm_batch_cluster(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                                    const td_lcm_params *params, int32_t *rows_out, int32_t *cols_out, int32_t *n_pairs_out,
+                                    int64_t *total_out, int32_t *last_min_out, void *stream) {
+    return td::lcm_batch<false>("td_lcm_batch_cluster", TD_BATCH_CLUSTER_MAX_N, costs, sizes, offsets, batch, n_max, params,
+                                rows_out, cols_out, n_pairs_out, total_out, last_min_out, stream);
+}
+
+extern "C" int td_assign_exact_batch_large(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch,
+                                           int n_max, int32_t *col_of_row_out, int64_t *objective_out, int64_t *u_out,
+                                           int64_t *v_out, void *stream) {
+    return td::assign_batch<true>("td_assign_exact_batch_large", TD_BATCH_LARGE_MAX_N, costs, sizes, offsets, batch, n_max,
+                                  col_of_row_out, objective_out, u_out, v_out, stream);
+}
+
+extern "C" int td_lcm_batch_large(const int32_t *costs, const int32_t *sizes, const int64_t *offsets, int batch, int n_max,
+                                  const td_lcm_params *params, int32_t *rows_out, int32_t *cols_out, int32_t *n_pairs_out,
+                                  int64_t *total_out, int32_t *last_min_out, void *stream) {
+    return td::lcm_batch<true>("td_lcm_batch_large", TD_BATCH_LARGE_MAX_N, costs, sizes, offsets, batch, n_max, params,
+                               rows_out, cols_out, n_pairs_out, total_out, last_min_out, stream);
 }

@@ -129,6 +129,18 @@ BATCH_CLUSTER_MAX_N = 640   # TD_BATCH_CLUSTER_MAX_N: the largest instance one 8
 # (profiles/cluster_batch_b200.json): at 600 x 600 the loop wins up to 3 instances (1.11 against 1.20 ms) and the cluster
 # from 4 (1.21 against 1.51 ms); at 240 x 240 both take 0.4 ms for 3.  The cluster assignment wins from one instance on.
 LCM_CLUSTER_MIN_BATCH = 4
+BATCH_LARGE_MAX_N = _lib.BATCH_LARGE_MAX_N   # TD_BATCH_LARGE_MAX_N: one cluster per instance, the matrix in global memory
+# run_batch sends the assignments / LCMs of fewer large instances (641 to 2048 rows) than these through single calls.
+# Measured on one NVIDIA B200 at 1000 W (profiles/large_batch_b200.json, 1 to 128 instances of 700 / 1300 / 2000 rows,
+# U[1,39] and stand-derived).  Assignment: from 2 instances the batch wins on stand-derived costs at every size (2 x
+# 2000: 46.7 against 48.1 ms; 8 x 2000: 48.1 against 175 ms), while a lone 2000-row instance loses (46.7 against 25.2
+# ms).  U[1,39] instances are cheap for the whole-GPU solver: the batch wins from 8 (700 rows), 16 (1300) and 32 (2000)
+# instances and loses at most 6 ms below that, so the stand-derived crossover decides.  LCM: a cluster iteration costs
+# about 4.5 us (3.1 ms for 700 rows), a whole-GPU td_lcm call 0.3 ms at 700 and 0.9 ms at 2000 rows, so the batch wins
+# from 64 instances at every size and kind (64 x 2000: 46.7 against 55.7 ms) and loses below (32 x 2000: 43.4
+# against 28.0 ms).
+ASSIGN_LARGE_MIN_BATCH = 2
+LCM_LARGE_MIN_BATCH = 64
 
 
 def pack_batch(costs: Sequence):
@@ -304,7 +316,7 @@ class Engine:
                           c.dual_objective == c.matched_real_cost)
         return out
 
-    # -- batches (td_assign_exact_batch / td_lcm_batch up to 232, the *_cluster kernels up to 640) ------
+    # -- batches (td_assign_exact_batch / td_lcm_batch up to 232, the *_cluster kernels up to 640, *_large up to 2048) --
     def _batch_out(self, out, name, shape, dtype):
         if out is not None and out.get(name) is not None:
             return out[name]
@@ -312,16 +324,19 @@ class Engine:
 
     @staticmethod
     def _batch_kernel(n_max: int, name: str) -> str:
-        """One CTA per instance up to BATCH_MAX_N, one thread-block cluster per instance up to BATCH_CLUSTER_MAX_N."""
+        """One CTA per instance up to BATCH_MAX_N, one thread-block cluster per instance with the matrix in its shared
+        memory up to BATCH_CLUSTER_MAX_N, and in global memory up to BATCH_LARGE_MAX_N."""
         if n_max <= BATCH_MAX_N:
             return name
         if n_max <= BATCH_CLUSTER_MAX_N:
             return name + "_cluster"
-        raise ValueError("batched %s holds instances up to %d rows, got n_max %d" % (name, BATCH_CLUSTER_MAX_N, n_max))
+        if n_max <= BATCH_LARGE_MAX_N:
+            return name + "_large"
+        raise ValueError("batched %s holds instances up to %d rows, got n_max %d" % (name, BATCH_LARGE_MAX_N, n_max))
 
     def assign_batch(self, packed: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor, n_max: int,
                      want_duals: bool = False, out: Optional[dict] = None):
-        """Exact optimum of every instance of a pack_batch() buffer, one launch (n_max <= BATCH_CLUSTER_MAX_N).  Returns
+        """Exact optimum of every instance of a pack_batch() buffer, one launch (n_max <= BATCH_LARGE_MAX_N).  Returns
         device tensors (col [B, n_max] int32, objective [B] int64, u, v) -- u / v are [B, n_max] int64 potentials or
         None.  `out` may supply any of them by name ("col", "objective", "u", "v")."""
         name = self._batch_kernel(int(n_max), "td_assign_exact_batch")
@@ -339,7 +354,7 @@ class Engine:
                   stop_above: int = INT32_MAX, stop_at_value: int = INT32_MAX, sum_below: int = INT32_MAX,
                   residual_size: int = 0, max_iters: int = -1, out: Optional[dict] = None):
         """LCM of every instance of a pack_batch() buffer, one launch, the same params for all (n_max <=
-        BATCH_CLUSTER_MAX_N).  Returns device tensors (rows [B, n_max], cols [B, n_max], n_pairs [B] int32, total [B]
+        BATCH_LARGE_MAX_N).  Returns device tensors (rows [B, n_max], cols [B, n_max], n_pairs [B] int32, total [B]
         int64, last_min [B] int32); `out` may supply any of them by name."""
         name = self._batch_kernel(int(n_max), "td_lcm_batch")
         B = int(sizes.numel())
@@ -712,7 +727,7 @@ def run_packed(packed: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor,
                assign: bool = True, want_duals: bool = False, lcm: Optional[dict] = None):
     """The launch and read-back half of run_batch for a packed buffer already on the device (pack_batch,
     pack_cost_matrices): one launch per kernel, both reading the same buffer, and one device->host copy.  ns are the
-    instance sizes on the host (n_max <= BATCH_CLUSTER_MAX_N).  Returns (assign results, LCM results) as run_batch."""
+    instance sizes on the host (n_max <= BATCH_LARGE_MAX_N).  Returns (assign results, LCM results) as run_batch."""
     eng = engine()
     B = len(ns)
     parts = []
@@ -756,11 +771,31 @@ def run_packed(packed: torch.Tensor, sizes: torch.Tensor, offsets: torch.Tensor,
 
 def size_groups(ns: Sequence[int]):
     """Positions of the instances per batched kernel: ([n <= BATCH_MAX_N], [BATCH_MAX_N < n <= BATCH_CLUSTER_MAX_N],
-    [larger])."""
+    [BATCH_CLUSTER_MAX_N < n <= BATCH_LARGE_MAX_N], [larger])."""
     small = [b for b, n in enumerate(ns) if n <= BATCH_MAX_N]
     mid = [b for b, n in enumerate(ns) if BATCH_MAX_N < n <= BATCH_CLUSTER_MAX_N]
-    large = [b for b, n in enumerate(ns) if n > BATCH_CLUSTER_MAX_N]
-    return small, mid, large
+    large = [b for b, n in enumerate(ns) if BATCH_CLUSTER_MAX_N < n <= BATCH_LARGE_MAX_N]
+    huge = [b for b, n in enumerate(ns) if n > BATCH_LARGE_MAX_N]
+    return small, mid, large, huge
+
+
+def batch_routes(ns: Sequence[int], assign: bool = True, lcm: bool = True):
+    """How run_batch serves instances of sizes ns: ([(positions, assignment batched, LCM batched)] for every batched
+    group that launches, positions whose assignment takes a single call, positions whose LCM takes a single call).  A
+    group goes to its batch kernel when it holds at least the kernel's minimum batch (LCM_CLUSTER_MIN_BATCH,
+    ASSIGN_LARGE_MIN_BATCH, LCM_LARGE_MIN_BATCH); instances above BATCH_LARGE_MAX_N always take single calls."""
+    small, mid, large, huge = size_groups(ns)
+    groups, single_a, single_l = [], list(huge) if assign else [], list(huge) if lcm else []
+    for group, a_min, l_min in ((small, 1, 1), (mid, 1, LCM_CLUSTER_MIN_BATCH),
+                                (large, ASSIGN_LARGE_MIN_BATCH, LCM_LARGE_MIN_BATCH)):
+        ga, gl = assign and len(group) >= a_min, lcm and len(group) >= l_min
+        if assign and not ga:
+            single_a += group
+        if lcm and not gl:
+            single_l += group
+        if group and (ga or gl):
+            groups.append((group, ga, gl))
+    return groups, sorted(single_a), sorted(single_l)
 
 
 def pack_cost_matrices(dist_d: torch.Tensor, instances: Sequence, fill: int = BIG_COST, cutoff: Optional[int] = None,
@@ -806,45 +841,40 @@ def pack_cost_matrices(dist_d: torch.Tensor, instances: Sequence, fill: int = BI
 
 def run_batch(costs: Sequence, assign: bool = True, want_duals: bool = False, lcm: Optional[dict] = None):
     """Exact assignment and / or LCM (`lcm` = its keyword parameters) of every square matrix in `costs`.  The instances
-    are grouped by size: up to BATCH_MAX_N (one CTA each) and up to BATCH_CLUSTER_MAX_N (one thread-block cluster each),
-    every group uploaded once and served by one launch per kernel, both kernels reading the same packed buffer, and
-    read back in one device->host copy; larger ones take the single-instance path.  Returns (assign results, LCM
+    are grouped by size: up to BATCH_MAX_N (one CTA each), up to BATCH_CLUSTER_MAX_N and up to BATCH_LARGE_MAX_N (one
+    thread-block cluster each), every group uploaded once and served by one launch per kernel, both kernels reading the
+    same packed buffer, and read back in one device->host copy; larger ones, and groups smaller than a kernel's minimum
+    batch (batch_routes), take the single-instance path.  Returns (assign results, LCM
     results): lists of (col_of_row, objective[, u, v]) and of LCM() dicts, None for the side not asked for."""
     mats = [np.asarray(c) for c in costs]
     for a in mats:
         if a.ndim != 2 or a.shape[0] != a.shape[1]:
             raise ValueError("run_batch takes square matrices, got shape %s" % (a.shape,))
-    small, mid, large = size_groups([a.shape[0] for a in mats])
+    groups, single_a, single_l = batch_routes([a.shape[0] for a in mats], assign, lcm is not None)
     res_a = [None] * len(mats) if assign else None
     res_l = [None] * len(mats) if lcm is not None else None
-    lcm_single = set(large)
-    for group in (small, mid):
-        group_lcm = lcm
-        if lcm is not None and group is mid and len(group) < LCM_CLUSTER_MIN_BATCH:
-            group_lcm = None                                       # a few mid-size LCMs: single calls are faster
-            lcm_single.update(group)
-        if not group or (not assign and group_lcm is None):
-            continue
+    for group, group_assign, group_lcm in groups:
         packed, sizes, offsets, n_max = pack_batch([mats[b] for b in group])
-        ra, rl = run_packed(packed, sizes, offsets, n_max, [mats[b].shape[0] for b in group], assign, want_duals, group_lcm)
+        ra, rl = run_packed(packed, sizes, offsets, n_max, [mats[b].shape[0] for b in group], group_assign, want_duals,
+                            lcm if group_lcm else None)
         for k, b in enumerate(group):
-            if assign:
+            if group_assign:
                 res_a[b] = ra[k]
-            if group_lcm is not None:
+            if group_lcm:
                 res_l[b] = rl[k]
-    for b in sorted(lcm_single if lcm is not None else large):     # one call each
+    for b in sorted(set(single_a) | set(single_l)):                # one call each
         a = mats[b]
         eng = engine()
         n = a.shape[0]
         c = _h2d_i32(a)
-        if assign and b in large:
+        if b in single_a:
             col, obj, _, _ = eng.assign(c)
             r = (_d2h(col), _d2h_int(obj))
             if want_duals:
                 u, v = eng.assign_duals(n)
                 r = r + (_d2h(u), _d2h(v))
             res_a[b] = r
-        if lcm is not None:
+        if b in single_l:
             res_l[b] = Engine.lcm_host_view(*eng.lcm(c, **lcm))
     return res_a, res_l
 

@@ -228,11 +228,11 @@ def _stage_runner(dist: np.ndarray, solver_batch: Optional[Callable], lcm_batch:
             if transpose and not dist_t:
                 dist_t.append(dist_d.t().contiguous())        # the stand table transposed: a layout copy
             ns = [max(len(c), len(d)) for c, d in insts]
-            small, mid, large = dispatch.size_groups(ns)
-            if large:
-                raise ValueError("the batched experiment holds instances up to %d rows" % dispatch.BATCH_CLUSTER_MAX_N)
+            small, mid, large, huge = dispatch.size_groups(ns)
+            if huge:
+                raise ValueError("the batched experiment holds instances up to %d rows" % dispatch.BATCH_LARGE_MAX_N)
             res_a, res_l = [None] * len(insts), [None] * len(insts)
-            for group in (small, mid):
+            for group in (small, mid, large):
                 if not group:
                     continue
                 packed, sizes, offsets, n_max, gns = dispatch.pack_cost_matrices(
