@@ -104,6 +104,7 @@ int td_cost_matrix_rows(const int32_t *dist, int n_stands,
  * array; stop rules are tested on that minimum; record (e / n, e % n); overwrite that row and
  * column with mask_value.  The mask is a value: masked cells still take part in the argmin
  * (SURVEY.md section 4 trap 4) -- results are bit-identical to the literal array algorithm.
+ * A 0-row call runs no iteration: n_pairs 0, total 0 and last_min INT32_MAX.
  * ------------------------------------------------------------------------------------------ */
 typedef struct td_lcm_params {
     int32_t mask_value;    /* heuristic.py:32 -> 100; split.py:173 / Simulator.java:541 -> big_cost */

@@ -124,3 +124,50 @@ def lcm_c(cost, mask_value, stop_above=INT32_MAX, stop_at_value=INT32_MAX, sum_b
     k = npairs.value
     return {"total": total.value, "rows": rows[:k].copy(), "cols": cols[:k].copy(), "n_pairs": k,
             "last_min": last.value}
+
+
+def lcm_sort_keys(cost) -> np.ndarray:
+    """Every cell's 64-bit key ((uint32(cost) ^ 0x80000000) << 32 | flat index), sorted: the first-index argmin order
+    of the whole matrix.  One sort serves every parameter set of lcm_walk.  n <= 65535 (the index fits 32 bits)."""
+    c = np.asarray(cost, dtype=np.int32)
+    n = int(round(c.size ** 0.5)) if c.ndim == 1 else c.shape[0]
+    assert c.size == n * n and n <= 65535
+    flat = c.reshape(-1)
+    keys = np.empty(n * n, dtype=np.uint64)
+    step = 1 << 24                                    # bounded temporaries at n = 20000 (400 M cells)
+    for lo in range(0, n * n, step):
+        hi = min(lo + step, n * n)
+        k = (flat[lo:hi].view(np.uint32) ^ np.uint32(0x80000000)).astype(np.uint64) << np.uint64(32)
+        k |= np.arange(lo, hi, dtype=np.uint64)
+        keys[lo:hi] = k
+    keys.sort()
+    return keys
+
+
+def lcm_walk(keys, n, mask_value, stop_above=INT32_MAX, stop_at_value=INT32_MAX, sum_below=INT32_MAX,
+             residual_size=0, max_iters=-1):
+    """The literal algorithm walked over lcm_sort_keys(cost) (oracle/lcm_oracle.c: lcm_sorted_walk); the dict of
+    lcm_c, equal to it for every input."""
+    keys = np.ascontiguousarray(keys, dtype=np.uint64)
+    assert keys.size == n * n
+    rows = np.zeros(max(n, 1), dtype=np.int32)
+    cols = np.zeros(max(n, 1), dtype=np.int32)
+    npairs = ctypes.c_int32(0)
+    total = ctypes.c_int64(0)
+    last = ctypes.c_int32(0)
+    p = _Params(mask_value, stop_above, stop_at_value, sum_below, residual_size, max_iters)
+    rc = _clib.lib().lcm_sorted_walk(keys.ctypes.data_as(ctypes.c_void_p), ctypes.c_int(n), ctypes.byref(p),
+                                     rows.ctypes.data_as(ctypes.c_void_p), cols.ctypes.data_as(ctypes.c_void_p),
+                                     ctypes.byref(npairs), ctypes.byref(total), ctypes.byref(last))
+    if rc != 0:
+        raise RuntimeError("lcm_sorted_walk rc=%d" % rc)
+    k = npairs.value
+    return {"total": total.value, "rows": rows[:k].copy(), "cols": cols[:k].copy(), "n_pairs": k,
+            "last_min": last.value}
+
+
+def lcm_sorted(cost, mask_value, **kw):
+    """lcm_c's result through the sorted walk: one sort and one walk."""
+    c = np.asarray(cost, dtype=np.int32)
+    n = int(round(c.size ** 0.5)) if c.ndim == 1 else c.shape[0]
+    return lcm_walk(lcm_sort_keys(c), n, mask_value, **kw)

@@ -416,9 +416,12 @@ lcm_finalize_kernel(const unsigned long long *__restrict__ sorted, int n, td_lcm
                 h |= (r == 0); m = min(m, c);
             }
         }
-        // candidate of iteration t_free: smallest free key (a remaining pick, or the minimum left
-        // behind when the rounds stopped) against the smallest masked cell
-        unsigned long long fk = t_free < P ? sorted[t_free] : ctrl->g_final;
+        // candidate of iteration t_free: smallest free key against the smallest masked cell.  The
+        // smallest free key is the smaller of the next remaining pick and the minimum left behind
+        // when the rounds stopped: the last round may pick a dominant cell above a cell it left
+        // free (that cell's smaller partner lost its other line in the same round).
+        unsigned long long fk = ctrl->g_final;
+        if (t_free < P && sorted[t_free] < fk) fk = sorted[t_free];
         unsigned long long mk = t_free >= 1 ? pack_key(prm.mask_value, h ? 0u : uint32_t(m)) : kKeyInf;
         unsigned long long cand = fk < mk ? fk : mk;
         if (cand != kKeyInf) {
@@ -532,6 +535,13 @@ lcm_batch_kernel(const int32_t *__restrict__ costs, const int32_t *__restrict__ 
     }
 }
 
+// the result of a 0-row call: no pairs, total 0, and last_min INT32_MAX like every other LCM path (no iteration ran)
+__global__ void lcm_empty_kernel(int32_t *n_pairs_out, long long *total_out, int32_t *last_min_out) {
+    *n_pairs_out = 0;
+    *total_out = 0;
+    if (last_min_out) *last_min_out = INT32_MAX;
+}
+
 static size_t lcm_batch_smem_bytes(int n_max) {
     return size_t(n_max) * 8 + size_t(n_max) * n_max * 4 + size_t(n_max) * 4;
 }
@@ -576,8 +586,8 @@ extern "C" int td_lcm(const int32_t *cost, int n, const td_lcm_params *params, i
     if (!have_device()) return TD_ERR_NO_DEVICE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (n == 0) {
-        TD_CUDA_TRY(cudaMemsetAsync(n_pairs_out, 0, sizeof(int32_t), st));
-        TD_CUDA_TRY(cudaMemsetAsync(total_out, 0, sizeof(int64_t), st));
+        lcm_empty_kernel<<<1, 1, 0, st>>>(n_pairs_out, reinterpret_cast<long long *>(total_out), last_min_out);
+        TD_LAUNCH_CHECK();
         return TD_OK;
     }
     if (!cost || !rows_out || !cols_out || !workspace) return TD_ERR_INVALID;
