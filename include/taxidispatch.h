@@ -269,6 +269,62 @@ int td_lcm_batch_large(const int32_t *costs, const int32_t *sizes, const int64_t
                        int32_t *last_min_out /* batch, may be NULL */, void *stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Stand-derived assignment as a stand-to-stand transportation problem, batched
+ *     the exact solve of split.py:139-155 / Simulator.java's solver step without the n x n matrix.
+ *
+ * calculate_cost gives every cab at stand a the same row and every customer at stand b the same
+ * column, so the optimum of the padded matrix M_b = td_cost_matrix(dist, cab_to_b, cust_from_b, fill,
+ * cutoff) (n_b = max(n_c, n_d)) is the optimum of the S x S transportation problem with supplies =
+ * cabs per stand, demands = customers per stand and arc costs C(a, b) = the K1 cell rule on
+ * dist[a][b], plus (n_b - min(n_c, n_d)) * fill for the padding.  M_b is never built: memory and
+ * time are O(S^2) per instance plus passes over the index arrays, at any n.
+ *
+ * Instance b: n_c[b] cab stand indices at cab_to + cab_off[b], n_d[b] customer stand indices at
+ * cust_from + cust_off[b] (all DEVICE arrays); dist (n_stands^2 int32) serves the whole batch.
+ *   objective[b]        the optimum of M_b (int64): what td_assign_exact_rect returns on M_b
+ *   col_of_row[b][i]    stride n_max, i < n_b: a permutation attaining it, from the stand flows
+ *                       f(a, b) by this rule: the cabs of stand a, in increasing index order, go to
+ *                       the customer stands in increasing b, f(a, b) each; the customers of stand b,
+ *                       in increasing index order, are dealt to the cab stands in increasing a.  If
+ *                       n_c < n_d, rows n_c.. take the customers no cab got, in increasing index order;
+ *                       if n_c > n_d, the cabs without a customer take columns n_d.. in increasing row
+ *                       order.  Slots n_b..n_max-1 hold -1.
+ *   cost_of_row[b][i]   (may be NULL) M_b[i][col_of_row[i]], stride n_max, -1 past n_b
+ *   u[b][a], v[b][b']   (may be NULL) int64 stand potentials, stride n_stands: C(a,b) - u[a] - v[b] >= 0
+ *                       for every stand a with a cab and b with a customer, == 0 where flow runs; the
+ *                       side with spare members has potentials <= 0, 0 at a stand with an unmatched
+ *                       member; stands with nobody get 0.  Expanded to rows (u[cab_to[i]]) and columns
+ *                       (v[cust_from[j]]) they pass td_assign_certify on M_b.
+ *   stats[b][0..1]      (may be NULL) shortest-path phases and augmentations of the solve
+ * The optimum returned depends on the instance alone (its stand counts and the table): not on its
+ * position, its neighbours, n_max or the run.  n_c == 0 or n_d == 0 gives n_b * fill and the identity.
+ *
+ * Four launches, always asynchronous.  An instance with a negative size, n_b > n_max, a negative
+ * offset or a stand index outside [0, n_stands) is withdrawn (objective INT64_MIN, col_of_row and
+ * cost_of_row -1, potentials 0); its neighbours are untouched.  The arguments are checked before any
+ * device lookup: TD_ERR_INVALID for batch < 0, n_stands outside [1, TD_STANDS_MAX_S], n_max < 0 or a
+ * NULL required pointer with batch > 0; TD_ERR_WORKSPACE for a workspace smaller than
+ * td_assign_stands_workspace_bytes(batch, n_stands, n_max).  batch == 0 returns TD_OK, launching
+ * nothing.  The workspace holds O(S^2) per instance and one int32 per possible cab (batch x n_max):
+ * pairing the k-th cab of a stand with the k'-th customer of another needs one side listed by stand.
+ *
+ * TD_STANDS_MAX_S: one warp per instance keeps the arc costs and the flows in shared memory, 2 x S x
+ * (S + 1) x 4 B = 132 KB at S = 128 plus O(S) labels and potentials, within one CTA's 227 KB; 128
+ * is also the table bound of the pair and pool kernels.
+ * ------------------------------------------------------------------------------------------ */
+#define TD_STANDS_MAX_S 128
+size_t td_assign_stands_workspace_bytes(int batch, int n_stands, int n_max);
+int td_assign_stands_batch(const int32_t *dist, int n_stands, int32_t fill, int32_t cutoff /* < 0: none */,
+                           const int32_t *cab_to, const int64_t *cab_off, const int32_t *n_c,
+                           const int32_t *cust_from, const int64_t *cust_off, const int32_t *n_d,
+                           int batch, int n_max,
+                           int32_t *col_of_row /* batch x n_max */, int32_t *cost_of_row /* batch x n_max or NULL */,
+                           int64_t *objective /* batch */,
+                           int64_t *u /* batch x n_stands or NULL */, int64_t *v /* batch x n_stands or NULL */,
+                           int32_t *stats /* batch x 2 or NULL */,
+                           void *workspace, size_t workspace_bytes, void *stream);
+
+/* ------------------------------------------------------------------------------------------
  * K4  pool finder          replaces one `pool_n <pool-size> <thread> <file> <n> <out>` process
  *     (pool_n.c:209-238): findPool :153-177, drop_customers :101-151, removeDuplicates :187-207,
  *     shard rule :226-229.
@@ -467,6 +523,12 @@ int tdh_pool_pairs_exact(const int32_t *from, const int32_t *to, int n, const in
  * of tdh_pool_pairs_exact; pairs_out holds n/2 rows */
 int tdh_pool_pairs(const int32_t *from, const int32_t *to, int n, const int32_t *dist, int n_stands,
                    int accept_all, double max_loss, int32_t *pairs_out, int32_t *n_pairs_out, int64_t *cost_out);
+/* one instance of td_assign_stands_batch from host buffers (what a JNI binding of Simulator.java's solver step calls):
+ * col_of_row / cost_of_row hold max(n_cabs, n_cust) entries (cost_of_row, u, v, stats may be NULL; u, v hold n_stands);
+ * a stand index outside the table is TD_ERR_INVALID here */
+int tdh_assign_stands(const int32_t *dist, int n_stands, const int32_t *cab_to, int n_cabs, const int32_t *cust_from,
+                      int n_cust, int32_t fill, int32_t cutoff, int32_t *col_of_row_out, int32_t *cost_of_row_out,
+                      int64_t *objective_out, int64_t *u_out, int64_t *v_out, int32_t *stats_out);
 /* all n_shards logical shards + merge, i.e. what `findpool` produces (findpool.c:122-176) */
 int tdh_pool_find_all(const int32_t *demand, int n, const int32_t *dist, int n_stands, int pool_size,
                       int n_shards, int32_t *plans_out, int32_t cap, int32_t *n_plans_out,

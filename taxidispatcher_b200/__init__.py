@@ -12,7 +12,7 @@ __version__ = "0.1.0"
 _DISPATCH = ("BIG_COST", "Engine", "engine", "calculate_cost", "solve", "solve_dispatch", "solve_full", "LCM",
              "LCM_heuristic", "LCM_split", "LCM_greedy_opt", "LCM_simulate", "LCM_java", "find_pool", "find_pool_all", "find_pool_block", "find_pool_pairs",
              "find_pool_pairs_batch", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "find_pool_all_batch",
-             "pool_merge", "pack_batch", "solve_batch", "LCM_batch", "TaxiDispatchError")
+             "pool_merge", "pack_batch", "solve_stands_batch", "solve_assignment_stands", "solve_batch", "LCM_batch", "TaxiDispatchError")
 
 
 def __getattr__(name):

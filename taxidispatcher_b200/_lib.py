@@ -21,6 +21,7 @@ PAIRS_EXACT_MAX_N = 4096    # TD_PAIRS_EXACT_MAX_N
 PAIRS_BATCH_MAX_N = 4096    # TD_PAIRS_BATCH_MAX_N
 POOL_BATCH_MAX_N = 512      # TD_POOL_BATCH_MAX_N
 BATCH_LARGE_MAX_N = 2048    # TD_BATCH_LARGE_MAX_N
+STANDS_MAX_S = 128          # TD_STANDS_MAX_S
 POOL_REC_W = 9
 PROF_COST, PROF_LCM, PROF_ASSIGN, PROF_POOL_ENUM, PROF_POOL_SELECT = range(5)
 
@@ -107,6 +108,10 @@ _SIGNATURES = {
     "td_pool_batch_workspace_bytes": (ctypes.c_size_t, [_I, _I, ctypes.c_int64]),
     "td_pool_find_all_batch": (_I, [c_vp, c_vp, c_vp, _I, _I, c_vp, _I, _I, _I, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                     ctypes.c_size_t, ctypes.c_int64, c_vp]),
+    "td_assign_stands_workspace_bytes": (ctypes.c_size_t, [_I, _I, _I]),
+    "td_assign_stands_batch": (_I, [c_vp, _I, ctypes.c_int32, ctypes.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, _I, _I,
+                                    c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_size_t, c_vp]),
+    "tdh_assign_stands": (_I, [c_vp, _I, c_vp, _I, c_vp, _I, ctypes.c_int32, ctypes.c_int32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "tdh_pool_pairs_exact": (_I, [c_vp, c_vp, _I, c_vp, _I, _I, ctypes.c_double, c_vp, c_vp, c_vp]),
     "tdh_pool_pairs": (_I, [c_vp, c_vp, _I, c_vp, _I, _I, ctypes.c_double, c_vp, c_vp, c_vp]),
     "tdh_cost_matrix": (_I, [c_vp, _I, c_vp, _I, c_vp, _I, ctypes.c_int32, ctypes.c_int32, c_vp]),

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libtaxidispatch.so")
-SOURCES = ["td_api.cu", "td_cost.cu", "td_lcm.cu", "td_assign.cu", "td_pool.cu", "td_pairs.cu", "td_batch_cluster.cu", "td_pool_batch.cu"]
+SOURCES = ["td_api.cu", "td_cost.cu", "td_lcm.cu", "td_assign.cu", "td_pool.cu", "td_pairs.cu", "td_batch_cluster.cu", "td_pool_batch.cu", "td_assign_stands.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC", "-Xcompiler", "-O3"]
 

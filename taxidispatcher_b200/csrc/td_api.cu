@@ -330,3 +330,44 @@ extern "C" int tdh_pool_find_all(const int32_t *demand, int n, const int32_t *di
     if (m > 0) TDH_TRY(cudaMemcpy(plans_out, d_out.p, size_t(m) * TD_POOL_REC_W * 4, cudaMemcpyDeviceToHost));
     return *n_plans_out > cap ? TD_ERR_CAPACITY : TD_OK;
 }
+
+extern "C" int tdh_assign_stands(const int32_t *dist, int n_stands, const int32_t *cab_to, int n_cabs, const int32_t *cust_from,
+                                 int n_cust, int32_t fill, int32_t cutoff, int32_t *col_of_row_out, int32_t *cost_of_row_out,
+                                 int64_t *objective_out, int64_t *u_out, int64_t *v_out, int32_t *stats_out) {
+    if (n_cabs < 0 || n_cust < 0 || n_stands < 1 || n_stands > TD_STANDS_MAX_S || !dist || !objective_out) return TD_ERR_INVALID;
+    const int n = n_cabs > n_cust ? n_cabs : n_cust;
+    if ((n_cabs && !cab_to) || (n_cust && !cust_from) || (n && !col_of_row_out)) return TD_ERR_INVALID;
+    for (int i = 0; i < n_cabs; ++i) if (cab_to[i] < 0 || cab_to[i] >= n_stands) return TD_ERR_INVALID;
+    for (int j = 0; j < n_cust; ++j) if (cust_from[j] < 0 || cust_from[j] >= n_stands) return TD_ERR_INVALID;
+    if (!td::have_device()) return TD_ERR_NO_DEVICE;
+    // one upload: dist, cab_to, cust_from, then the sizes and (8-byte aligned) offsets of the single instance
+    const size_t S2 = size_t(n_stands) * n_stands, at_cab = S2, at_cust = at_cab + n_cabs, at_size = at_cust + n_cust;
+    const size_t at_off = (at_size + 2 + 1) & ~size_t(1), words = at_off + 4;
+    std::vector<int32_t> h(words, 0);
+    memcpy(h.data(), dist, S2 * 4);
+    if (n_cabs) memcpy(h.data() + at_cab, cab_to, size_t(n_cabs) * 4);
+    if (n_cust) memcpy(h.data() + at_cust, cust_from, size_t(n_cust) * 4);
+    h[at_size] = n_cabs; h[at_size + 1] = n_cust;                 // cab_off = cust_off = 0 (int64 zeros)
+    const size_t nn = size_t(n > 0 ? n : 1), S = size_t(n_stands);
+    const size_t out_bytes = 8 + 8 + 2 * S * 8 + 2 * nn * 4;      // objective, stats, u, v, col, cost
+    const size_t wsb = td_assign_stands_workspace_bytes(1, n_stands, n);
+    td::DevBuf d_in, d_out, d_ws;
+    TDH_TRY(d_in.alloc(words * 4)); TDH_TRY(d_out.alloc(out_bytes)); TDH_TRY(d_ws.alloc(wsb));
+    TDH_TRY(cudaMemcpy(d_in.p, h.data(), words * 4, cudaMemcpyHostToDevice));
+    int32_t *in = d_in.as<int32_t>();
+    char *out = d_out.as<char>();
+    const int64_t *offs = reinterpret_cast<const int64_t *>(in + at_off);
+    int64_t *obj_d = reinterpret_cast<int64_t *>(out), *u_d = reinterpret_cast<int64_t *>(out + 16), *v_d = u_d + S;
+    int32_t *stats_d = reinterpret_cast<int32_t *>(out + 8), *col_d = reinterpret_cast<int32_t *>(v_d + S), *cost_d = col_d + nn;
+    TDH_RC(td_assign_stands_batch(in, n_stands, fill, cutoff, in + at_cab, offs, in + at_size, in + at_cust, offs + 1,
+                                  in + at_size + 1, 1, n, col_d, cost_d, obj_d, u_d, v_d, stats_d, d_ws.p, wsb, nullptr));
+    std::vector<char> host(out_bytes);
+    TDH_TRY(cudaMemcpy(host.data(), out, out_bytes, cudaMemcpyDeviceToHost));
+    memcpy(objective_out, host.data(), 8);
+    if (stats_out) memcpy(stats_out, host.data() + 8, 8);
+    if (u_out) memcpy(u_out, host.data() + 16, S * 8);
+    if (v_out) memcpy(v_out, host.data() + 16 + S * 8, S * 8);
+    if (n) memcpy(col_of_row_out, host.data() + 16 + 2 * S * 8, size_t(n) * 4);
+    if (n && cost_of_row_out) memcpy(cost_of_row_out, host.data() + 16 + 2 * S * 8 + nn * 4, size_t(n) * 4);
+    return TD_OK;
+}

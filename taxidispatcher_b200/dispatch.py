@@ -14,6 +14,7 @@ Host functions mirror the reference's names, argument order and return layouts
   find_pool_pairs_batch(...)                       Simulator.findPool over many instances in one launch
   find_pool_all_batch(...)                         the whole findpool job over many small demand sets in one launch
   find_pool_pairs_exact(...) / find_pool_pairs_exact_batch(...)   the optimum of pool_optimum.py / pool_opt_min.py
+  solve_stands_batch(...) / solve_assignment_stands(...)    exact stand-derived solves as S x S transportation problems
 
 PyTorch is used only for device buffers, pinned staging and streams.  All arithmetic runs in the
 hand-written CUDA kernels behind the C ABI (include/taxidispatch.h).  There is no CPU fallback:
@@ -31,7 +32,7 @@ import torch
 from . import _lib
 from ._lib import BIG_COST, INT32_MAX, PAIRS_EXACT_MAX_N, POOL_REC_W, AssignStats, LcmParams, PoolStats, TaxiDispatchError, check
 
-__all__ = ["BIG_COST", "Engine", "calculate_cost", "solve", "solve_dispatch", "solve_full", "solve_assignment", "LCM", "LCM_heuristic",
+__all__ = ["BIG_COST", "Engine", "calculate_cost", "solve", "solve_dispatch", "solve_full", "solve_assignment", "solve_assignment_stands", "solve_stands_batch", "pack_stands_batch", "LCM", "LCM_heuristic",
            "LCM_split", "LCM_greedy_opt", "LCM_simulate", "LCM_java", "find_pool", "find_pool_all", "find_pool_block",
            "find_pool_pairs", "find_pool_pairs_batch", "find_pool_pairs_exact", "find_pool_pairs_exact_batch", "find_pool_all_batch", "pack_pool_batch", "pool_merge", "pack_batch", "pack_cost_matrices", "run_packed", "run_batch", "solve_batch", "LCM_batch",
            "TaxiDispatchError"]
@@ -129,6 +130,7 @@ BATCH_CLUSTER_MAX_N = 640   # TD_BATCH_CLUSTER_MAX_N: the largest instance one 8
 # (profiles/cluster_batch_b200.json): at 600 x 600 the loop wins up to 3 instances (1.11 against 1.20 ms) and the cluster
 # from 4 (1.21 against 1.51 ms); at 240 x 240 both take 0.4 ms for 3.  The cluster assignment wins from one instance on.
 LCM_CLUSTER_MIN_BATCH = 4
+STANDS_MAX_S = _lib.STANDS_MAX_S   # TD_STANDS_MAX_S: the largest stand table td_assign_stands_batch holds
 BATCH_LARGE_MAX_N = _lib.BATCH_LARGE_MAX_N   # TD_BATCH_LARGE_MAX_N: one cluster per instance, the matrix in global memory
 # run_batch sends the assignments / LCMs of fewer large instances (641 to 2048 rows) than these through single calls.
 # Measured on one NVIDIA B200 at 1000 W (profiles/large_batch_b200.json, 1 to 128 instances of 700 / 1300 / 2000 rows,
@@ -369,6 +371,30 @@ class Engine:
                                      _ptr(cols), _ptr(npairs), _ptr(total), _ptr(last), _stream())
         check(rc, name)
         return rows, cols, npairs, total, last
+
+    # -- stand-derived assignment as S x S transportation problems (td_assign_stands_batch) ---------------------------
+    def assign_stands_batch(self, dist: torch.Tensor, cab_to: torch.Tensor, cab_off: torch.Tensor, n_c: torch.Tensor,
+                            cust_from: torch.Tensor, cust_off: torch.Tensor, n_d: torch.Tensor, n_max: int,
+                            fill: int = BIG_COST, cutoff: Optional[int] = None, want_cost: bool = False,
+                            want_duals: bool = False, want_stats: bool = False, out: Optional[dict] = None):
+        """Exact optimum of every stand-derived instance (include/taxidispatch.h, td_assign_stands_batch), device tensors
+        in and out: (col [B, n_max] int32, cost [B, n_max] int32 or None, objective [B] int64, u [B, S], v [B, S] int64
+        or None, stats [B, 2] int32 or None).  `out` may supply any of them by name."""
+        B, S = int(n_c.numel()), int(dist.shape[0])
+        col = self._batch_out(out, "col", (B, n_max), torch.int32)
+        cost = self._batch_out(out, "cost", (B, n_max), torch.int32) if want_cost else None
+        obj = self._batch_out(out, "objective", (B,), torch.int64)
+        u = self._batch_out(out, "u", (B, S), torch.int64) if want_duals else None
+        v = self._batch_out(out, "v", (B, S), torch.int64) if want_duals else None
+        stats = self._batch_out(out, "stats", (B, 2), torch.int32) if want_stats else None
+        nbytes = self.lib.td_assign_stands_workspace_bytes(B, S, int(n_max))
+        ws = self._workspace("stands", nbytes)
+        rc = self.lib.td_assign_stands_batch(_ptr(dist), S, int(fill), -1 if cutoff is None else int(cutoff), _ptr(cab_to),
+                                             _ptr(cab_off), _ptr(n_c), _ptr(cust_from), _ptr(cust_off), _ptr(n_d), B,
+                                             int(n_max), _ptr(col), _ptr(cost), _ptr(obj), _ptr(u), _ptr(v), _ptr(stats),
+                                             _ptr(ws), ws.numel(), _stream())
+        check(rc, "td_assign_stands_batch")
+        return col, cost, obj, u, v, stats
 
     # -- K4 ---------------------------------------------------------------------------------------
     def pool_find(self, demand: torch.Tensor, dist: torch.Tensor, pool_size: int, shard: int = 0, n_shards: int = 8,
@@ -798,6 +824,23 @@ def batch_routes(ns: Sequence[int], assign: bool = True, lcm: bool = True):
     return groups, sorted(single_a), sorted(single_l)
 
 
+def _stand_indices(dist_d: torch.Tensor, instances: Sequence):
+    """(cab_to, cust_from) pairs of stand index arrays -> (cabs, custs, idx, pos): the int32 host arrays, their
+    concatenation (all cab arrays, then all customer arrays, then one pad word) and the start of every array in it.
+    Raises IndexError for a stand outside the table, as calculate_cost does."""
+    cabs = [np.asarray(c, dtype=np.int32).reshape(-1) for c, _ in instances]
+    custs = [np.asarray(d, dtype=np.int32).reshape(-1) for _, d in instances]
+    s = int(dist_d.shape[0]) if dist_d.numel() else 0
+    for c, d in zip(cabs, custs):
+        if len(c) and len(d) and (int(c.max()) >= s or int(c.min()) < 0 or int(d.max()) >= s or int(d.min()) < 0):
+            raise IndexError("stand index out of range of the distance table")   # as calculate_cost
+    idx = np.concatenate(cabs + custs + [np.zeros(1, np.int32)])
+    pos = [0]
+    for a in cabs + custs:
+        pos.append(pos[-1] + len(a))
+    return cabs, custs, idx, pos
+
+
 def pack_cost_matrices(dist_d: torch.Tensor, instances: Sequence, fill: int = BIG_COST, cutoff: Optional[int] = None,
                        transpose: bool = False):
     """calculate_cost (positional, square-padded with `fill`, optional cutoff) of every (cab_to, cust_from) pair of stand
@@ -806,8 +849,7 @@ def pack_cost_matrices(dist_d: torch.Tensor, instances: Sequence, fill: int = BI
     transposed stand table).  The index arrays and the sizes / offsets travel in ONE host->device copy.  Returns
     (packed, sizes, offsets, n_max, ns)."""
     eng = engine()
-    cabs = [np.asarray(c, dtype=np.int32).reshape(-1) for c, _ in instances]
-    custs = [np.asarray(d, dtype=np.int32).reshape(-1) for _, d in instances]
+    cabs, custs, idx, pos = _stand_indices(dist_d, instances)
     ns = [max(len(c), len(d)) for c, d in zip(cabs, custs)]
     B = len(ns)
     offsets = np.zeros(B, dtype=np.int64)
@@ -815,20 +857,12 @@ def pack_cost_matrices(dist_d: torch.Tensor, instances: Sequence, fill: int = BI
     for b, n in enumerate(ns):
         offsets[b] = total
         total += (n * n + 3) & ~3
-    s = int(dist_d.shape[0]) if dist_d.numel() else 0
-    for c, d in zip(cabs, custs):
-        if len(c) and len(d) and (int(c.max()) >= s or int(c.min()) < 0 or int(d.max()) >= s or int(d.min()) < 0):
-            raise IndexError("stand index out of range of the distance table")   # as calculate_cost
-    idx = np.concatenate(cabs + custs + [np.zeros(1, np.int32)])
     off_at = (B + 1) & ~1                                 # offsets at an even int32 index (int64 view)
     meta = np.zeros(off_at + 2 * B + 1, dtype=np.int32)
     meta[:B] = ns
     meta[off_at: off_at + 2 * B] = offsets.view(np.int32)
     idx_d, meta_d = _h2d_i32_many([idx, meta])
     packed = torch.empty(max(total, 4), dtype=torch.int32, device=eng.device)
-    pos = [0]
-    for a in cabs + custs:
-        pos.append(pos[-1] + len(a))
     for b, n in enumerate(ns):
         if n == 0:
             continue
@@ -837,6 +871,95 @@ def pack_cost_matrices(dist_d: torch.Tensor, instances: Sequence, fill: int = BI
         rows, cols = (cust_d, cab_d) if transpose else (cab_d, cust_d)
         eng.cost_matrix(dist_d, rows, cols, fill, cutoff, out=packed[int(offsets[b]): int(offsets[b]) + n * n].view(n, n))
     return packed, meta_d[:B], meta_d[off_at: off_at + 2 * B].view(torch.int64), (max(ns) if B else 0), ns
+
+
+def pack_stands_batch(instances: Sequence, dist=None):
+    """(cab_to, cust_from) stand index arrays of every instance -> the device arguments of Engine.assign_stands_batch,
+    in ONE pinned host->device copy: a dict with cab_to, cab_off, n_c, cust_from, cust_off, n_d (device tensors; both
+    index arguments view the same concatenated buffer), n_max and ns (host).  With `dist` (host stand table) the table
+    travels in the same copy and comes back as "dist"; without it the stand check is left to the kernel (an instance
+    with a stand outside the table is withdrawn)."""
+    dist_np = None if dist is None else np.ascontiguousarray(np.asarray(dist, dtype=np.int32))
+    probe = torch.empty((0, 0)) if dist_np is None else torch.from_numpy(dist_np)
+    if dist_np is None:
+        cabs = [np.asarray(c, dtype=np.int32).reshape(-1) for c, _ in instances]
+        custs = [np.asarray(d, dtype=np.int32).reshape(-1) for _, d in instances]
+        idx = np.concatenate(cabs + custs + [np.zeros(1, np.int32)])
+    else:
+        cabs, custs, idx, _ = _stand_indices(probe, instances)
+    B = len(cabs)
+    nc = np.array([len(c) for c in cabs], dtype=np.int32)
+    nd = np.array([len(d) for d in custs], dtype=np.int32)
+    cab_off = np.zeros(B, dtype=np.int64)
+    cust_off = np.zeros(B, dtype=np.int64)
+    if B:
+        cab_off[1:] = np.cumsum(nc[:-1])
+        cust_off[:] = int(nc.sum()) + np.concatenate([[0], np.cumsum(nd[:-1])])
+    off_at = (2 * B + 1) & ~1
+    meta = np.zeros(off_at + 4 * B + 1, dtype=np.int32)
+    meta[:B], meta[B: 2 * B] = nc, nd
+    meta[off_at: off_at + 2 * B] = cab_off.view(np.int32)
+    meta[off_at + 2 * B: off_at + 4 * B] = cust_off.view(np.int32)
+    parts = [idx, meta] + ([] if dist_np is None else [dist_np])
+    up = _h2d_i32_many(parts)
+    idx_d, meta_d = up[0], up[1]
+    ns = [int(max(a, b)) for a, b in zip(nc, nd)]
+    out = {"cab_to": idx_d, "cust_from": idx_d, "n_c": meta_d[:B], "n_d": meta_d[B: 2 * B],
+           "cab_off": meta_d[off_at: off_at + 2 * B].view(torch.int64),
+           "cust_off": meta_d[off_at + 2 * B: off_at + 4 * B].view(torch.int64), "n_max": max(ns) if B else 0, "ns": ns}
+    if dist_np is not None:
+        out["dist"] = up[2]
+    return out
+
+
+def solve_stands_batch(distances, instances: Sequence, fill: int = BIG_COST, cutoff: Optional[int] = None,
+                       want_duals: bool = False):
+    """Exact optimum of calculate_cost(distances, ...) for every (cab_to, cust_from) pair of stand index arrays, solved
+    as S x S transportation problems (td_assign_stands_batch, S <= STANDS_MAX_S): one upload, one call and one read-back,
+    no n x n matrix anywhere.  Returns a list of (col_of_row, objective), or (col_of_row, objective, u, v) with the
+    stand potentials (u per cab stand, v per customer stand) when want_duals.  Raises IndexError for a stand outside the
+    table, as calculate_cost does."""
+    eng = engine()
+    dist = np.asarray(distances)
+    pk = pack_stands_batch(instances, dist)
+    B, n_max, S = len(pk["ns"]), pk["n_max"], int(dist.shape[0])
+    parts = [(B * n_max, torch.int32), (B, torch.int64)] + ([(B * S, torch.int64)] * 2 if want_duals else [])
+    arena = _Arena(eng.device, parts)
+    views = list(arena.views)
+    out = {"col": views[0].view(B, n_max), "objective": views[1]}
+    if want_duals:
+        out["u"], out["v"] = views[2].view(B, S), views[3].view(B, S)
+    eng.assign_stands_batch(pk["dist"], pk["cab_to"], pk["cab_off"], pk["n_c"], pk["cust_from"], pk["cust_off"], pk["n_d"],
+                            n_max, fill, cutoff, want_duals=want_duals, out=out)
+    host = arena.host()
+    col, obj = host[0].reshape(B, n_max), host[1]
+    res = []
+    for b, n in enumerate(pk["ns"]):
+        r = (col[b, :n].copy(), int(obj[b]))
+        res.append(r + (host[2].reshape(B, S)[b].copy(), host[3].reshape(B, S)[b].copy()) if want_duals else r)
+    return res
+
+
+def solve_assignment_stands(dist_d: torch.Tensor, cab_to, cust_from, fill: int = BIG_COST, cutoff: Optional[int] = None):
+    """solve_assignment through the stand transportation solver: the same (n, col_of_row[n], cost_of_row[n]) triple
+    with the same optimum (possibly another of the tied optima), no n x n matrix built.  dist_d is the stand table on
+    the device (n_stands <= STANDS_MAX_S).  IndexError for a stand outside the table (as calculate_cost);
+    TaxiDispatchError when the kernel withdraws the instance."""
+    n = max(len(cab_to), len(cust_from))
+    if n == 0:
+        return 0, np.zeros(0, np.int32), np.zeros(0, np.int32)
+    eng = engine()
+    _stand_indices(dist_d, [(cab_to, cust_from)])
+    pk = pack_stands_batch([(cab_to, cust_from)])
+    arena = _Arena(eng.device, [(n, torch.int32), (n, torch.int32), (1, torch.int64)])
+    col, cost, obj = arena.views
+    eng.assign_stands_batch(dist_d, pk["cab_to"], pk["cab_off"], pk["n_c"], pk["cust_from"], pk["cust_off"], pk["n_d"], n,
+                            fill, cutoff, out={"col": col.view(1, n), "cost": cost.view(1, n), "objective": obj},
+                            want_cost=True)
+    col_h, cost_h, obj_h = arena.host()
+    if int(obj_h[0]) == -(1 << 63):
+        raise TaxiDispatchError(_lib.TD_ERR_INVALID, "td_assign_stands_batch", "instance withdrawn")
+    return n, col_h.copy(), cost_h.copy()
 
 
 def run_batch(costs: Sequence, assign: bool = True, want_duals: bool = False, lcm: Optional[dict] = None):
